@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: PnP-ADMM image-iterations/sec at 256x256 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--size S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch B] [--size S] [--dump-outputs DIR]
 
 One "step" = one PnP-ADMM iteration (U-Net denoise -> centred FFT -> masked k-space solve -> inverse FFT ->
 dual update; reference evaluation/env.py:85-93) over one batch of B synthetic 256x256 CS-MRI images
@@ -15,6 +15,10 @@ dual update; reference evaluation/env.py:85-93) over one batch of B synthetic 25
                launch durations (CUDA events around every launch, pnp_unet_profile) vs the measured bf16 peak
   cpu_baseline the CPU oracle (restatement of the reference's PyTorch path) on this host's cores, bounded sample
   --impl reference   only the CPU leg, as its own JSON line
+  --dump-outputs DIR after the timed steps, rank 0 writes what the timed path computed in its last step as DIR/<name>.npy
+                     (float32 or float64; complex arrays get a trailing (re, im) axis; at most 64 MB, a seeded
+                     sample of the images when the whole batch is larger): the state x, z, u and, for `ours`, the rewards.
+                     Inputs and weights are seeded, so two builds run with the same arguments can be compared file by file.
 """
 from __future__ import annotations
 
@@ -168,6 +172,34 @@ def make_inputs(B, S, seed0=0):
     return {k: np.concatenate([v] * reps, axis=0)[:B] for k, v in base.items()}
 
 
+DUMP_LIMIT_BYTES = 64_000_000     # --dump-outputs writes at most this much
+
+
+def dump_index(B, image_bytes, other_bytes):
+    """Images whose per-image outputs --dump-outputs writes: all B when they fit under DUMP_LIMIT_BYTES next to
+    `other_bytes`, else a fixed seeded sample (sorted), the same on every run with the same arguments.  ValueError when
+    not even one image fits."""
+    import torch
+    n = min(B, (DUMP_LIMIT_BYTES - other_bytes) // image_bytes)
+    if n < 1:
+        raise ValueError(f"--dump-outputs: x, z and u of one image ({image_bytes} bytes) do not fit in the "
+                         f"{DUMP_LIMIT_BYTES}-byte limit; use a smaller --size")
+    idx = np.arange(B) if n >= B else np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    return torch.from_numpy(idx)
+
+
+def write_outputs(out_dir, arrays):
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a.detach().cpu()
+        if a.is_complex():
+            a = torch.view_as_real(a)
+        if a.dtype != torch.float64:
+            a = a.to(torch.float32)
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.numpy())
+
+
 # ------------------------------------------------------------------------------------------------
 def cpu_leg(S, threads, sample_B, steps, warmup):
     """The reference's PyTorch CPU path (oracle restatement) on this host."""
@@ -186,7 +218,7 @@ def cpu_leg(S, threads, sample_B, steps, warmup):
         st, _ = O.step(params, st, a)
         ts.append(time.perf_counter() - t0)
     t = float(np.mean(ts[warmup:]))
-    return sample_B / t, t
+    return sample_B / t, t, st
 
 
 def run_reference(args):
@@ -196,7 +228,10 @@ def run_reference(args):
     threads = os.cpu_count() or 1
     S = args.size
     sample_B = 8 if S <= 256 else 2
-    v, t = cpu_leg(S, threads, sample_B, args.steps, args.warmup)
+    v, t, st = cpu_leg(S, threads, sample_B, args.steps, args.warmup)
+    if args.dump_outputs:
+        idx = dump_index(sample_B, 20 * S * S, 0)      # x fp32 + z, u complex64: 20 bytes per pixel
+        write_outputs(args.dump_outputs, {k: st[k].index_select(0, idx) for k in ("x", "z", "u")})
     out = {"metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
            "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
            "data": "synthetic", "impl": "reference",
@@ -329,6 +364,13 @@ def run_ours(args):
     t1 = time.time()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop(t0, t1)
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # copied now: the legs below step the same engine again.  The rewards are those of every rank, in rank order
+        reward = rew if world == 1 else (allr[:, :B].reshape(-1) if peer is not None else allr)
+        idx = dump_index(B, 20 * S * S, 4 * reward.numel()).to(dev)     # x fp32 + z, u complex64: 20 bytes per pixel
+        dumped = {"x": eng.x.index_select(0, idx), "z": eng.z.index_select(0, idx), "u": eng.u.index_select(0, idx),
+                  "reward": reward.clone()}
     tmax = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
@@ -772,12 +814,12 @@ def run_ours(args):
     if rank == 0 and world == 1 and not args.no_cpu:
         threads = os.cpu_count() or 1
         sB = 8 if S <= 256 else 2
-        v, t = cpu_leg(S, threads, sB, 3, 1)
+        v, t, _ = cpu_leg(S, threads, sB, 3, 1)
         cpu = {"value": v, "unit": UNIT, "cores": threads, "kind": "port",
                "sample": f"3 steps of {sB} images at {S}x{S} after 1 warm-up (oracle = PyTorch CPU restatement of the "
                          f"reference step), {threads} threads"}
         if S <= 256:            # SURVEY 8d: the one-thread figure next to the all-cores one (2 images, 1 step after 1 warm-up)
-            v1, _ = cpu_leg(S, 1, 2, 1, 1)
+            v1, _, _ = cpu_leg(S, 1, 2, 1, 1)
             cpu["value_1_thread"] = v1
 
     if rank == 0:
@@ -807,6 +849,8 @@ def run_ours(args):
                "dt_driven": variants.get("dt_driven_rollout"),   # BASELINE config 2 as named (policy in the loop)
                "tflops_whole_step": world * B * K * GFLOP_PER_IMAGE.get(S, 0) / (ms * 1e-3) / 1e3}
         print(json.dumps(out), flush=True)
+    if dumped is not None:
+        write_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 
@@ -823,7 +867,14 @@ def main():
     ap.add_argument("--noise", type=float, default=0.0, help="complex Gaussian k-space noise sigma (x/255)")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-variants", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.dump_outputs:
+        try:            # refused before the run rather than after its timed steps
+            dump_index(args.batch, 20 * args.size ** 2, 4 * args.gpus * args.batch)
+        except ValueError as ex:
+            ap.error(str(ex))
     global ACCEL, NOISE
     ACCEL, NOISE = args.accel, args.noise
     if args.impl == "reference":

@@ -196,10 +196,12 @@ def test_batched_step_equals_per_image_steps():
 
 @pytest.mark.ref
 def test_oracle_equals_live_reference():
-    """Only where /root/reference exists: re-run the pin live (same checks as make_golden, one step)."""
+    """One step of the original project's own ``PnPEnv`` against the oracle, on a case no stored fixture covers (kaiming
+    seed 5, 128x128 radial 25 %, k-space noise 5).  Needs the original's source tree (``PNP_REFERENCE_ROOT``, see
+    oracle/ref_shim.py); no stored result of the original exists for this case, so without the tree it skips."""
     from oracle import ref_shim
     if not ref_shim.available():
-        pytest.skip("reference tree not present")
+        pytest.skip("the original project's source tree is not present (PNP_REFERENCE_ROOT); no stored result for this case")
     ns = ref_shim.load()
     params = O.init_unet_params(5, "kaiming")
     item = synth.make_item(synth.phantom(128, 128, 2), synth.radial_mask(128, 128, 0.25), 5.0, 2)
