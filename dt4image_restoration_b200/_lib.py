@@ -65,8 +65,6 @@ SIGNATURES = {
     "pnp_conv3x3_packed_bytes": (c_size_t, [c_int, c_int]),
     "pnp_conv3x3_bf16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                  c_int, c_int, c_int, c_void_p]),
-    "pnp_conv3x3_ups_bf16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
-                                     c_int, c_int, c_int, c_void_p]),
     "pnp_policy_packed_floats": (c_size_t, [c_int, c_int]),
     "pnp_policy_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                 C.c_float, C.c_float, C.c_float, c_int, c_int, c_int, c_int, c_void_p]),

@@ -324,15 +324,6 @@ int pnp_conv3x3_bf16(const void* in0, int C0, const void* in1, int C1, const flo
                                   B, H, W, Cout, cudaStream_t(stream)), "pnp_conv3x3_bf16");
 }
 
-int pnp_conv3x3_ups_bf16(const void* in0, int C0, const void* in1_half, int C1, const float* weights, const float* bias,
-                         void* out, void* scratch, int B, int H, int W, int Cout, void* stream) {
-  REQUIRE_INIT();
-  if (!in1_half || C1 <= 0) { set_error("pnp_conv3x3_ups_bf16: the half-resolution segment is required"); return -1; }
-  return fail_cuda(conv3x3_single(static_cast<const __nv_bfloat16*>(in0), C0, static_cast<const __nv_bfloat16*>(in1_half),
-                                  C1, weights, bias, static_cast<__nv_bfloat16*>(out), static_cast<uint8_t*>(scratch),
-                                  B, H, W, Cout, cudaStream_t(stream), 1), "pnp_conv3x3_ups_bf16");
-}
-
 int pnp_step_prepared(pnp_unet_plan* plan, const float* v, const float* sigma, const void* u_in, const void* y0T,
                       const uint8_t* maskT, long long mask_batch_stride, const float* mu, int mu_stride, float* x_out,
                       void* z_out, void* u_out, float* v_next, void* stream) {

@@ -65,6 +65,6 @@ int unet_set_splitk(int mode);
 size_t conv_packed_bytes(int Cin, int Cout);
 int conv3x3_single(const __nv_bfloat16* in0, int C0, const __nv_bfloat16* in1, int C1, const float* w_fp32,
                    const float* bias, __nv_bfloat16* out, uint8_t* wpk_scratch, int B, int H, int W, int Cout,
-                   cudaStream_t st, int in1_is_half_res = 0);
+                   cudaStream_t st);
 
 }  // namespace pnp

@@ -4,7 +4,6 @@
 //                         on CUDA cores (K = 18 is not tensor-core work), NHWC bf16 out
 //   conv3x3_umma_kernel : every other 3x3 conv (unet_conv.cuh), incl. the fused 1x1 output conv + global
 //                         residual + clamp in the FINAL epilogue
-//   maxpool2_kernel     : nn.MaxPool2d(2) (noise.py:23), NHWC bf16
 //   upsample2x_kernel   : nn.Upsample(x2, bilinear, align_corners=True) + zero pad to the skip size
 //                         (noise.py:39,46-53), NHWC bf16; the channel concat (noise.py:59) is never
 //                         materialised - the consuming conv walks two tensor maps
@@ -117,23 +116,6 @@ __global__ void __launch_bounds__(256) conv_first_kernel(const float* __restrict
   }
 }
 
-
-// in [B,H,W,C] -> out [B,H/2,W/2,C]; grid (ceil(Wo*C8/256), Ho, B), one thread per 8 channels of one output pixel.
-__global__ void __launch_bounds__(256) maxpool2_kernel(const uint4* __restrict__ in, uint4* __restrict__ out, int B,
-                                                       int H, int W, int C8) {
-  grid_dep_launch();
-  grid_dep_wait();
-  const int Ho = H / 2, Wo = W / 2;
-  const int e = blockIdx.x * blockDim.x + threadIdx.x;
-  if (e >= Wo * C8) return;
-  const int c = e % C8, xo = e / C8;
-  const int yo = blockIdx.y, b = blockIdx.z;
-  const size_t r0 = ((size_t(b) * H + 2 * yo) * W + 2 * xo) * C8 + c;
-  const size_t r1 = r0 + size_t(W) * C8;
-  const uint4 m = bf16x8_max(bf16x8_max(__ldg(in + r0), __ldg(in + r0 + C8)),
-                             bf16x8_max(__ldg(in + r1), __ldg(in + r1 + C8)));
-  out[(size_t(b) * Ho + yo) * Wo * C8 + e] = m;
-}
 
 // in [B,h,w,C] -> out [B,Ho,Wo,C]: bilinear x2 (align_corners=True) placed at offset (py,px), zeros elsewhere.
 // grid (ceil(Wo*C8/256), ceil(Ho/4), B); each thread produces 8 channels of 4 vertically adjacent output pixels
@@ -373,13 +355,10 @@ int unet_global_init() {
   rc |= set_conv_attr<32, 64, EPI_BF16>();
   rc |= set_conv_attr<64, 64, EPI_BF16>();
   rc |= set_conv_attr<64, 128, EPI_BF16>();
-  rc |= int(cudaFuncSetAttribute(conv3x3_pair_kernel<32, 32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
   rc |= int(cudaFuncSetAttribute(conv3x3_pair_kernel<32, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
   rc |= int(cudaFuncSetAttribute(conv3x3_pair_kernel<64, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
   rc |= int(cudaFuncSetAttribute(conv3x3_pair_kernel<64, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
-  rc |= int(cudaFuncSetAttribute(conv3x3_kws_kernel<EPI_BF16>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
-  rc |= int(cudaFuncSetAttribute(conv3x3_kws_kernel<EPI_FINAL>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
-  rc |= int(cudaFuncSetAttribute(conv3x3_kws_kernel<EPI_BF16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
+  rc |= int(cudaFuncSetAttribute(conv3x3_kws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kConvSmemMax));
   rc |= int(cudaFuncSetAttribute(conv3x3_splitk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSkSmem));
   if (rc) set_error("cudaFuncSetAttribute(MaxDynamicSharedMemorySize) failed");
   return rc;
@@ -389,15 +368,14 @@ int num_sms() { return g_num_sms; }
 
 // NHWC bf16 activation tensor -> 4-D map (C, W, H, N), box (KC, 18, 18, 1), swizzle = KC*2 bytes.
 static int make_act_map(CUtensorMap* m, const void* base, int B, int H, int W, int C, int KC, int box_w = kHalo,
-                        int box_h = kHalo, bool linear = false) {
+                        int box_h = kHalo) {
   if (!g_encode) { set_error("pnp_init() has not been called"); return -3; }
   cuuint64_t dims[4] = {cuuint64_t(C), cuuint64_t(W), cuuint64_t(H), cuuint64_t(B)};
   cuuint64_t strides[3] = {cuuint64_t(C) * 2, cuuint64_t(W) * C * 2, cuuint64_t(H) * W * C * 2};
   cuuint32_t box[4] = {cuuint32_t(KC), cuuint32_t(box_w), cuuint32_t(box_h), 1};
   cuuint32_t estr[4] = {1, 1, 1, 1};
   CUresult r = g_encode(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, estr,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE,
-                        linear ? CU_TENSOR_MAP_SWIZZLE_NONE : (KC == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B),
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, KC == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("cuTensorMapEncodeTiled failed (code " + std::to_string(int(r)) + ")");
@@ -418,30 +396,39 @@ struct ConvLaunch {
   int smem;
 };
 
-// Ring sizing: weights stay resident when the whole n-tile fits next to >= 3 halo stages; otherwise they are
-// streamed through as deep a ring as fits (latency of an L2 fetch ~1 us vs ~0.1-0.3 us of MMA work per tap).
+// barriers + epilogue constants of a conv CTA, sized for ConvCfg::NACC = 4 (BN = 32); what is left of the budget after
+// them and the alignment slack goes to the rings
+static const int kConvBarBytes = (4 * 16 + 2 * 4 + 2) * 8 + 16 + kEpiSmemFloats * 4;
+static const int kConvRingBytes = kConvSmemBudget - 1024 - kConvBarBytes - 1024;
+static int halo_stage_bytes(int KC) { return (kHalo * kHalo * KC * 2 + 1023) / 1024 * 1024; }
+
+// A CTA keeps its weights resident when it has one n-tile and all of it (wbytes) fits next to >= 3 halo stages; otherwise
+// they are streamed through as deep a ring as fits (latency of an L2 fetch ~1 us vs ~0.1-0.3 us of MMA work per tap).
+static bool weights_fit(int KC, int n_tiles, long long wbytes) {
+  return n_tiles == 1 && wbytes + 3 * halo_stage_bytes(KC) <= kConvRingBytes;
+}
+
 static void size_rings(ConvLaunch& L) {
   if (L.kws) {
     const int bar = KwsCfg::BAR_BYTES;
     const int avail = kConvSmemBudget - 1024 - bar - 1024;
     const int wtotal = (L.p.nchunks0 + L.p.nchunks1) * 3 * KwsCfg::B_BYTES;
-    const int src = L.p.ups_fused ? kKwsSrcStages * kKwsSrcStage : 0;     // low-resolution patches of the fused upsample
-    int sa = (avail - wtotal - src) / KwsCfg::A_STAGE;
+    int sa = (avail - wtotal) / KwsCfg::A_STAGE;
     L.p.wres = 1; L.p.sb = 1;
     L.p.sa = sa > 8 ? 8 : sa;
-    L.smem = 1024 + L.p.sa * KwsCfg::A_STAGE + ((wtotal + 1023) & ~1023) + src + bar;
+    L.smem = 1024 + L.p.sa * KwsCfg::A_STAGE + ((wtotal + 1023) & ~1023) + bar;
     return;
   }
   const int ROWB = L.KC * 2;
-  const int a_stage = (kHalo * kHalo * ROWB + 1023) / 1024 * 1024;
+  const int a_stage = halo_stage_bytes(L.KC);
   const int b_bytes = L.BN * ROWB / (L.pair ? 2 : 1);       // a CTA of a pair keeps half of every weight blob
   const int b_stage = (b_bytes + 1023) / 1024 * 1024;
-  const int bar = (4 * 16 + 2 * 4 + 2) * 8 + 16 + kEpiSmemFloats * 4;   // sized for ConvCfg::NACC = 4 (BN = 32)
-  const int avail = kConvSmemBudget - 1024 - bar - 1024;
+  const int bar = kConvBarBytes;
+  const int avail = kConvRingBytes;
   const int nchunks = L.p.nchunks0 + L.p.nchunks1;
   const int wtotal = nchunks * 9 * b_bytes;
   ConvParams& p = L.p;
-  if (p.n_tiles == 1 && wtotal + 3 * a_stage <= avail) {
+  if (weights_fit(L.KC, p.n_tiles, wtotal)) {
     p.wres = 1;
     p.sb = 1;
     int sa = (avail - wtotal) / a_stage;
@@ -473,7 +460,7 @@ size_t conv_packed_bytes(int Cin, int Cout) { return size_t(Cin) * Cout * 9 * 2;
 
 static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __nv_bfloat16* in1, int C1,
                       const uint8_t* wpk, const float* bias, __nv_bfloat16* out, int B, int H, int W, int Cout,
-                      int epi, int img0 = 0, int nimg = -1, bool in1_is_half_res = false) {
+                      int epi) {
   const bool kws = use_kws(C0, C1, Cout);
   const int KC = (!kws && C0 % 64 == 0 && C1 % 64 == 0) ? 64 : 32;
   if (C0 % KC || C1 % KC || C0 <= 0) { set_error("conv: channel counts must be multiples of 32"); return -4; }
@@ -483,32 +470,21 @@ static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __n
   L = ConvLaunch{};
   L.KC = KC; L.BN = BN; L.EPI = epi; L.kws = kws ? 1 : 0;
   {
-    // CTA-pair kernel (unet_conv_pair.cuh).  PNP_CONV_PAIR: 0 off, 1 every eligible layer, 64 / 128 only that BN, unset =
-    // auto: the layers whose weights do not stay resident in a single CTA (streamed weights: -4..-12 % per layer, both
-    // in burst and in the power-capped sustained run); layers with resident weights gain nothing from halving them.
+    // CTA-pair kernel (unet_conv_pair.cuh) for the layers whose weights do not stay resident in a single CTA (streamed
+    // weights: -4..-12 % per layer, both in burst and in the power-capped sustained run); layers with resident weights
+    // gain nothing from halving them.  PNP_CONV_PAIR=0 / 1 forces the single-CTA / pair kernel for every eligible layer.
     static const int pair_env = [] { const char* e = getenv("PNP_CONV_PAIR"); return e ? atoi(e) : -1; }();
-    const bool eligible = !kws && epi == EPI_BF16 && (BN == 64 || BN == 128 || (BN == 32 && pair_env == 32));
-    bool want = false;
-    if (pair_env < 0) {
-      const int rowb = KC * 2;
-      const long long wtotal = (long long)((C0 + C1) / KC) * 9 * BN * rowb;
-      const int a_stage = (kHalo * kHalo * rowb + 1023) / 1024 * 1024;
-      const int avail = kConvSmemBudget - 1024 - ((4 * 16 + 2 * 2 + 2) * 8 + 16 + kEpiSmemFloats * 4) - 1024;
-      const bool resident_single = (Cout / BN == 1) && (wtotal + 3 * a_stage <= avail);
-      want = !resident_single;
-    } else {
-      want = pair_env == 1 || pair_env == BN;
-    }
-    L.pair = (eligible && want && pair_env != 0) ? 1 : 0;
+    const bool eligible = !kws && epi == EPI_BF16 && (BN == 64 || BN == 128);
+    const bool want = pair_env < 0 ? !weights_fit(KC, Cout / BN, (long long)(C0 + C1) * 9 * BN * 2) : pair_env == 1;
+    L.pair = (eligible && want) ? 1 : 0;
   }
   ConvParams& p = L.p;
-  if (nimg < 0) nimg = B;
   {
     // Split-K kernel (unet_conv_splitk.cuh) when it puts at least kSkGain times as many CTAs to work as the ordinary
     // kernels would (one image, or a few, at the deep levels) and still runs as ONE wave.  S = the largest power of two
     // <= 8 that divides the 64-channel slices and keeps units * S within the SM count.
-    const long long pix_tiles = (long long)nimg * ((W + kTile - 1) / kTile) * ((H + kTile - 1) / kTile);
-    const bool eligible = !kws && epi == EPI_BF16 && KC == 64 && !in1_is_half_res && Cout % kSkBN == 0;
+    const long long pix_tiles = (long long)B * ((W + kTile - 1) / kTile) * ((H + kTile - 1) / kTile);
+    const bool eligible = !kws && epi == EPI_BF16 && KC == 64 && Cout % kSkBN == 0;
     const long long units = pix_tiles * (Cout / kSkBN);
     if (eligible && g_splitk_mode != 0 && (units <= g_num_sms || g_splitk_mode == 1) && units < (1ll << 24)) {
       const int nch = (C0 + C1) / kSkKC;
@@ -521,24 +497,15 @@ static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __n
       }
     }
   }
-  p.B = nimg; p.H = H; p.W = W;
+  p.B = B; p.H = H; p.W = W;
   p.tiles_x = kws ? (W + kKwsTileW - 1) / kKwsTileW : (W + kTile - 1) / kTile;
   p.tiles_y = kws ? (H + kKwsTileH - 1) / kKwsTileH : (H + kTile - 1) / kTile;
   p.n_tiles = Cout / BN;
   p.nchunks0 = C0 / KC; p.nchunks1 = C1 / KC;
   p.Cout = Cout; p.wpk = wpk; p.bias = bias; p.out = out; p.slope = 0.2f;
-  p.img0 = img0;
-  p.direct_store = 0;      // the lane-transposed 64-byte stores won every measurement (DESIGN.md 4.1)
-  if (in1_is_half_res) {
-    // in1 is the [B, H/2, W/2, C1] tensor whose x2 bilinear upsample (align_corners) is the second input segment
-    if (!kws || epi != EPI_BF16 || (H & 1) || (W & 1) || H < 4 || W < 4) { set_error("conv: fused upsample needs the kw-stacked kernel and even H, W"); return -4; }
-    p.ups_fused = 1;
-    p.ups_sy = float(H / 2 - 1) / float(H - 1);
-    p.ups_sx = float(W / 2 - 1) / float(W - 1);
-  }
   p.mg_n = conv_magic(uint32_t(p.n_tiles)); p.mg_x = conv_magic(uint32_t(p.tiles_x)); p.mg_y = conv_magic(uint32_t(p.tiles_y));
   {
-    const long long tiles_all = (long long)nimg * p.tiles_x * p.tiles_y * p.n_tiles;
+    const long long tiles_all = (long long)B * p.tiles_x * p.tiles_y * p.n_tiles;
     const int dmax = std::max(p.n_tiles, std::max(p.tiles_x, p.tiles_y));
     if (tiles_all * dmax >= (1ll << 32) || Cout > 512) { set_error("conv: problem too large for the tile index arithmetic"); return -4; }
   }
@@ -546,8 +513,7 @@ static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __n
   const int bw = kws ? kKwsHaloW : kHalo, bh = kws ? kKwsHaloH : kHalo;
   int rc = make_act_map(&L.tm0, in0, B, H, W, C0, KC, bw, bh);
   if (rc) return rc;
-  if (in1_is_half_res) rc = make_act_map(&L.tm1, in1, B, H / 2, W / 2, C1, KC, kKwsSrcW, kKwsSrcH, true);
-  else rc = C1 > 0 ? make_act_map(&L.tm1, in1, B, H, W, C1, KC, bw, bh) : make_act_map(&L.tm1, in0, B, H, W, C0, KC, bw, bh);
+  rc = C1 > 0 ? make_act_map(&L.tm1, in1, B, H, W, C1, KC, bw, bh) : make_act_map(&L.tm1, in0, B, H, W, C0, KC, bw, bh);
   if (rc) return rc;
   if (L.pair) {
     // rows = all blobs of the layer back to back (blob = BN rows of KC bf16, already swizzled: copied verbatim)
@@ -561,9 +527,9 @@ static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __n
                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled (weights) failed (code " + std::to_string(int(r)) + ")"); return 1000 + int(r); }
   }
-  long long tiles = (long long)nimg * p.tiles_x * p.tiles_y * p.n_tiles;
+  long long tiles = (long long)B * p.tiles_x * p.tiles_y * p.n_tiles;
   if (L.pair) {     // pair tiles: two pixel tiles with the same n-tile; grid = 2 CTAs per pair
-    const long long pix = (long long)nimg * p.tiles_x * p.tiles_y;
+    const long long pix = (long long)B * p.tiles_x * p.tiles_y;
     tiles = (pix + 1) / 2 * p.n_tiles;
     p.total_tiles = int(tiles);
     const long long pairs = g_num_sms / 2;
@@ -573,7 +539,7 @@ static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __n
   L.grid = int(tiles < g_num_sms ? tiles : g_num_sms);
   }
   if (L.splitk) {
-    L.grid = int((long long)nimg * p.tiles_x * p.tiles_y * (Cout / kSkBN) * p.sk_split);
+    L.grid = int((long long)B * p.tiles_x * p.tiles_y * (Cout / kSkBN) * p.sk_split);
     L.smem = sk_smem_bytes(p.sk_stages);
   }
   return 0;
@@ -581,7 +547,6 @@ static int build_conv(ConvLaunch& L, const __nv_bfloat16* in0, int C0, const __n
 
 // All kernels of the denoiser are launched with programmatic stream serialization (PDL): each one may begin while its
 // predecessor drains (see grid_dep_launch / grid_dep_wait in common.cuh).
-static bool pdl_enabled() { return true; }
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg{};
@@ -590,7 +555,7 @@ static cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
 
@@ -608,13 +573,11 @@ static int launch_conv(const ConvLaunch& L, cudaStream_t st) {
     attr[0].val.clusterDim.x = unsigned(L.p.sk_split); attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr; cfg.numAttrs = pdl_enabled() ? 2 : 1;
+    cfg.attrs = attr; cfg.numAttrs = 2;
     return int(cudaLaunchKernelEx(&cfg, conv3x3_splitk_kernel, L.p, L.tm0, L.tm1));
   }
   if (L.pair) {
-    if (L.KC == 32 && L.BN == 32)
-      launch_k(conv3x3_pair_kernel<32, 32>, dim3(L.grid), dim3(kConvThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1, L.tmw);
-    else if (L.KC == 32 && L.BN == 64)
+    if (L.KC == 32 && L.BN == 64)
       launch_k(conv3x3_pair_kernel<32, 64>, dim3(L.grid), dim3(kConvThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1, L.tmw);
     else if (L.KC == 64 && L.BN == 64)
       launch_k(conv3x3_pair_kernel<64, 64>, dim3(L.grid), dim3(kConvThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1, L.tmw);
@@ -624,12 +587,7 @@ static int launch_conv(const ConvLaunch& L, cudaStream_t st) {
     return int(cudaGetLastError());
   }
   if (L.kws) {
-    if (L.p.ups_fused)
-      launch_k(conv3x3_kws_kernel<EPI_BF16, true>, dim3(L.grid), dim3(kKwsUpsThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1);
-    else if (L.EPI == EPI_FINAL)
-      launch_k(conv3x3_kws_kernel<EPI_FINAL>, dim3(L.grid), dim3(kConvThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1);
-    else
-      launch_k(conv3x3_kws_kernel<EPI_BF16>, dim3(L.grid), dim3(kConvThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1);
+    launch_k(conv3x3_kws_kernel, dim3(L.grid), dim3(kConvThreads), size_t(L.smem), st, L.p, L.tm0, L.tm1);
     return int(cudaGetLastError());
   }
   if (L.EPI == EPI_FINAL) launch_conv_t<32, 32, EPI_FINAL>(L, st);
@@ -660,30 +618,12 @@ int pack_conv_weights(const float* w_fp32, uint8_t* out, int Cin, int Cout, int 
 // Single conv (test / bench entry): packs the weights into `wpk_scratch` and runs one launch.
 int conv3x3_single(const __nv_bfloat16* in0, int C0, const __nv_bfloat16* in1, int C1, const float* w_fp32,
                    const float* bias, __nv_bfloat16* out, uint8_t* wpk_scratch, int B, int H, int W, int Cout,
-                   cudaStream_t st, int in1_is_half_res) {
+                   cudaStream_t st) {
   ConvLaunch L;
-  int rc = build_conv(L, in0, C0, in1, C1, wpk_scratch, bias, out, B, H, W, Cout, EPI_BF16, 0, -1, in1_is_half_res != 0);
+  int rc = build_conv(L, in0, C0, in1, C1, wpk_scratch, bias, out, B, H, W, Cout, EPI_BF16);
   if (rc) return rc;
   rc = pack_conv_weights(w_fp32, wpk_scratch, C0 + C1, Cout, L.KC, st, L.kws != 0);
   if (rc) return rc;
-  if (getenv("PNP_CONV_DBG")) {   // developer aid: per-CTA stall counters of one launch, printed to stderr (synchronises)
-    long long* d = nullptr;
-    cudaMalloc(&d, size_t(L.grid) * kDbgSlots * sizeof(long long));
-    cudaMemsetAsync(d, 0, size_t(L.grid) * kDbgSlots * sizeof(long long), st);
-    L.p.dbg = d;
-    rc = launch_conv(L, st);
-    cudaStreamSynchronize(st);
-    std::vector<long long> h(size_t(L.grid) * kDbgSlots);
-    cudaMemcpy(h.data(), d, h.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-    cudaFree(d);
-    double s[kDbgSlots] = {0};
-    for (int i = 0; i < L.grid; ++i)
-      for (int k = 0; k < kDbgSlots; ++k) s[k] += double(h[size_t(i) * kDbgSlots + k]) / L.grid;
-    fprintf(stderr, "conv dbg KC=%d BN=%d wres=%d sa=%d sb=%d grid=%d | mma: acc_empty %.0f a_full %.0f b_full %.0f total %.0f | "
-            "producer: a_empty %.0f b_empty %.0f | epilogue: acc_full %.0f total %.0f [tmem ld %.0f math %.0f stores %.0f] (clk, mean per CTA)\n",
-            L.KC, L.BN, L.p.wres, L.p.sa, L.p.sb, L.grid, s[0], s[1], s[2], s[3], s[4], s[5], s[6], s[7], s[8], s[9], s[10]);
-    return rc;
-  }
   return launch_conv(L, st);
 }
 
@@ -694,13 +634,12 @@ static const int kCh[5] = {32, 64, 128, 256, 512};
 
 struct TensorSlot { size_t off; int C, H, W; };
 
-enum { K_FIRST = 0, K_UMMA = 1, K_POOL = 2, K_UPS = 3 };
+enum { K_FIRST = 0, K_UMMA = 1, K_UPS = 3 };      // values reported by unet_profile (kinds[])
 
 struct Op {
   int kind;
-  int id;                   // conv: layer index 0..26; pool: 100 + level; upsample: 200 + level
+  int id;                   // conv: layer index 0..26; upsample: 200 + level
   int level;                // pyramid level the op writes
-  int img0, nimg;           // image range of this launch
   int conv;                 // index into convs (K_UMMA)
   int rev;                  // sweep direction (alternates launch by launch, see ConvParams::rev)
 };
@@ -715,8 +654,6 @@ struct UnetPlan {
   TensorSlot tA[5], tB[5], skip[5], pooled[5], ups[4];
   std::vector<ConvLaunch> convs;   // tensor-core conv launches
   std::vector<Op> ops;             // execution order
-  int chunk, shallow;
-  int ups_fused[4];                // level l: the upsample feeding up-block l is fused into its first conv (not materialised)
   FirstConvW first;                // host copy of the 2->32 conv (passed by value as a kernel parameter)
 };
 
@@ -795,9 +732,8 @@ size_t unet_workspace_bytes(int B, int H, int W) {
   return plan_layout(&P);
 }
 
-// Execution schedule.  Levels < `shallow` (full and half resolution) run in chunks of `chunk` images so that a
-// layer's output is still L2-resident (126 MB) when the next layer reads it; the deep levels, which are
-// tensor-bound and need the whole batch to fill 148 SMs, run once over the full batch in between.
+// Execution schedule: the first conv, the down blocks, the up blocks, every launch over the whole (micro-)batch.  Running the
+// shallow levels in chunks of images for L2 residency was measured on B200 (profiles/r01_*) and lost to the launch count.
 int unet_plan_create(UnetPlan** out, const uint8_t* packed, uint8_t* workspace, size_t workspace_bytes, int B, int H,
                      int W) {
   if (B <= 0 || H < 16 || W < 16) { set_error("unet plan: need B>0 and H,W >= 16"); return -1; }
@@ -810,53 +746,23 @@ int unet_plan_create(UnetPlan** out, const uint8_t* packed, uint8_t* workspace, 
     delete P; set_error("unet plan: workspace / packed weights must be 1024-byte aligned"); return -6;
   }
   P->ws = workspace; P->ws_bytes = workspace_bytes; P->wts = packed;
-  // plain layer-by-layer over the whole (micro-)batch: chunking the shallow levels for L2 residency was measured on B200
-  // (profiles/r01_*) and loses to the launch count, so the schedule below always runs with one chunk
-  P->chunk = B; P->shallow = 0;
   LayerDesc L[27]; size_t ow, ob, n, pk;
   layer_table(L, ow, ob, n, pk);
   const float* flat = reinterpret_cast<const float*>(packed + pk);
   auto T = [&](const TensorSlot& s) { return reinterpret_cast<__nv_bfloat16*>(P->ws + s.off); };
   int rc = 0;
-  // fused upsample (unet_conv_kws.cuh): correct; 0.40 ms instead of 0.13 + 0.24 ms for up4 at B=64 256^2, end to end a
-  // tie (+0.4 % in the sustained run), so it stays opt-in (PNP_UNET_FUSE_UPS=1)
-  const bool fuse_ups_env = getenv("PNP_UNET_FUSE_UPS") && atoi(getenv("PNP_UNET_FUSE_UPS")) != 0;
-  // MaxPool2d(2) is fused into the epilogue of the conv that produces the skip tensor unless PNP_UNET_FUSE_POOL=0
-  const bool fuse_pool = true;
-  auto conv = [&](int li, const TensorSlot& in0, const TensorSlot* in1, const TensorSlot& o, int lvl, int img0,
-                  int nimg, const TensorSlot* pooled = nullptr, bool in1_half = false) {
+  auto conv = [&](int li, const TensorSlot& in0, const TensorSlot* in1, const TensorSlot& o, int lvl,
+                  const TensorSlot* pooled = nullptr) {
     if (rc) return;
     ConvLaunch cl;
     const int epi = (li == 26) ? EPI_FINAL : EPI_BF16;
     rc = build_conv(cl, T(in0), in0.C, in1 ? T(*in1) : nullptr, in1 ? in1->C : 0, packed + L[li].pk_off,
-                    flat + L[li].b_off, T(o), B, P->Hl[lvl], P->Wl[lvl], L[li].cout, epi, img0, nimg, in1_half);
+                    flat + L[li].b_off, T(o), B, P->Hl[lvl], P->Wl[lvl], L[li].cout, epi);
     if (rc) return;
     if (epi == EPI_FINAL) { cl.p.wout = flat + ow; cl.p.bout = flat + ob; }
     if (pooled) cl.p.pool_out = T(*pooled);
     P->convs.push_back(cl);
-    P->ops.push_back(Op{K_UMMA, li, lvl, img0, nimg, int(P->convs.size()) - 1});
-  };
-  auto down_block = [&](int l, int img0, int nimg, bool with_pool) {     // l = 1..4
-    if (with_pool && !fuse_pool) P->ops.push_back(Op{K_POOL, 100 + l, l, img0, nimg, -1});
-    conv(l * 3 + 0, P->pooled[l], nullptr, P->tA[l], l, img0, nimg);
-    conv(l * 3 + 1, P->tA[l], nullptr, P->tB[l], l, img0, nimg);
-    conv(l * 3 + 2, P->tB[l], nullptr, P->skip[l], l, img0, nimg, (fuse_pool && l < 4) ? &P->pooled[l + 1] : nullptr);
-  };
-  auto up_block = [&](int l, int img0, int nimg) {                        // l = 3..0 (up1..up4)
-    const int blk = 5 + (3 - l);
-    // up4: optionally fuse the upsample into the conv (kw-stacked kernel) when the size doubles exactly
-    const TensorSlot& lo = (l == 3) ? P->skip[4] : P->tA[l + 1];
-    const bool fuse_ups = fuse_ups_env && use_kws(kCh[l], kCh[l + 1], kCh[l]) && P->Hl[l] == 2 * P->Hl[l + 1] &&
-                          P->Wl[l] == 2 * P->Wl[l + 1] && P->Hl[l] >= 4 && P->Wl[l] >= 4;
-    if (fuse_ups) {
-      P->ups_fused[l] = 1;
-      conv(blk * 3 + 0, P->skip[l], &lo, P->tA[l], l, img0, nimg, nullptr, true);
-    } else {
-      P->ops.push_back(Op{K_UPS, 200 + l, l, img0, nimg, -1});
-      conv(blk * 3 + 0, P->skip[l], &P->ups[l], P->tA[l], l, img0, nimg);
-    }
-    conv(blk * 3 + 1, P->tA[l], nullptr, P->tB[l], l, img0, nimg);
-    conv(blk * 3 + 2, P->tB[l], nullptr, P->tA[l], l, img0, nimg);
+    P->ops.push_back(Op{K_UMMA, li, lvl, int(P->convs.size()) - 1});
   };
   {
     // first-layer weights to the host (plan creation may synchronise): fp32 [32][2][3][3] + bias[32]
@@ -879,35 +785,28 @@ int unet_plan_create(UnetPlan** out, const uint8_t* packed, uint8_t* workspace, 
         }
     }
   }
-  const int SL = P->shallow;
-  // phase A: shallow levels of the contracting path, chunk by chunk (when SL == 0 this is the whole batch once)
-  const int stepA = SL > 0 ? P->chunk : B;
-  for (int i0 = 0; i0 < B; i0 += stepA) {
-    const int ni = (B - i0 < stepA) ? B - i0 : stepA;
-    P->ops.push_back(Op{K_FIRST, 0, 0, i0, ni, -1});
-    conv(1, P->tA[0], nullptr, P->tB[0], 0, i0, ni);
-    conv(2, P->tB[0], nullptr, P->skip[0], 0, i0, ni, fuse_pool ? &P->pooled[1] : nullptr);
-    for (int l = 1; l < (SL > 0 ? SL : 1); ++l) down_block(l, i0, ni, true);
-    if (SL > 0 && SL <= 4 && !fuse_pool) P->ops.push_back(Op{K_POOL, 100 + SL, SL, i0, ni, -1});   // input of the first deep level
+  // MaxPool2d(2) is fused into the epilogue of the conv that produces the skip tensor
+  P->ops.push_back(Op{K_FIRST, 0, 0, -1});
+  conv(1, P->tA[0], nullptr, P->tB[0], 0);
+  conv(2, P->tB[0], nullptr, P->skip[0], 0, &P->pooled[1]);
+  for (int l = 1; l <= 4; ++l) {
+    conv(l * 3 + 0, P->pooled[l], nullptr, P->tA[l], l);
+    conv(l * 3 + 1, P->tA[l], nullptr, P->tB[l], l);
+    conv(l * 3 + 2, P->tB[l], nullptr, P->skip[l], l, l < 4 ? &P->pooled[l + 1] : nullptr);
   }
-  // phase B: deep levels over the full batch
-  const int first_deep = SL > 0 ? SL : 1;
-  for (int l = first_deep; l <= 4; ++l) down_block(l, 0, B, !(SL > 0 && l == SL));
-  for (int l = 3; l >= SL; --l) up_block(l, 0, B);
-  // phase C: shallow levels of the expanding path, chunk by chunk
-  if (SL > 0) {
-    for (int i0 = 0; i0 < B; i0 += P->chunk) {
-      const int ni = (B - i0 < P->chunk) ? B - i0 : P->chunk;
-      for (int l = (SL - 1 < 3 ? SL - 1 : 3); l >= 0; --l) up_block(l, i0, ni);
-    }
+  for (int l = 3; l >= 0; --l) {                    // up1 .. up4
+    const int blk = 5 + (3 - l);
+    P->ops.push_back(Op{K_UPS, 200 + l, l, -1});
+    conv(blk * 3 + 0, P->skip[l], &P->ups[l], P->tA[l], l);
+    conv(blk * 3 + 1, P->tA[l], nullptr, P->tB[l], l);
+    conv(blk * 3 + 2, P->tB[l], nullptr, P->tA[l], l);
   }
   if (rc) { delete P; return rc; }
   {
     // alternate the sweep direction launch by launch: a consumer starts with what its producer wrote last (L2 hits)
-    const bool alt = true;
     int k = 0;
     for (Op& op : P->ops) {
-      op.rev = alt ? (k & 1) : 0;
+      op.rev = k & 1;
       if (op.kind == K_UMMA) P->convs[op.conv].p.rev = op.rev;
       ++k;
     }
@@ -937,7 +836,7 @@ int unet_plan_tensor(const UnetPlan* P, const char* name, size_t* off, int* C, i
     for (int k = 1; k <= 4 && !s; ++k) {
       const int l = 4 - k;
       const std::string u = "up" + std::to_string(k);
-      if (n == u + ".upsampled" && !P->ups_fused[l]) s = &P->ups[l];
+      if (n == u + ".upsampled") s = &P->ups[l];
     }
   }
   if (!s) return -1;
@@ -961,9 +860,7 @@ static int unet_forward_impl(UnetPlan* P, const float* v, const float* sigma, fl
                              cudaStream_t st, ProfileCtx* prof, const uint8_t* active = nullptr) {
   LayerDesc L[27]; size_t ow, ob, n, pk;
   layer_table(L, ow, ob, n, pk);
-  auto T = [&](const TensorSlot& s, int img0) {
-    return reinterpret_cast<__nv_bfloat16*>(P->ws + s.off) + size_t(img0) * s.H * s.W * s.C;
-  };
+  auto T = [&](const TensorSlot& s) { return reinterpret_cast<__nv_bfloat16*>(P->ws + s.off); };
   int rc = 0;
   for (const Op& op : P->ops) {
     if (prof) prof->begin();
@@ -972,25 +869,15 @@ static int unet_forward_impl(UnetPlan* P, const float* v, const float* sigma, fl
         const int bd = P->W >= 256 ? 256 : ((P->W + 31) / 32) * 32;
         const int gx = (P->W + bd - 1) / bd, pairs = (P->H + 1) / 2;
         int ppt = 4;                                 // long walks only when the grid still fills the machine twice over
-        while (ppt > 1 && size_t(gx) * ((pairs + ppt - 1) / ppt) * op.nimg < 4 * 148) ppt >>= 1;
-        launch_k(conv_first_kernel, dim3(gx, (pairs + ppt - 1) / ppt, op.nimg), dim3(bd), 0, st,
-                 v + size_t(op.img0) * P->H * P->W, sigma + op.img0, P->first, T(P->tA[0], op.img0), op.nimg, P->H, P->W,
-                 0.2f, op.rev, ppt);
+        while (ppt > 1 && size_t(gx) * ((pairs + ppt - 1) / ppt) * P->B < 4 * 148) ppt >>= 1;
+        launch_k(conv_first_kernel, dim3(gx, (pairs + ppt - 1) / ppt, P->B), dim3(bd), 0, st, v, sigma, P->first,
+                 T(P->tA[0]), P->B, P->H, P->W, 0.2f, op.rev, ppt);
         break;
       }
       case K_UMMA: {
         ConvLaunch& cl = P->convs[op.conv];
         if (cl.EPI == EPI_FINAL) { cl.p.noisy = v; cl.p.x_out = x_out; cl.p.preclamp = preclamp; cl.p.active = active; }
         rc = launch_conv(cl, st);
-        break;
-      }
-      case K_POOL: {
-        const int l = op.level;
-        const int C8 = kCh[l - 1] / 8;
-        // MaxPool2d floors odd sizes; the pooled slot is (H>>1, W>>1)
-        launch_k(maxpool2_kernel, dim3((P->Wl[l] * C8 + 255) / 256, P->Hl[l], op.nimg), dim3(256), 0, st,
-                 reinterpret_cast<const uint4*>(T(P->skip[l - 1], op.img0)),
-                 reinterpret_cast<uint4*>(T(P->pooled[l], op.img0)), op.nimg, P->Hl[l - 1], P->Wl[l - 1], C8);
         break;
       }
       case K_UPS: {
@@ -1005,15 +892,15 @@ static int unet_forward_impl(UnetPlan* P, const float* v, const float* sigma, fl
         {
           const int gx = ((w + 1) * C8 + 255) / 256;
           int walk = 8;                              // long walks only while the grid still fills the machine
-          while (walk > 1 && size_t(gx) * ((h + walk) / walk) * op.nimg < 4 * size_t(g_num_sms)) walk >>= 1;
-          launch_k(upsample2x_fast_kernel, dim3(gx, (h + walk) / walk, op.nimg), dim3(256), 0, st,
-                   reinterpret_cast<const uint4*>(T(lo, op.img0)), reinterpret_cast<uint4*>(T(P->ups[l], op.img0)), h, w,
-                   C8, sy, sx, op.nimg, op.rev, (C8 == 64 ? 6 : (C8 == 32 ? 5 : (C8 == 16 ? 4 : 3))), walk);   // kCh / 8 = 8 .. 64
+          while (walk > 1 && size_t(gx) * ((h + walk) / walk) * P->B < 4 * size_t(g_num_sms)) walk >>= 1;
+          launch_k(upsample2x_fast_kernel, dim3(gx, (h + walk) / walk, P->B), dim3(256), 0, st,
+                   reinterpret_cast<const uint4*>(T(lo)), reinterpret_cast<uint4*>(T(P->ups[l])), h, w,
+                   C8, sy, sx, P->B, op.rev, (C8 == 64 ? 6 : (C8 == 32 ? 5 : (C8 == 16 ? 4 : 3))), walk);   // kCh / 8 = 8 .. 64
         }
         else
-          launch_k(upsample2x_kernel, dim3((Wo * C8 + 255) / 256, (Ho + kUpsRows - 1) / kUpsRows, op.nimg), dim3(256), 0,
-                   st, reinterpret_cast<const uint4*>(T(lo, op.img0)), reinterpret_cast<uint4*>(T(P->ups[l], op.img0)),
-                   op.nimg, h, w, Ho, Wo, C8, dy / 2, dx / 2, sy, sx);
+          launch_k(upsample2x_kernel, dim3((Wo * C8 + 255) / 256, (Ho + kUpsRows - 1) / kUpsRows, P->B), dim3(256), 0,
+                   st, reinterpret_cast<const uint4*>(T(lo)), reinterpret_cast<uint4*>(T(P->ups[l])),
+                   P->B, h, w, Ho, Wo, C8, dy / 2, dx / 2, sy, sx);
         break;
       }
     }
@@ -1031,8 +918,8 @@ int unet_forward(UnetPlan* P, const float* v, const float* sigma, float* x_out, 
 int unet_num_launches(const UnetPlan* P) { return int(P->ops.size()); }
 
 // Profiling pass: one forward with a CUDA-event pair around every launch; SYNCHRONISES the stream.
-// ms[i] = duration of launch i; kinds[i] in {0 first conv, 1 tcgen05 conv, 2 maxpool, 3 upsample};
-// ids[i] = layer index 0..26 (convs), 100+level (pools), 200+level (upsamples).
+// ms[i] = duration of launch i; kinds[i] in {0 first conv, 1 tcgen05 conv, 3 upsample};
+// ids[i] = layer index 0..26 (convs), 200+level (upsamples).
 int unet_profile(UnetPlan* P, const float* v, const float* sigma, float* x_out, cudaStream_t st, float* ms,
                  int* kinds, int* ids, int* n_inout) {
   ProfileCtx prof;

@@ -33,7 +33,6 @@ constexpr int kHalo = kTile + 2;          // halo tile edge
 constexpr int kConvThreads = 384;         // 12 warps
 constexpr int kEpiWarp0 = 4;              // first epilogue warp
 constexpr int kNumEpiWarps = 8;
-constexpr int kDbgSlots = 12;            // per-CTA stall counters (developer aid, ConvParams::dbg)
 constexpr int kNumMmaWarps = 2;           // warps 1 and 3: M-block 0 / 1 of every tile
 
 struct ConvParams {
@@ -44,10 +43,6 @@ struct ConvParams {
   int Cout;
   int sa, sb;               // ring depths: halo tiles / weight tiles (sb unused when wres)
   int wres;                 // 1: all weights of this CTA's n-tile stay resident in smem (loaded once)
-  int img0;                 // first image of this launch (micro-batching over the batch dimension)
-  int ups_fused;            // kws kernel: segment 1 is the x2 bilinear upsample (align_corners) of a half-resolution
-  float ups_sy, ups_sx;     //   tensor (tensor map 1), interpolated on the fly into the halo stages; scale (h-1)/(2h-1)
-  int direct_store;         // BN = 32: skip the lane transpose, every lane stores its own 64-byte pixel
   int sk_split, sk_cpc;     // split-K kernel (unet_conv_splitk.cuh): cluster size S and 64-channel slices per CTA
   int sk_stages;            //   pipeline stages in shared memory: min(sk_cpc, 2)
   int rev;                  // 1: walk the tiles in descending order (the plan alternates the direction layer by layer so
@@ -65,8 +60,6 @@ struct ConvParams {
   float* preclamp;          // optional [B,H,W] fp32 noisy + residual
   const uint8_t* active;    // optional [B]: 0 = leave x_out / preclamp of this image untouched (early exit, env.py:79-81)
   float slope;              // LeakyReLU negative slope (0.2)
-  long long* dbg;           // optional [grid][kDbgSlots] stall counters (clock64): MMA warp acc_empty / a_full / b_full / total,
-                            // producer a_empty / b_empty, epilogue acc_full / total
 };
 
 enum { EPI_BF16 = 0, EPI_FINAL = 1 };
@@ -87,7 +80,7 @@ __device__ __forceinline__ TileCoord decode_tile(const ConvParams& p, int tile) 
   c.tx = int(t - q * p.tiles_x); t = q;
   q = fast_div(t, p.tiles_y, p.mg_y);
   c.ty = int(t - q * p.tiles_y);
-  c.img = p.img0 + int(q);
+  c.img = int(q);
   return c;
 }
 
@@ -119,6 +112,54 @@ __device__ __forceinline__ void quad_transpose(uint4 (&v)[4], int lane) {
   for (int j = 0; j < 2; ++j) {
     const uint4 r = shfl_xor_u4(b1 ? v[j] : v[j + 2], 2);
     if (b1) v[j] = r; else v[j + 2] = r;
+  }
+}
+
+// bf16 epilogue of one 32-channel chunk (conv3x3_umma_kernel, conv3x3_pair_kernel).  r = the fp32 accumulators of
+// channels ch0 .. ch0+31 of this lane's pixel (img, y, x), bias = their biases.  The warp holds 4 rows x 8 columns of
+// pixels, lane = 8 * row + column with the first row even: lane ^ 1 is the right neighbour, lane ^ 8 the one below.
+// Writes bias + LeakyReLU as bf16 to p.out and, when p.pool_out is set, its MaxPool2d(2) (reference noise.py:23).
+// store = false computes without storing (a duplicated tile); the shuffles stay warp-uniform.
+__device__ __forceinline__ void epilogue_bf16_chunk(const ConvParams& p, const uint32_t (&r)[32], const float* bias, int ch0,
+                                                    int img, int y, int x, int lane, bool store) {
+  uint4 o[4];
+  const float2 sl2 = make_float2(p.slope, p.slope);
+#pragma unroll
+  for (int i = 0; i < 32; i += 8) {
+    const float4 ba = *reinterpret_cast<const float4*>(bias + i);
+    const float4 bb = *reinterpret_cast<const float4*>(bias + i + 4);
+    // bias + LeakyReLU on packed fp32 pairs: max(v, slope v) == LeakyReLU(v) for 0 < slope < 1
+    const float2 a0 = __fadd2_rn(make_float2(__uint_as_float(r[i]), __uint_as_float(r[i + 1])), make_float2(ba.x, ba.y));
+    const float2 a1 = __fadd2_rn(make_float2(__uint_as_float(r[i + 2]), __uint_as_float(r[i + 3])), make_float2(ba.z, ba.w));
+    const float2 a2 = __fadd2_rn(make_float2(__uint_as_float(r[i + 4]), __uint_as_float(r[i + 5])), make_float2(bb.x, bb.y));
+    const float2 a3 = __fadd2_rn(make_float2(__uint_as_float(r[i + 6]), __uint_as_float(r[i + 7])), make_float2(bb.z, bb.w));
+    const float2 m0 = __fmul2_rn(a0, sl2), m1 = __fmul2_rn(a1, sl2), m2 = __fmul2_rn(a2, sl2), m3 = __fmul2_rn(a3, sl2);
+    const float v0 = fmaxf(a0.x, m0.x), v1 = fmaxf(a0.y, m0.y), v2 = fmaxf(a1.x, m1.x), v3 = fmaxf(a1.y, m1.y);
+    const float v4 = fmaxf(a2.x, m2.x), v5 = fmaxf(a2.y, m2.y), v6 = fmaxf(a3.x, m3.x), v7 = fmaxf(a3.y, m3.y);
+    o[i / 8] = make_uint4(pack_bf16x2(v0, v1), pack_bf16x2(v2, v3), pack_bf16x2(v4, v5), pack_bf16x2(v6, v7));
+  }
+  // after the quad transpose this lane holds 16-byte chunk r4 of the pixels x0 .. x0+3 (x0 a multiple of 4) of row y
+  quad_transpose(o, lane);
+  const int r4 = lane & 3, x0 = x - r4;
+  if (store && y < p.H) {
+    uint8_t* obase = reinterpret_cast<uint8_t*>(p.out + ((size_t(img) * p.H + y) * p.W + x0) * p.Cout + ch0) + r4 * 16;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if (x0 + i < p.W) *reinterpret_cast<uint4*>(obase + size_t(i) * p.Cout * 2) = o[i];
+  }
+  if (p.pool_out) {
+    // MaxPool2d(2) on the transposed registers: the horizontal maxima need no shuffle; the row below (y even) lives in
+    // lane ^ 8.  8 SHFL; four lanes store 64 contiguous bytes per pooled pixel.
+    uint4 h0 = bf16x8_max(o[0], o[1]), h1 = bf16x8_max(o[2], o[3]);
+    h0 = bf16x8_max(h0, shfl_xor_u4(h0, 8));
+    h1 = bf16x8_max(h1, shfl_xor_u4(h1, 8));
+    const int Hp = p.H >> 1, Wp = p.W >> 1;
+    if (store && ((lane & 8) == 0) && (y >> 1) < Hp) {
+      uint8_t* pd = reinterpret_cast<uint8_t*>(p.pool_out + ((size_t(img) * Hp + (y >> 1)) * Wp + (x0 >> 1)) * p.Cout + ch0) +
+                    r4 * 16;
+      if ((x0 >> 1) < Wp) *reinterpret_cast<uint4*>(pd) = h0;
+      if ((x0 >> 1) + 1 < Wp) *reinterpret_cast<uint4*>(pd + size_t(p.Cout) * 2) = h1;
+    }
   }
 }
 
@@ -198,7 +239,6 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
     // ===================================== TMA producer =====================================
     if (lane == 0) {
       int sa = 0, pa = 0, sb = 0, pb = 0;
-      long long w_ae = 0, w_be = 0;
       if (p.wres && int(blockIdx.x) < total_tiles) {
         // n_tiles == 1 here: the layer's packed weights are one contiguous run of nchunks*9 blobs
         const uint32_t wbytes = uint32_t(nchunks) * 9 * Cfg::B_BYTES;
@@ -211,8 +251,7 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
         const TileCoord tc = decode_tile(p, tile);
         const int nt = tc.nt, tx = tc.tx, ty = tc.ty, img = tc.img;
         for (int c = 0; c < nchunks; ++c) {
-          if (p.dbg) { const long long tt = clock64(); mbar_wait(&a_empty[sa], pa ^ 1); w_ae += clock64() - tt; }
-          else mbar_wait(&a_empty[sa], pa ^ 1);
+          mbar_wait(&a_empty[sa], pa ^ 1);
           mbar_arrive_expect_tx(&a_full[sa], Cfg::A_BYTES);
           const bool seg0 = c < p.nchunks0;
           tma_load_4d(a_smem + sa * Cfg::A_STAGE, seg0 ? &tmA0 : &tmA1, &a_full[sa],
@@ -221,8 +260,7 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
           if (p.wres) continue;
           const uint8_t* wsrc = p.wpk + (size_t(c) * 9 * p.n_tiles + nt) * Cfg::B_BYTES;
           for (int tap = 0; tap < 9; ++tap) {
-            if (p.dbg) { const long long tt = clock64(); mbar_wait(&b_empty[sb], pb ^ 1); w_be += clock64() - tt; }
-            else mbar_wait(&b_empty[sb], pb ^ 1);
+            mbar_wait(&b_empty[sb], pb ^ 1);
             mbar_arrive_expect_tx(&b_full[sb], Cfg::B_BYTES);
             bulk_load_1d(b_smem + sb * Cfg::B_STAGE, wsrc + size_t(tap) * p.n_tiles * Cfg::B_BYTES, Cfg::B_BYTES,
                          &b_full[sb]);
@@ -230,7 +268,6 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
           }
         }
       }
-      if (p.dbg) { long long* d = p.dbg + size_t(blockIdx.x) * kDbgSlots; d[4] = w_ae; d[5] = w_be; }
     }
   } else if (warp == 1 || warp == 3) {
     // ===================================== MMA issuers ======================================
@@ -248,19 +285,14 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
     constexpr uint32_t b_hi = (uint32_t(8 * ROWB) >> 4) | (1u << 14) | (kLayout << 29);
     int sa = 0, pa = 0, sb = 0, pb = 0;
     int it = 0;
-    long long w_acc = 0, w_a = 0, w_b = 0;
-    const bool dbg = p.dbg != nullptr && mb == 0;
-    const long long t_begin = dbg ? clock64() : 0;
     if (p.wres && int(blockIdx.x) < total_tiles) mbar_wait(w_full, 0);
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
       const int as = it % NACC;
       const uint32_t aph = (it / NACC) & 1;
-      if (dbg) { const long long t = clock64(); mbar_wait(&acc_empty[as], aph ^ 1); w_acc += clock64() - t; }
-      else mbar_wait(&acc_empty[as], aph ^ 1);
+      mbar_wait(&acc_empty[as], aph ^ 1);
       const uint32_t d0 = tmem_base + as * (2 * BN) + mb * BN;
       for (int c = 0; c < nchunks; ++c) {
-        if (dbg) { const long long t = clock64(); mbar_wait(&a_full[sa], pa); w_a += clock64() - t; }
-        else mbar_wait(&a_full[sa], pa);
+        mbar_wait(&a_full[sa], pa);
         tc_fence_after();
         // descriptor low word: (addr >> 4) | LBO(=1) << 16 ; smem addresses are < 256 KB so no masking is needed
         const uint32_t a_lo0 = ((smem_u32(a_smem + sa * Cfg::A_STAGE) + uint32_t(mb * 8 * ROWB)) >> 4) | (1u << 16);
@@ -280,8 +312,7 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
         } else {
 #pragma unroll 1
           for (int tap = 0; tap < 9; ++tap) {
-            if (dbg) { const long long t = clock64(); mbar_wait(&b_full[sb], pb); w_b += clock64() - t; }
-            else mbar_wait(&b_full[sb], pb);
+            mbar_wait(&b_full[sb], pb);
             tc_fence_after();
             const uint32_t b_tap = (smem_u32(b_smem + sb * Cfg::B_STAGE) >> 4) | (1u << 16);
             const uint32_t a_tap = a_lo0 + uint32_t(((tap / 3) * kHalo + (tap % 3)) * ROWB) / 16;
@@ -302,10 +333,6 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
       if (elect_one()) tc_commit(&acc_full[as]);      // this M-block's accumulator complete -> epilogue
       __syncwarp();
     }
-    if (dbg && lane == 0) {
-      long long* d = p.dbg + size_t(blockIdx.x) * kDbgSlots;
-      d[0] = w_acc; d[1] = w_a; d[2] = w_b; d[3] = clock64() - t_begin;
-    }
   } else if (warp >= kEpiWarp0) {
     // ===================================== epilogue =========================================
     const int q = warp & 3;                    // TMEM lane quarter this warp may access
@@ -313,8 +340,6 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
     const int m = q * 32 + lane;               // row of the M=128 accumulator = pixel within the 16x8 block
     const int prow = m >> 3, pcol = (m & 7) + mb * 8;
     int it = 0;
-    long long w_full_acc = 0, e_ld = 0, e_math = 0, e_st = 0;
-    const long long t_begin = p.dbg ? clock64() : 0;
     for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, ++it) {
       const TileCoord tc = decode_tile(p, tile);
       const int nt = tc.nt;
@@ -326,21 +351,13 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
       // MMAs instead of sitting between the last FMA and the store)
       float noisy_px = 0.f;
       if constexpr (EPI == EPI_FINAL) { if ((y < p.H) && (x < p.W)) noisy_px = __ldg(p.noisy + pix); }
-      if (p.dbg) { const long long tt = clock64(); mbar_wait(&acc_full[as], aph); w_full_acc += clock64() - tt; }
-      else mbar_wait(&acc_full[as], aph);
+      mbar_wait(&acc_full[as], aph);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (uint32_t(q * 32) << 16) + as * (2 * BN) + mb * BN;
       if constexpr (EPI == EPI_BF16) {
-        // after the quad transpose this lane stores 16-byte chunk (lane & 3) of the 4 pixels of its lane group:
-        // pixel (4*(lane/4) + i) is (i - (lane & 3)) pixels to the right of this lane's own pixel, same image row
-        const int r4 = lane & 3;
-        uint8_t* obase = reinterpret_cast<uint8_t*>(p.out + (pix - r4) * p.Cout + nt * BN) + r4 * 16;
-        const int x0 = x - r4;
-        const float* bias_s = epi_s + nt * BN;
 #pragma unroll 1
         for (int cc = 0; cc < BN / 32; ++cc) {
           uint32_t r[32];
-          const long long e0 = p.dbg ? clock64() : 0;
           tmem_ld_32x32(taddr + cc * 32, r);
           tmem_ld_wait();
           if (cc == BN / 32 - 1) {     // accumulator stage drained: hand it back before the math and the stores
@@ -348,72 +365,7 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
             __syncwarp();
             if (lane == 0) mbar_arrive(&acc_empty[as]);
           }
-          const long long e1 = p.dbg ? clock64() : 0;
-          uint4 o[4];
-#pragma unroll
-          for (int i = 0; i < 32; i += 8) {
-            const float4 ba = *reinterpret_cast<const float4*>(bias_s + cc * 32 + i);
-            const float4 bb = *reinterpret_cast<const float4*>(bias_s + cc * 32 + i + 4);
-            // bias + LeakyReLU on packed fp32 pairs: max(v, slope v) == LeakyReLU(v) for 0 < slope < 1
-            const float2 sl2 = make_float2(p.slope, p.slope);
-            const float2 a0 = __fadd2_rn(make_float2(__uint_as_float(r[i]), __uint_as_float(r[i + 1])), make_float2(ba.x, ba.y));
-            const float2 a1 = __fadd2_rn(make_float2(__uint_as_float(r[i + 2]), __uint_as_float(r[i + 3])), make_float2(ba.z, ba.w));
-            const float2 a2 = __fadd2_rn(make_float2(__uint_as_float(r[i + 4]), __uint_as_float(r[i + 5])), make_float2(bb.x, bb.y));
-            const float2 a3 = __fadd2_rn(make_float2(__uint_as_float(r[i + 6]), __uint_as_float(r[i + 7])), make_float2(bb.z, bb.w));
-            const float2 m0 = __fmul2_rn(a0, sl2), m1 = __fmul2_rn(a1, sl2), m2 = __fmul2_rn(a2, sl2), m3 = __fmul2_rn(a3, sl2);
-            const float v0 = fmaxf(a0.x, m0.x), v1 = fmaxf(a0.y, m0.y), v2 = fmaxf(a1.x, m1.x), v3 = fmaxf(a1.y, m1.y);
-            const float v4 = fmaxf(a2.x, m2.x), v5 = fmaxf(a2.y, m2.y), v6 = fmaxf(a3.x, m3.x), v7 = fmaxf(a3.y, m3.y);
-            o[i / 8] = make_uint4(pack_bf16x2(v0, v1), pack_bf16x2(v2, v3), pack_bf16x2(v4, v5), pack_bf16x2(v6, v7));
-          }
-          const long long e2 = p.dbg ? clock64() : 0;
-          if (p.pool_out && (BN == 32 && p.direct_store)) {
-            // MaxPool2d(2) (reference noise.py:23) of the tile while it is in registers: the 2x2 window of an even
-            // (y, x) pixel lives in lanes l, l^1 (x+1) and l^8 (y+1) of this warp
-            uint4 mx[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              mx[i] = bf16x8_max(o[i], shfl_xor_u4(o[i], 1));
-              mx[i] = bf16x8_max(mx[i], shfl_xor_u4(mx[i], 8));
-            }
-            const int Hp = p.H >> 1, Wp = p.W >> 1;
-            if (((lane & 9) == 0) && (y >> 1) < Hp && (x >> 1) < Wp) {
-              uint4* pd = reinterpret_cast<uint4*>(p.pool_out + ((size_t(tc.img) * Hp + (y >> 1)) * Wp + (x >> 1)) * p.Cout +
-                                                   nt * BN + cc * 32);
-#pragma unroll
-              for (int i = 0; i < 4; ++i) pd[i] = mx[i];
-            }
-          }
-          if (BN == 32 && p.direct_store) {
-            // 32 channels = the whole 64-byte pixel in this lane: store it directly (two lanes per 128-byte line)
-            if (y < p.H && x < p.W) {
-              uint4* dst = reinterpret_cast<uint4*>(p.out + pix * p.Cout + nt * BN);
-#pragma unroll
-              for (int i = 0; i < 4; ++i) dst[i] = o[i];
-            }
-          } else {
-            quad_transpose(o, lane);
-            if (y < p.H) {
-#pragma unroll
-              for (int i = 0; i < 4; ++i)
-                if (x0 + i < p.W) *reinterpret_cast<uint4*>(obase + size_t(i) * p.Cout * 2 + cc * 64) = o[i];
-            }
-            if (p.pool_out) {
-              // MaxPool2d(2) (reference noise.py:23) on the transposed registers: this lane now holds 16-byte chunk r4 of
-              // the pixels x0 .. x0+3 (x0 a multiple of 4) of row y, so the horizontal maxima need no shuffle; the row below
-              // (y even) lives in lane ^ 8.  8 SHFL instead of 32; four lanes store 64 contiguous bytes per pooled pixel.
-              uint4 h0 = bf16x8_max(o[0], o[1]), h1 = bf16x8_max(o[2], o[3]);
-              h0 = bf16x8_max(h0, shfl_xor_u4(h0, 8));
-              h1 = bf16x8_max(h1, shfl_xor_u4(h1, 8));
-              const int Hp = p.H >> 1, Wp = p.W >> 1;
-              if (((lane & 8) == 0) && (y >> 1) < Hp) {
-                uint8_t* pd = reinterpret_cast<uint8_t*>(p.pool_out + ((size_t(tc.img) * Hp + (y >> 1)) * Wp + (x0 >> 1)) * p.Cout +
-                                                         nt * BN + cc * 32) + r4 * 16;
-                if ((x0 >> 1) < Wp) *reinterpret_cast<uint4*>(pd) = h0;
-                if ((x0 >> 1) + 1 < Wp) *reinterpret_cast<uint4*>(pd + size_t(p.Cout) * 2) = h1;
-              }
-            }
-          }
-          if (p.dbg) { const long long e3 = clock64(); e_ld += e1 - e0; e_math += e2 - e1; e_st += e3 - e2; }
+          epilogue_bf16_chunk(p, r, epi_s + nt * BN + cc * 32, nt * BN + cc * 32, tc.img, y, x, lane, true);
         }
       } else {
         static_assert(EPI == EPI_BF16 || BN == 32, "FINAL epilogue needs all 32 channels in one thread");
@@ -436,10 +388,6 @@ conv3x3_umma_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
           p.x_out[pix] = fminf(fmaxf(o, 0.f), 1.f);
         }
       }
-    }
-    if (p.dbg && warp == kEpiWarp0 && lane == 0) {
-      long long* d = p.dbg + size_t(blockIdx.x) * kDbgSlots;
-      d[6] = w_full_acc; d[7] = clock64() - t_begin; d[8] = e_ld; d[9] = e_math; d[10] = e_st;
     }
   }
 

@@ -11,19 +11,7 @@
 // neighbours x'+1, x'+2 are the next two lanes as long as the output column is one of the first 6 of its 8-wide
 // M-block window.  Tile = 16 rows x 12 columns (two M-blocks whose windows start 6 columns apart), halo 18 x 14.
 // Everything else (TMA halo ring, resident weights, two MMA-issuing warps, TMEM double buffering, fused bias /
-// LeakyReLU / max-pool / final 1x1 conv + residual + clamp) follows conv3x3_umma_kernel.
-//
-// Fused upsample (p.ups_fused, the first conv of `up4`, reference noise.py:39,46-59): the second input segment is
-// nn.Upsample(x2, bilinear, align_corners=True) of a half-resolution tensor.  Instead of materialising it (537 MB
-// written and read again at B=64, 256^2) the halo stages of that segment are interpolated on the fly: the producer
-// TMA-loads the 10 x 8 low-resolution patch under the 18 x 14 halo (zero fill outside the image), warp 2 turns it into
-// the halo tile - the halo starts at an odd row / column, so it decomposes exactly into the 2x2 output blocks of
-// upsample2x_fast_kernel, each from one 2x2 source block - and writes it in the TMA's SWIZZLE_64B layout, followed by
-// fence.proxy.async and the stage's full-barrier arrive.  Pixels outside the image are written as zeros (= the conv's
-// zero padding of the UPSAMPLED tensor).  Five warps interpolate (warp 2 and four extra warps of the UPS variant, which
-// therefore runs 512 threads at 128 registers).  Status: parity-tested (pnp_conv3x3_ups_bf16); 0.40 ms for up4's first
-// conv instead of 0.13 (upsample kernel) + 0.24, the U-Net and the sustained bench are equal within 0.5 % (with one
-// interpolating warp it was 0.83 ms), so the plan uses it only with PNP_UNET_FUSE_UPS=1.
+// LeakyReLU / max-pool) follows conv3x3_umma_kernel.
 #pragma once
 #include "unet_conv.cuh"
 
@@ -32,10 +20,6 @@ namespace pnp {
 constexpr int kKwsTileW = 12, kKwsTileH = 16;
 constexpr int kKwsHaloW = kKwsTileW + 2, kKwsHaloH = kKwsTileH + 2;
 constexpr int kKwsN = 96;
-constexpr int kKwsSrcW = kKwsHaloW / 2 + 1, kKwsSrcH = kKwsHaloH / 2 + 1;   // 8 x 10 low-resolution patch under a halo tile
-constexpr int kKwsSrcBytes = kKwsSrcW * kKwsSrcH * 64;                       // 32 channels bf16 per pixel
-constexpr int kKwsSrcStage = (kKwsSrcBytes + 1023) / 1024 * 1024;
-constexpr int kKwsSrcStages = 2;
 
 struct KwsCfg {
   static constexpr int KC = 32, ROWB = 64;
@@ -61,12 +45,7 @@ __device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&r)[16])
 
 // ConvParams is shared with conv3x3_umma_kernel; here tiles_x = ceil(W/12), tiles_y = ceil(H/16), n_tiles = 1,
 // wres = 1 (the layer's weights, at most 96 x 32 x 9 bf16 = 54 KB, always stay resident), Cout = 32.
-constexpr int kKwsUpsWarps = 5;                 // interpolating warps of the fused-upsample variant: warp 2 and warps 12..15
-constexpr int kKwsUpsThreads = kConvThreads + 4 * 32;
-
-// UPS = true: fused-upsample variant (p.ups_fused), launched with kKwsUpsThreads threads
-template <int EPI, bool UPS = false>
-__global__ void __launch_bounds__(UPS ? kKwsUpsThreads : kConvThreads, 1)
+__global__ void __launch_bounds__(kConvThreads, 1)
 conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
                    const __grid_constant__ CUtensorMap tmA1) {
   using Cfg = KwsCfg;
@@ -79,12 +58,9 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* a_smem = smem;
   uint8_t* b_smem = smem + SA * Cfg::A_STAGE;
-  uint8_t* src_smem = b_smem + ((b_region + 1023) & ~1023);                         // low-resolution patches (ups_fused)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(src_smem + (UPS ? kKwsSrcStages * kKwsSrcStage : 0));
+  uint64_t* bars = reinterpret_cast<uint64_t*>(b_smem + ((b_region + 1023) & ~1023));
   uint64_t* a_full = bars;
   uint64_t* a_empty = a_full + Cfg::MAX_RING;
-  uint64_t* src_full = a_empty + Cfg::MAX_RING;           // the plain kernel's b_full / b_empty slots
-  uint64_t* src_empty = src_full + Cfg::MAX_RING;
   uint64_t* acc_full = a_empty + 3 * Cfg::MAX_RING;       // same barrier block layout as the plain kernel
   uint64_t* acc_empty = acc_full + NACC;
   uint64_t* w_full = acc_empty + NACC;
@@ -102,7 +78,6 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
   }
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < SA; ++i) { mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], kNumMmaWarps); }
-    for (int i = 0; i < kKwsSrcStages; ++i) { mbar_init(&src_full[i], 1); mbar_init(&src_empty[i], 1); }
     for (int i = 0; i < NACC; ++i) { mbar_init(&acc_full[i], kNumMmaWarps); mbar_init(&acc_empty[i], kNumEpiWarps); }
     mbar_init(w_full, 1);
     fence_mbar_init();
@@ -111,10 +86,9 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
     tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
     tmem_relinquish();
   }
-  if (warp >= kEpiWarp0 && warp < kEpiWarp0 + kNumEpiWarps) {
+  if (warp >= kEpiWarp0) {
     const int t = threadIdx.x - kEpiWarp0 * 32;
     if (t < 32) epi_s[t] = __ldg(p.bias + t);
-    if (EPI == EPI_FINAL && t < 33) epi_s[512 + t] = t < 32 ? __ldg(p.wout + t) : __ldg(p.bout);
   }
   tc_fence_before();
   __syncthreads();
@@ -124,7 +98,7 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
   if (warp == 0) {
     // ===================================== TMA producer =====================================
     if (lane == 0 && int(blockIdx.x) < total_tiles) {
-      int sa = 0, pa = 0, ss = 0, sp = 0;
+      int sa = 0, pa = 0;
       const uint32_t wbytes = uint32_t(b_region);
       mbar_arrive_expect_tx(w_full, wbytes);
       for (uint32_t off = 0; off < wbytes; off += 3 * Cfg::B_BYTES)
@@ -134,94 +108,12 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
         const TileCoord tc = decode_tile(p, tile);
         for (int c = 0; c < nchunks; ++c) {
           const bool seg0 = c < p.nchunks0;
-          if (UPS && !seg0) {
-            // low-resolution patch under this halo tile; warp 2 interpolates it into halo stage `sa`
-            mbar_wait(&src_empty[ss], sp ^ 1);
-            mbar_arrive_expect_tx(&src_full[ss], kKwsSrcBytes);
-            tma_load_4d(src_smem + ss * kKwsSrcStage, &tmA1, &src_full[ss], (c - p.nchunks0) * KC,
-                        tc.tx * (kKwsTileW / 2) - 1, tc.ty * (kKwsTileH / 2) - 1, tc.img);
-            if (++ss == kKwsSrcStages) { ss = 0; sp ^= 1; }
-          } else {
-            mbar_wait(&a_empty[sa], pa ^ 1);
-            mbar_arrive_expect_tx(&a_full[sa], Cfg::A_BYTES);
-            tma_load_4d(a_smem + sa * Cfg::A_STAGE, seg0 ? &tmA0 : &tmA1, &a_full[sa],
-                        (seg0 ? c : c - p.nchunks0) * KC, tc.tx * kKwsTileW - 1, tc.ty * kKwsTileH - 1, tc.img);
-          }
+          mbar_wait(&a_empty[sa], pa ^ 1);
+          mbar_arrive_expect_tx(&a_full[sa], Cfg::A_BYTES);
+          tma_load_4d(a_smem + sa * Cfg::A_STAGE, seg0 ? &tmA0 : &tmA1, &a_full[sa],
+                      (seg0 ? c : c - p.nchunks0) * KC, tc.tx * kKwsTileW - 1, tc.ty * kKwsTileH - 1, tc.img);
           if (++sa == SA) { sa = 0; pa ^= 1; }
         }
-      }
-    }
-  } else if (UPS && (warp == 2 || warp >= kEpiWarp0 + kNumEpiWarps)) {
-    // ===================================== upsampling warps =================================
-    const int iw = warp == 2 ? 0 : warp - (kEpiWarp0 + kNumEpiWarps) + 1;       // 0 .. kKwsUpsWarps-1
-    int sa = 0, pa = 0, ss = 0, sp = 0;
-    for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
-      const TileCoord tc = decode_tile(p, tile);
-      // halo pixel (0, 0) has the odd image coordinates (ty * kKwsTileH - 1, tx * kKwsTileW - 1)
-      const int m0 = tc.ty * (kKwsTileH / 2) - 1, n0 = tc.tx * (kKwsTileW / 2) - 1;   // source coordinates of patch (0, 0)
-      for (int c = 0; c < nchunks; ++c) {
-        if (c >= p.nchunks0) {
-          mbar_wait(&a_empty[sa], pa ^ 1);
-          mbar_wait(&src_full[ss], sp);
-          const uint8_t* src = src_smem + ss * kKwsSrcStage;
-          uint8_t* dst = a_smem + sa * Cfg::A_STAGE;
-          constexpr int kBlocksX = kKwsHaloW / 2, kBlocksY = kKwsHaloH / 2;   // 7 x 9 blocks of 2 x 2 halo pixels
-          for (int t = iw * 32 + lane; t < kBlocksX * kBlocksY * 4; t += kKwsUpsWarps * 32) {
-            const int v = t & 3, bj = (t >> 2) % kBlocksX, bi = (t >> 2) / kBlocksX;
-            const uint4 q00 = *reinterpret_cast<const uint4*>(src + ((bi * kKwsSrcW + bj) * 64 + v * 16));
-            const uint4 q01 = *reinterpret_cast<const uint4*>(src + ((bi * kKwsSrcW + bj + 1) * 64 + v * 16));
-            const uint4 q10 = *reinterpret_cast<const uint4*>(src + (((bi + 1) * kKwsSrcW + bj) * 64 + v * 16));
-            const uint4 q11 = *reinterpret_cast<const uint4*>(src + (((bi + 1) * kKwsSrcW + bj + 1) * 64 + v * 16));
-            const int m = m0 + bi, n = n0 + bj;                                // source row / column of q00
-            float ly[2], lx[2];
-            bool oky[2], okx[2];
-#pragma unroll
-            for (int a = 0; a < 2; ++a) {
-              const int Y = 2 * m + 1 + a, X = 2 * n + 1 + a;                 // = Y0 + 2 bi + a, X0 + 2 bj + a
-              ly[a] = p.ups_sy * float(Y) - float(m);
-              lx[a] = p.ups_sx * float(X) - float(n);
-              oky[a] = Y >= 0 && Y < p.H;
-              okx[a] = X >= 0 && X < p.W;
-            }
-            const uint32_t* a00 = reinterpret_cast<const uint32_t*>(&q00);
-            const uint32_t* a01 = reinterpret_cast<const uint32_t*>(&q01);
-            const uint32_t* a10 = reinterpret_cast<const uint32_t*>(&q10);
-            const uint32_t* a11 = reinterpret_cast<const uint32_t*>(&q11);
-            uint4 res[2][2];
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const float2 f00 = make_float2(__uint_as_float(a00[k] << 16), __uint_as_float(a00[k] & 0xffff0000u));
-              const float2 f01 = make_float2(__uint_as_float(a01[k] << 16), __uint_as_float(a01[k] & 0xffff0000u));
-              const float2 f10 = make_float2(__uint_as_float(a10[k] << 16), __uint_as_float(a10[k] & 0xffff0000u));
-              const float2 f11 = make_float2(__uint_as_float(a11[k] << 16), __uint_as_float(a11[k] & 0xffff0000u));
-#pragma unroll
-              for (int j = 0; j < 2; ++j) {
-                const float2 l2 = make_float2(lx[j], lx[j]), h2 = make_float2(1.f - lx[j], 1.f - lx[j]);
-                const float2 top = __ffma2_rn(f01, l2, __fmul2_rn(f00, h2));
-                const float2 bot = __ffma2_rn(f11, l2, __fmul2_rn(f10, h2));
-#pragma unroll
-                for (int i = 0; i < 2; ++i) {
-                  const float2 ll = make_float2(ly[i], ly[i]), hh = make_float2(1.f - ly[i], 1.f - ly[i]);
-                  const float2 r = __ffma2_rn(bot, ll, __fmul2_rn(top, hh));
-                  reinterpret_cast<uint32_t*>(&res[i][j])[k] = pack_bf16x2(r.x, r.y);
-                }
-              }
-            }
-#pragma unroll
-            for (int i = 0; i < 2; ++i)
-#pragma unroll
-              for (int j = 0; j < 2; ++j) {
-                const uint32_t off = uint32_t(((2 * bi + i) * kKwsHaloW + 2 * bj + j) * 64 + v * 16);
-                const uint32_t phys = off ^ (((off >> 7) & 3) << 4);          // SWIZZLE_64B, stage base 1024-aligned
-                *reinterpret_cast<uint4*>(dst + phys) = (oky[i] && okx[j]) ? res[i][j] : make_uint4(0, 0, 0, 0);
-              }
-          }
-          fence_proxy_async_smem();            // generic-proxy writes -> visible to the tensor core (async proxy)
-          asm volatile("bar.sync 1, %0;" ::"n"(kKwsUpsWarps * 32) : "memory");     // all interpolating warps are done
-          if (iw == 0 && lane == 0) { mbar_arrive(&a_full[sa]); mbar_arrive(&src_empty[ss]); }
-          if (++ss == kKwsSrcStages) { ss = 0; sp ^= 1; }
-        }
-        if (++sa == SA) { sa = 0; pa ^= 1; }
       }
     }
   } else if (warp == 1 || warp == 3) {
@@ -261,7 +153,7 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
       if (elect_one()) tc_commit(&acc_full[as]);
       __syncwarp();
     }
-  } else if (warp >= kEpiWarp0 && warp < kEpiWarp0 + kNumEpiWarps) {
+  } else if (warp >= kEpiWarp0) {
     // ===================================== epilogue =========================================
     const int q = warp & 3;
     const int mb = (warp - kEpiWarp0) >> 2;
@@ -275,13 +167,10 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
       const uint32_t aph = (it / NACC) & 1;
       const int y = tc.ty * kKwsTileH + yl, x = tc.tx * kKwsTileW + mb * 6 + i8;
       const size_t pix = (size_t(tc.img) * p.H + y) * p.W + x;
-      float noisy_px = 0.f;                    // FINAL: fetched before the wait so that its latency overlaps the MMAs
-      if constexpr (EPI != EPI_BF16) { if (i8 < 6 && y < p.H && x < p.W) noisy_px = __ldg(p.noisy + pix); }
       mbar_wait(&acc_full[as], aph);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (uint32_t(q * 32) << 16) + as * Cfg::ACC_COLS + mb * kKwsN;
       uint4 o[4];
-      float facc = 0.f;
 #pragma unroll
       for (int half = 0; half < 2; ++half) {
         uint32_t r0[16], r1[16], r2[16];
@@ -304,47 +193,34 @@ conv3x3_kws_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0,
           float v = (__uint_as_float(r0[c]) + p1) + p2 + epi_s[half * 16 + c];
           s[c] = v > 0.f ? v : v * p.slope;
         }
-        if constexpr (EPI == EPI_BF16) {
 #pragma unroll
-          for (int g = 0; g < 2; ++g)
-            o[half * 2 + g] = make_uint4(pack_bf16x2(s[g * 8], s[g * 8 + 1]), pack_bf16x2(s[g * 8 + 2], s[g * 8 + 3]),
-                                         pack_bf16x2(s[g * 8 + 4], s[g * 8 + 5]), pack_bf16x2(s[g * 8 + 6], s[g * 8 + 7]));
-        } else {
+        for (int g = 0; g < 2; ++g)
+          o[half * 2 + g] = make_uint4(pack_bf16x2(s[g * 8], s[g * 8 + 1]), pack_bf16x2(s[g * 8 + 2], s[g * 8 + 3]),
+                                       pack_bf16x2(s[g * 8 + 4], s[g * 8 + 5]), pack_bf16x2(s[g * 8 + 6], s[g * 8 + 7]));
+      }
+      if (p.pool_out) {
+        // 2x2 max-pool partners: x+1 = lane^1 (x and i8 have the same parity, i8+1 <= 5 for even i8 < 6), y+1 = lane^8
+        uint4 mx[4];
 #pragma unroll
-          for (int c = 0; c < 16; ++c) facc = fmaf(s[c], epi_s[512 + half * 16 + c], facc);
+        for (int g = 0; g < 4; ++g) {
+          mx[g] = bf16x8_max(o[g], shfl_xor_u4(o[g], 1));
+          mx[g] = bf16x8_max(mx[g], shfl_xor_u4(mx[g], 8));
+        }
+        const int Hp = p.H >> 1, Wp = p.W >> 1;
+        if (((lane & 9) == 0) && i8 < 6 && (y >> 1) < Hp && (x >> 1) < Wp) {
+          uint4* pd = reinterpret_cast<uint4*>(p.pool_out + ((size_t(tc.img) * Hp + (y >> 1)) * Wp + (x >> 1)) * 32);
+#pragma unroll
+          for (int g = 0; g < 4; ++g) pd[g] = mx[g];
         }
       }
-      if constexpr (EPI == EPI_BF16) {
-        if (p.pool_out) {
-          // 2x2 max-pool partners: x+1 = lane^1 (x and i8 have the same parity, i8+1 <= 5 for even i8 < 6), y+1 = lane^8
-          uint4 mx[4];
+      quad_transpose(o, lane);
+      // lane 4g+r now holds 16-byte chunk r of the pixels of lanes 4g .. 4g+3
+      if (y < p.H) {
+        uint8_t* obase = reinterpret_cast<uint8_t*>(p.out + (pix - r4) * 32) + r4 * 16;
+        const int x0 = x - r4, i0 = i8 - r4;
 #pragma unroll
-          for (int g = 0; g < 4; ++g) {
-            mx[g] = bf16x8_max(o[g], shfl_xor_u4(o[g], 1));
-            mx[g] = bf16x8_max(mx[g], shfl_xor_u4(mx[g], 8));
-          }
-          const int Hp = p.H >> 1, Wp = p.W >> 1;
-          if (((lane & 9) == 0) && i8 < 6 && (y >> 1) < Hp && (x >> 1) < Wp) {
-            uint4* pd = reinterpret_cast<uint4*>(p.pool_out + ((size_t(tc.img) * Hp + (y >> 1)) * Wp + (x >> 1)) * 32);
-#pragma unroll
-            for (int g = 0; g < 4; ++g) pd[g] = mx[g];
-          }
-        }
-        quad_transpose(o, lane);
-        // lane 4g+r now holds 16-byte chunk r of the pixels of lanes 4g .. 4g+3
-        if (y < p.H) {
-          uint8_t* obase = reinterpret_cast<uint8_t*>(p.out + (pix - r4) * 32) + r4 * 16;
-          const int x0 = x - r4, i0 = i8 - r4;
-#pragma unroll
-          for (int j = 0; j < 4; ++j)
-            if (i0 + j < 6 && x0 + j < p.W) *reinterpret_cast<uint4*>(obase + size_t(j) * 64) = o[j];
-        }
-      } else {
-        if (i8 < 6 && y < p.H && x < p.W) {
-          const float ov = noisy_px + (facc + epi_s[512 + 32]);
-          if (p.preclamp) p.preclamp[pix] = ov;
-          p.x_out[pix] = fminf(fmaxf(ov, 0.f), 1.f);
-        }
+        for (int j = 0; j < 4; ++j)
+          if (i0 + j < 6 && x0 + j < p.W) *reinterpret_cast<uint4*>(obase + size_t(j) * 64) = o[j];
       }
     }
   }

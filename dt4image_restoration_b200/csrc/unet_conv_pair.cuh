@@ -14,7 +14,8 @@
 //     completions with remote arrives - 2.70 ms per U-Net at BN=128 instead of 2.67 single-CTA);
 //   * the peer's epilogue warps hand their accumulator stage back with a remote arrive on the leader's acc_empty.
 // Accumulators: every CTA's TMEM holds its own 128 rows x BN columns per M-block, double buffered, exactly as before.
-// Opt-in (PNP_CONV_PAIR=1) for layers with the plain bf16 epilogue and BN in {64, 128}.
+// Used for the layers with the plain bf16 epilogue and BN in {64, 128} whose weights do not stay resident in a single
+// CTA (build_conv in unet.cu).
 #pragma once
 #include <cooperative_groups.h>
 #include "unet_conv.cuh"
@@ -173,7 +174,7 @@ conv3x3_pair_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
     if (dup) pt = pixel_tiles - 1;
     tx = pt % p.tiles_x; pt /= p.tiles_x;
     ty = pt % p.tiles_y;
-    img = p.img0 + pt / p.tiles_y;
+    img = pt / p.tiles_y;
   };
 
   if (warp == 0) {
@@ -280,14 +281,9 @@ conv3x3_pair_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
       const int as = it % NACC;
       const uint32_t aph = (it / NACC) & 1;
       const int y = ty * kTile + prow, x = tx * kTile + pcol;
-      const size_t pix = (size_t(img) * p.H + y) * p.W + x;
       mbar_wait(&acc_full[as], aph);
       tc_fence_after();
       const uint32_t taddr = tmem_base + (uint32_t(q * 32) << 16) + as * (2 * BN) + mb * BN;
-      const int r4 = lane & 3;
-      uint8_t* obase = reinterpret_cast<uint8_t*>(p.out + (pix - r4) * p.Cout + nt * BN) + r4 * 16;
-      const int x0 = x - r4;
-      const float* bias_s = epi_s + nt * BN;
 #pragma unroll 1
       for (int cc = 0; cc < BN / 32; ++cc) {
         uint32_t r[32];
@@ -298,43 +294,7 @@ conv3x3_pair_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tmA0
           __syncwarp();
           if (lane == 0) { if (leader) mbar_arrive(&acc_empty[as]); else mbar_arrive_remote(&acc_empty[as], 0); }
         }
-        uint4 o[4];
-#pragma unroll
-        for (int i = 0; i < 32; i += 8) {
-          const float4 ba = *reinterpret_cast<const float4*>(bias_s + cc * 32 + i);
-          const float4 bb = *reinterpret_cast<const float4*>(bias_s + cc * 32 + i + 4);
-          // bias + LeakyReLU on packed fp32 pairs: max(v, slope v) == LeakyReLU(v) for 0 < slope < 1
-          const float2 sl2 = make_float2(p.slope, p.slope);
-          const float2 a0 = __fadd2_rn(make_float2(__uint_as_float(r[i]), __uint_as_float(r[i + 1])), make_float2(ba.x, ba.y));
-          const float2 a1 = __fadd2_rn(make_float2(__uint_as_float(r[i + 2]), __uint_as_float(r[i + 3])), make_float2(ba.z, ba.w));
-          const float2 a2 = __fadd2_rn(make_float2(__uint_as_float(r[i + 4]), __uint_as_float(r[i + 5])), make_float2(bb.x, bb.y));
-          const float2 a3 = __fadd2_rn(make_float2(__uint_as_float(r[i + 6]), __uint_as_float(r[i + 7])), make_float2(bb.z, bb.w));
-          const float2 m0 = __fmul2_rn(a0, sl2), m1 = __fmul2_rn(a1, sl2), m2 = __fmul2_rn(a2, sl2), m3 = __fmul2_rn(a3, sl2);
-          const float v0 = fmaxf(a0.x, m0.x), v1 = fmaxf(a0.y, m0.y), v2 = fmaxf(a1.x, m1.x), v3 = fmaxf(a1.y, m1.y);
-          const float v4 = fmaxf(a2.x, m2.x), v5 = fmaxf(a2.y, m2.y), v6 = fmaxf(a3.x, m3.x), v7 = fmaxf(a3.y, m3.y);
-          o[i / 8] = make_uint4(pack_bf16x2(v0, v1), pack_bf16x2(v2, v3), pack_bf16x2(v4, v5), pack_bf16x2(v6, v7));
-        }
-        if (p.pool_out) {
-          uint4 mx[4];
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            mx[i] = bf16x8_max(o[i], shfl_xor_u4(o[i], 1));
-            mx[i] = bf16x8_max(mx[i], shfl_xor_u4(mx[i], 8));
-          }
-          const int Hp = p.H >> 1, Wp = p.W >> 1;
-          if (!dup && ((lane & 9) == 0) && (y >> 1) < Hp && (x >> 1) < Wp) {
-            uint4* pd = reinterpret_cast<uint4*>(p.pool_out + ((size_t(img) * Hp + (y >> 1)) * Wp + (x >> 1)) * p.Cout +
-                                                 nt * BN + cc * 32);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) pd[i] = mx[i];
-          }
-        }
-        quad_transpose(o, lane);
-        if (!dup && y < p.H) {
-#pragma unroll
-          for (int i = 0; i < 4; ++i)
-            if (x0 + i < p.W) *reinterpret_cast<uint4*>(obase + size_t(i) * p.Cout * 2 + cc * 64) = o[i];
-        }
+        epilogue_bf16_chunk(p, r, epi_s + nt * BN + cc * 32, nt * BN + cc * 32, img, y, x, lane, !dup);
       }
     }
   }

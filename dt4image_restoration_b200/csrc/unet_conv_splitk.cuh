@@ -76,7 +76,7 @@ conv3x3_splitk_kernel(const ConvParams p, const __grid_constant__ CUtensorMap tm
   const int ns = unit % n_sub; unit /= n_sub;
   const int tx = unit % p.tiles_x; unit /= p.tiles_x;
   const int ty = unit % p.tiles_y;
-  const int img = p.img0 + unit / p.tiles_y;
+  const int img = unit / p.tiles_y;
 
   grid_dep_launch();
   if (warp == 0 && lane == 0) { tma_prefetch_desc(&tmA0); tma_prefetch_desc(&tmA1); }

@@ -195,19 +195,14 @@ def prox_dual(x, u, y0, mask, mu, want_v: bool = True, out=None, workspace=None)
     return z, un, v
 
 
-def conv3x3_bf16(in0: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, in1: torch.Tensor | None = None,
-                 in1_half_res: bool = False):
-    """NHWC bf16 3x3 conv + bias + LeakyReLU(0.2) on the tensor cores; ``in1`` = second concat segment.
-    ``in1_half_res``: ``in1`` is ``[B,H/2,W/2,C1]`` and its x2 bilinear upsample (align_corners=True) is the segment
-    (the fused first conv of an ``up`` block, reference noise.py:39,59)."""
+def conv3x3_bf16(in0: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, in1: torch.Tensor | None = None):
+    """NHWC bf16 3x3 conv + bias + LeakyReLU(0.2) on the tensor cores; ``in1`` = second concat segment."""
     in0 = _req(in0, torch.bfloat16, "in0")
     B, H, W, C0 = in0.shape
     C1 = 0
     if in1 is not None:
         in1 = _req(in1, torch.bfloat16, "in1")
         C1 = in1.shape[-1]
-        if in1_half_res and tuple(in1.shape[1:3]) != (H // 2, W // 2):
-            raise ValueError(f"half-resolution segment must be {(H // 2, W // 2)}, got {tuple(in1.shape[1:3])}")
     weight = _req(weight, torch.float32, "weight")
     bias = _req(bias, torch.float32, "bias")
     Cout = weight.shape[0]
@@ -215,10 +210,9 @@ def conv3x3_bf16(in0: torch.Tensor, weight: torch.Tensor, bias: torch.Tensor, in
     l = _lib.lib()
     out = torch.empty(B, H, W, Cout, dtype=torch.bfloat16, device=in0.device)
     scratch = aligned_empty(l.pnp_conv3x3_packed_bytes(C0 + C1, Cout), in0.device)
-    fn = l.pnp_conv3x3_ups_bf16 if in1_half_res else l.pnp_conv3x3_bf16
-    check(fn(in0.data_ptr(), C0, in1.data_ptr() if in1 is not None else None, C1, weight.data_ptr(),
-             bias.data_ptr(), out.data_ptr(), scratch.data_ptr(), B, H, W, Cout, _lib.stream_ptr()),
-          "pnp_conv3x3_ups_bf16" if in1_half_res else "pnp_conv3x3_bf16")
+    check(l.pnp_conv3x3_bf16(in0.data_ptr(), C0, in1.data_ptr() if in1 is not None else None, C1, weight.data_ptr(),
+                             bias.data_ptr(), out.data_ptr(), scratch.data_ptr(), B, H, W, Cout, _lib.stream_ptr()),
+          "pnp_conv3x3_bf16")
     return out
 
 

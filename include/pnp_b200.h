@@ -113,8 +113,8 @@ void pnp_unet_plan_destroy(pnp_unet_plan* plan);
 int pnp_unet_forward(pnp_unet_plan* plan, const float* v, const float* sigma, float* x_out, float* preclamp,
                      void* stream);
 /* Profiling pass (SYNCHRONISES the stream): one forward with a CUDA-event pair around every launch.  On return
- * ms[i], kinds[i] (0 first conv, 1 tcgen05 conv, 2 maxpool, 3 upsample) and ids[i] (conv: layer 0..26 in
- * state_dict order; pool: 100+level; upsample: 200+level) describe launch i; *n_inout = capacity in, count out. */
+ * ms[i], kinds[i] (0 first conv, 1 tcgen05 conv, 3 upsample) and ids[i] (conv: layer 0..26 in state_dict order;
+ * upsample: 200+level) describe launch i; *n_inout = capacity in, count out. */
 int pnp_unet_profile(pnp_unet_plan* plan, const float* v, const float* sigma, float* x_out, void* stream, float* ms,
                      int* kinds, int* ids, int* n_inout);
 /* Kernel launches one pnp_unet_forward issues for this plan (all micro-batches). */
@@ -138,11 +138,6 @@ int pnp_unet_plan_tensor(const pnp_unet_plan* plan, const char* name, size_t* by
 size_t pnp_conv3x3_packed_bytes(int Cin, int Cout);
 int pnp_conv3x3_bf16(const void* in0, int C0, const void* in1, int C1, const float* weights, const float* bias,
                      void* out, void* scratch, int B, int H, int W, int Cout, void* stream);
-/* The first conv of an `up` block with the upsample fused (noise.py:39,46-59,75-89): in1_half is the [B,H/2,W/2,C1]
- * tensor BEFORE nn.Upsample(x2, bilinear, align_corners=True); out = LeakyReLU(conv3x3(cat[in0, upsample(in1_half)])).
- * Supported where the kw-stacked kernel applies: Cout = 32, C0 and C1 multiples of 32 with 64 <= C0+C1 <= 96, even H, W. */
-int pnp_conv3x3_ups_bf16(const void* in0, int C0, const void* in1_half, int C1, const float* weights, const float* bias,
-                         void* out, void* scratch, int B, int H, int W, int Cout, void* stream);
 
 /* The policy that produces the actions (SURVEY 8f row 1; reference transformer/decision_transformer.py:212-275 as driven by
  * evaluation/eval.py:147-186): ONE kernel per rollout iteration computes the action head at the newest observation token and,

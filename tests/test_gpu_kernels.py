@@ -296,13 +296,10 @@ def test_unet_layerwise_against_oracle(B, H, W, kind, splitk, splitk_mode):
     out, pre = den(v.to(DEV), sigma.to(DEV), preclamp=True)
     plan = den.plan(B, H, W)
     # layers whose buffers are not recycled by later layers
-    for name in ["inc.conv-2", "down1.pooled", "down1.conv-2", "down2.conv-2", "down3.conv-2", "down4.conv-0",
-                 "down4.conv-1", "down4.conv-2", "up1.upsampled", "up2.upsampled", "up3.upsampled", "up4.upsampled"]:
-        try:
-            got = plan.activation(name).float().cpu().permute(0, 3, 1, 2)
-        except KeyError:
-            assert name == "up4.upsampled"        # fused into up4's first conv: never materialised
-            continue
+    for name in ["inc.conv-2", "down1.pooled", "down1.conv-2", "down2.pooled", "down2.conv-2", "down3.pooled", "down3.conv-2",
+                 "down4.pooled", "down4.conv-0", "down4.conv-1", "down4.conv-2", "up1.upsampled", "up2.upsampled",
+                 "up3.upsampled", "up4.upsampled"]:
+        got = plan.activation(name).float().cpu().permute(0, 3, 1, 2)
         ref = taps[name]
         rel = (got - ref).norm() / (ref.norm() + 1e-12)
         assert rel < 2e-2, f"{name}: relative L2 error {rel.item():.3e}"
@@ -366,26 +363,6 @@ def test_unet_golden_odd_sizes(golden_dir):
         _, pre = den(inp[:, :1].to(DEV), sig.to(DEV), preclamp=True)
         r_ref, r_got = ref - inp[:, :1], pre.cpu() - inp[:, :1]
         assert (r_got - r_ref).norm() / r_ref.norm() < 3e-2
-
-
-@pytest.mark.parametrize("B,H,W,C0,C1", [(2, 32, 24, 32, 64), (1, 64, 64, 32, 32), (3, 20, 36, 32, 64), (1, 256, 256, 32, 64),
-                                         (2, 16, 12, 64, 32)])
-def test_conv3x3_with_fused_upsample_matches_reference(B, H, W, C0, C1):
-    """First conv of an `up` block with nn.Upsample(x2, bilinear, align_corners=True) fused into the operand producer
-    (unet_conv_kws.cuh): conv(cat[skip, upsample(lo)]) vs the fp32 reference on bf16-rounded operands."""
-    g = torch.Generator().manual_seed(H * 7 + W + C1)
-    in0 = torch.randn(B, H, W, C0, generator=g).to(torch.bfloat16)
-    lo = torch.randn(B, H // 2, W // 2, C1, generator=g).to(torch.bfloat16)
-    w = torch.randn(32, C0 + C1, 3, 3, generator=g) * (2.0 / (9 * (C0 + C1))) ** 0.5
-    b = torch.randn(32, generator=g) * 0.1
-    up = F.interpolate(lo.float().permute(0, 3, 1, 2), scale_factor=2, mode="bilinear", align_corners=True)
-    up = bf16r(up).permute(0, 2, 3, 1)                       # the unfused path rounds the upsampled tensor to bf16 too
-    ref = conv_ref(in0, up.to(torch.bfloat16), w, b)
-    got = ops.conv3x3_bf16(in0.to(DEV), w.to(DEV), b.to(DEV), lo.to(DEV), in1_half_res=True).float().cpu()
-    err = (got - ref).abs()
-    # bf16 output rounding + accumulation order + 1-ulp differences of the bf16-rounded interpolated operand
-    tol = 1e-2 * ref.abs() + 4e-3
-    assert bool((err <= tol).all()), f"max err {err.max().item()} at {np.unravel_index(err.argmax(), err.shape)}"
 
 
 @pytest.mark.parametrize("pair", ["0", "1"])

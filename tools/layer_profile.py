@@ -21,7 +21,6 @@ blocks = [("inc", [(2, 32), (32, 32), (32, 32)], 0), ("down1", [(32, 64), (64, 6
 info = {}
 order = []
 for bi, (bn, convs, lvl) in enumerate(blocks):
-    if bn.startswith("down"): info[100 + lvl] = (f"{bn}.pool", None); order.append(100 + lvl)
     if bn.startswith("up"): info[200 + lvl] = (f"{bn}.upsample", None); order.append(200 + lvl)
     for i, (ci, co) in enumerate(convs):
         info[bi * 3 + i] = (f"{bn}.conv{i} {ci}->{co} @{S >> lvl}", (ci, co, lvl)); order.append(bi * 3 + i)
