@@ -28,6 +28,8 @@ SIGNATURES = {
     "pnp_psnr": (c_int, [c_void_p, c_void_p, c_ll, c_void_p, c_int, c_int, c_void_p]),
     "pnp_psnr_allgather": (c_int, [c_void_p, c_void_p, c_ll, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int,
                                    c_void_p, C.c_uint, C.c_uint, c_void_p, c_int, c_int, c_void_p]),
+    "pnp_ssim_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
+    "pnp_ssim": (c_int, [c_void_p, c_void_p, c_ll, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "pnp_fft2c": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "pnp_residual_real": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_void_p]),
     "pnp_prox_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),

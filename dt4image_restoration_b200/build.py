@@ -17,7 +17,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libpnp_b200.so")
 STAMP = os.path.join(CSRC, ".build_stamp")
-SOURCES = ["api.cu", "psnr.cu", "fftprox.cu", "unet.cu", "policy.cu", "policy_observe.cu"]
+SOURCES = ["api.cu", "psnr.cu", "ssim.cu", "fftprox.cu", "unet.cu", "policy.cu", "policy_observe.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "-Xptxas", "-v",

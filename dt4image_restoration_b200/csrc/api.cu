@@ -102,6 +102,18 @@ int pnp_psnr_allgather(const float* x, const float* gt, long long gt_batch_strid
                                          cudaStream_t(stream)), "pnp_psnr_allgather");
 }
 
+size_t pnp_ssim_workspace_bytes(int B, int H, int W) { return ssim_workspace_bytes(B, H, W); }
+
+int pnp_ssim(const float* x, const float* gt, long long gt_batch_stride, float* out, void* workspace, int B, int H, int W,
+             void* stream) {
+  REQUIRE_INIT();
+  if (!x || !gt || !out || !workspace) { set_error("pnp_ssim: null pointer"); return -1; }
+  if (B <= 0) { set_error("pnp_ssim: need B > 0"); return -1; }
+  if (H < 11 || W < 11) { set_error("pnp_ssim: H and W must be at least 11 (11x11 window, valid filtering)"); return -2; }
+  if (reinterpret_cast<uintptr_t>(workspace) & 15) { set_error("pnp_ssim: workspace must be 16-byte aligned"); return -1; }
+  return fail_cuda(ssim_launch(x, gt, gt_batch_stride, out, workspace, B, H, W, cudaStream_t(stream)), "pnp_ssim");
+}
+
 int pnp_fft2c(const void* src, void* dst, int B, int H, int W, int inverse, void* stream) {
   REQUIRE_INIT();
   if (!src || !dst || B <= 0) { set_error("pnp_fft2c: bad argument"); return -1; }

@@ -17,6 +17,11 @@ int psnr_allgather_launch(const float* x, const float* gt, long long gt_bstride,
                           unsigned int* local_count, unsigned int count_target, unsigned int flag_target, int* err,
                           int B, int HW, cudaStream_t st);
 
+// ssim.cu
+size_t ssim_workspace_bytes(int B, int H, int W);
+int ssim_launch(const float* x, const float* gt, long long gt_bstride, float* out, void* workspace, int B, int H, int W,
+                cudaStream_t st);
+
 // fftprox.cu
 void init_fft_tables();
 int fft_shape_supported(int H, int W);       // radix kernels + prepared path: powers of two in 32..512

@@ -35,6 +35,8 @@ class PnPEngine:
         self.sigma = self.actions[0]
         self.mu = self.actions[1]
         self.reward = torch.zeros(B, dtype=torch.float32, device=dev)
+        self.ssim_out = torch.zeros(B, dtype=torch.float32, device=dev)
+        self.ssim_work = ops.aligned_empty(_lib.lib().pnp_ssim_workspace_bytes(B, H, W), dev, align=16)
         self.work = torch.empty(_lib.lib().pnp_prox_workspace_bytes(B, H, W), dtype=torch.uint8, device=dev)
         # shapes with a prepared single-launch prox kernel keep transposed, sign-folded copies of y0 / mask
         self.prepared = bool(_lib.lib().pnp_prox_prepared_supported(H, W))
@@ -137,6 +139,13 @@ class PnPEngine:
         check(_lib.lib().pnp_psnr(self.x.data_ptr(), self.gt.data_ptr(), self.H * self.W, self.reward.data_ptr(), self.B,
                                   self.H * self.W, _lib.stream_ptr()), "pnp_psnr")
         return self.reward
+
+    def ssim(self) -> torch.Tensor:
+        """Per-image SSIM of the current ``x`` against ``gt`` (see ``ops.ssim``), on the device; allocation-free, so it can
+        be captured in a CUDA graph.  Returns the same ``[B]`` buffer on every call."""
+        check(_lib.lib().pnp_ssim(self.x.data_ptr(), self.gt.data_ptr(), self.H * self.W, self.ssim_out.data_ptr(),
+                                  self.ssim_work.data_ptr(), self.B, self.H, self.W, _lib.stream_ptr()), "pnp_ssim")
+        return self.ssim_out
 
     def run(self, sigmas, mus, n_iters: int | None = None):
         """Fixed-schedule trajectory: ``sigmas[k]``, ``mus[k]`` scalars or ``[B]`` per iteration."""

@@ -282,6 +282,15 @@ class PnPEnv:
         dev = x.device if x.is_cuda else (gt.device if gt.is_cuda else torch.device('cuda'))
         return ops.psnr(x.to(dev), gt.to(dev)).reshape(N, 1).cpu()
 
+    @staticmethod
+    def compute_ssim(x, gt):
+        """SSIM per image (``ops.ssim``) shaped like ``compute_reward``: a CPU ``[N,1]`` tensor computed on the device."""
+        x = x.detach()
+        N = x.shape[0]
+        gt = gt.detach().reshape(-1, *x.shape[1:]) if gt.numel() != x[0].numel() else gt.detach()
+        dev = x.device if x.is_cuda else (gt.device if gt.is_cuda else torch.device('cuda'))
+        return ops.ssim(x.to(dev), gt.to(dev)).reshape(N, 1).cpu()
+
 
 def torch_psnr(output, gt):
     """env.py:120-125 on the device; returns ``[N,1]`` on the inputs' device."""

@@ -49,6 +49,29 @@ def psnr(x: torch.Tensor, gt: torch.Tensor) -> torch.Tensor:
     return out
 
 
+def ssim(x: torch.Tensor, gt: torch.Tensor) -> torch.Tensor:
+    """SSIM per image (Gaussian 11x11 window, sigma 1.5, valid filtering; see ``pnp_ssim`` in include/pnp_b200.h):
+    ``[N,...,H,W]`` vs ``[N,...,H,W]`` (or one shared ``[H,W]`` gt) -> fp32 ``[N]`` on the device.  ``x`` is clamped to
+    [0, 1], ``gt`` is not."""
+    if x.is_complex():
+        x = x.real
+    N, (H, W) = x.shape[0], x.shape[-2:]
+    x = _req(x.reshape(N, H * W).float(), torch.float32, "x")
+    gt = _req(gt.float(), torch.float32, "gt")
+    if gt.numel() == N * H * W:
+        stride = H * W
+    elif gt.numel() == H * W:
+        stride = 0
+    else:
+        raise RuntimeError(f"ssim: gt has {gt.numel()} elements, expected {N * H * W} or {H * W}")
+    l = _lib.lib()
+    out = torch.empty(N, dtype=torch.float32, device=x.device)
+    work = aligned_empty(max(int(l.pnp_ssim_workspace_bytes(N, H, W)), 16), x.device, align=16)
+    check(l.pnp_ssim(x.data_ptr(), gt.data_ptr(), stride, out.data_ptr(), work.data_ptr(), N, H, W, _lib.stream_ptr()),
+          "pnp_ssim")
+    return out
+
+
 def fft2c(x: torch.Tensor, inverse: bool = False) -> torch.Tensor:
     """Centred orthonormal 2-D (i)FFT over the last two dims (transformations.py:6-19)."""
     if not x.is_complex():

@@ -48,6 +48,20 @@ int pnp_psnr_allgather(const float* x, const float* gt, long long gt_batch_strid
                        int flag_word, unsigned int* local_count, unsigned int count_target, unsigned int flag_target,
                        int* err_flag, int B, int HW, void* stream);
 
+/* Image-quality metric next to the PSNR reward: SSIM per image.  The reference ships `calculate_ssim`
+ * (evaluation/utils/transformations.py:61-95) but never calls it; this is the standard SSIM of Wang et al. (2004) in the
+ * form of pytorch-msssim / BasicSR, and parity with that function is not claimed:
+ *   X = clamp(x[b], 0, 1), Y = gt[b] (not clamped, as in pnp_psnr);  g[k] = exp(-(k-5)^2 / 4.5) / sum, k = 0..10, applied
+ *   separably with VALID filtering ((H-10) x (W-10) map, no padding);  mu_x = g*X, mu_y = g*Y, s_xx = g*(X.X) - mu_x^2,
+ *   s_yy = g*(Y.Y) - mu_y^2, s_xy = g*(X.Y) - mu_x mu_y (population moments);  C1 = 0.01^2, C2 = 0.03^2 (L = 1);
+ *   out[b] = mean of ((2 mu_x mu_y + C1)(2 s_xy + C2)) / ((mu_x^2 + mu_y^2 + C1)(s_xx + s_yy + C2)).
+ * gt_batch_stride = H*W, or 0 to share one gt.  out: fp32 [B].  H, W >= 11, no upper limit.  workspace:
+ * pnp_ssim_workspace_bytes(B,H,W) bytes, 16-byte aligned.  The value of an image is bitwise the same on every call and at
+ * any position of any batch (the summation order depends on H and W only). */
+size_t pnp_ssim_workspace_bytes(int B, int H, int W);
+int pnp_ssim(const float* x, const float* gt, long long gt_batch_stride, float* out, void* workspace, int B, int H, int W,
+             void* stream);
+
 /* Centred orthonormal 2-D FFT / inverse FFT: replaces fft / ifft (evaluation/utils/transformations.py:6-12,
  * 14-19).  H, W in 2..1024: radix kernels for powers of two in 32..512, a dense-DFT path for every other size (torch.fft
  * is mixed-radix, so the reference accepts them).  dst may alias src. */
