@@ -122,6 +122,55 @@ int pnp_fft2c(const void* src, void* dst, int B, int H, int W, int inverse, void
                                  cudaStream_t(stream)), "pnp_fft2c");
 }
 
+// Byte ranges [lo, hi) of the buffers of pnp_simulate_measurements, for the overlap test.
+static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
+  const uintptr_t pa = reinterpret_cast<uintptr_t>(a), pb = reinterpret_cast<uintptr_t>(b);
+  return a && b && pa < pb + nb && pb < pa + na;
+}
+
+// The argument checks of the two simulator entry points come before REQUIRE_INIT, so a bad call is refused with its own
+// message whether or not pnp_init has run.
+int pnp_simulate_measurements(const float* gt, long long gt_batch_stride, const uint8_t* mask, long long mask_batch_stride,
+                              const float* sigma_n, int sigma_stride, const unsigned long long* seeds, void* y0_out,
+                              void* x0_out, void* aty0_out, int B, int H, int W, void* stream) {
+  if (!gt || !mask || !sigma_n || !seeds || !y0_out || !x0_out) {
+    set_error("pnp_simulate_measurements: null pointer");
+    return -1;
+  }
+  if (B <= 0 || gt_batch_stride < 0 || mask_batch_stride < 0 || sigma_stride < 0) {
+    set_error("pnp_simulate_measurements: need B > 0 and non-negative strides");
+    return -1;
+  }
+  if (!fft_any_shape_supported(H, W)) { set_error("pnp_simulate_measurements: H and W must be in [2, 1024]"); return -2; }
+  const size_t hw = size_t(H) * W, nout = size_t(B) * hw * sizeof(float2);
+  const size_t ngt = (size_t(B - 1) * gt_batch_stride + hw) * sizeof(float);
+  const size_t nmask = size_t(B - 1) * mask_batch_stride + hw;
+  const void* outs[3] = {y0_out, x0_out, aty0_out};
+  for (int k = 0; k < 3; ++k) {
+    bool bad = ranges_overlap(outs[k], nout, gt, ngt) || ranges_overlap(outs[k], nout, mask, nmask);
+    for (int q = k + 1; q < 3; ++q) bad |= ranges_overlap(outs[k], nout, outs[q], nout);
+    if (bad) { set_error("pnp_simulate_measurements: outputs overlap each other, gt or mask"); return -1; }
+  }
+  REQUIRE_INIT();
+  return fail_cuda(simulate_measurements(gt, gt_batch_stride, mask, mask_batch_stride, sigma_n, sigma_stride, seeds,
+                                         static_cast<float2*>(y0_out), static_cast<float2*>(x0_out),
+                                         static_cast<float2*>(aty0_out), B, H, W, cudaStream_t(stream)),
+                   "pnp_simulate_measurements");
+}
+
+int pnp_cartesian_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_cols, uint8_t* mask_out,
+                        int B, int H, int W, void* stream) {
+  if (!accel || !seeds || !mask_out) { set_error("pnp_cartesian_masks: null pointer"); return -1; }
+  if (B <= 0 || accel_stride < 0 || acs_cols < 1) {
+    set_error("pnp_cartesian_masks: need B > 0, accel_stride >= 0 and acs_cols >= 1");
+    return -1;
+  }
+  if (!fft_any_shape_supported(H, W)) { set_error("pnp_cartesian_masks: H and W must be in [2, 1024]"); return -2; }
+  REQUIRE_INIT();
+  return fail_cuda(cartesian_masks(accel, accel_stride, seeds, acs_cols, mask_out, B, H, W, cudaStream_t(stream)),
+                   "pnp_cartesian_masks");
+}
+
 int pnp_residual_real(const void* z, const void* u, float* v, long long n, void* stream) {
   REQUIRE_INIT();
   long long g = (n + 255) / 256;

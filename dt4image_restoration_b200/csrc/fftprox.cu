@@ -39,6 +39,7 @@ void init_fft_tables() {
 #include "fftprox_cl.cuh"
 #include "fftprox_cl128.cuh"
 #include "fftprox_any.cuh"
+#include "measure.cuh"
 namespace pnp {
 
 enum { ROWS_LOAD_XU = 0, ROWS_LOAD_C = 1 };

@@ -37,6 +37,12 @@ int prox_dual_prepared(const float* x, const float2* u_in, const float2* y0T, co
                        float* v_out, int B, int H, int W, int kind, cudaStream_t st, const uint8_t* active = nullptr);
 const int* prox_prepared_flag(const uint8_t* maskp, long long mask_bstride, int B, int H, int W);
 int fft2c_general(const float2* src, float2* dst, int B, int H, int W, int inverse, cudaStream_t st);
+// measure.cuh (compiled into fftprox.cu)
+int simulate_measurements(const float* gt, long long gt_bstride, const uint8_t* mask, long long mask_bstride,
+                          const float* sigma, int sigma_stride, const unsigned long long* seeds, float2* y0, float2* x0,
+                          float2* aty0, int B, int H, int W, cudaStream_t st);
+int cartesian_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_cols, uint8_t* mask,
+                    int B, int H, int W, cudaStream_t st);
 
 // policy.cu
 size_t policy_packed_floats(int n_time, int n_task);

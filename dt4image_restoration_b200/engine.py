@@ -85,6 +85,29 @@ class PnPEngine:
         self.prepare()
         self.iters = 0
 
+    def reset_from_gt(self, gt, sigma_n, seeds, mask=None, accel=None):
+        """Start B new trajectories from fully-sampled images, simulating the measurements straight into the engine's
+        buffers (``ops.simulate_measurements``; no host<->device copy of image data): ``y0``, ``z`` = x0, ``x`` = ``v`` =
+        Re x0, ``u`` = 0, ``mask``, ``gt``.  Same state as ``reset(ops.make_items(gt, sigma_n, seeds, mask, accel))``.
+        ``gt`` fp32 CUDA ``[B,1,H,W]`` / ``[B,H,W]`` / ``[H,W]``; pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H,
+        W]``, CUDA) and ``accel`` (Cartesian masks drawn with ``seeds``)."""
+        if (mask is None) == (accel is None):
+            raise ValueError("pass exactly one of mask / accel")
+        B, H, W = self.B, self.H, self.W
+        seeds = ops._seed_tensor(seeds, B, self.device)
+        if mask is None:
+            ops.cartesian_masks(B, H, W, accel, seeds, out=self.mask)
+        else:
+            m = ops._mask_u8(mask).reshape(-1, 1, H, W)
+            self.mask.copy_(m.ne(0).expand(B, 1, H, W))
+        self.gt.copy_(ops._req(gt, torch.float32, "gt").reshape(-1, 1, H, W).expand(B, 1, H, W))
+        ops.simulate_measurements(self.gt, self.mask, sigma_n, seeds, aty0=False, out=(self.y0, self.z, None))
+        self.u.zero_()
+        self.x.copy_(self.z.real)
+        self.v.copy_(self.z.real)           # Re(z - u) with u = 0
+        self.prepare()
+        self.iters = 0
+
     def prepare(self):
         """Refresh the prepared copies after ``y0`` / ``mask`` changed (they are constants of a trajectory)."""
         if self.prepared:

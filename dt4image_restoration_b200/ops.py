@@ -84,6 +84,118 @@ def fft2c(x: torch.Tensor, inverse: bool = False) -> torch.Tensor:
     return out
 
 
+def _mask_u8(mask: torch.Tensor) -> torch.Tensor:
+    if mask.dtype == torch.bool:
+        mask = mask.contiguous().view(torch.uint8)
+    return _req(mask, torch.uint8, "mask")
+
+
+def _seed_tensor(seeds, B: int, device) -> torch.Tensor:
+    """int64 ``[B]`` seeds on the device; an int ``s0`` stands for ``s0 + arange(B)`` (synth.make_batch's image numbering)."""
+    if isinstance(seeds, int):
+        return torch.arange(seeds, seeds + B, dtype=torch.int64, device=device)
+    seeds = _req(seeds.reshape(-1), torch.int64, "seeds")
+    if seeds.numel() != B:
+        raise RuntimeError(f"seeds must have {B} elements, got {seeds.numel()}")
+    return seeds
+
+
+def _per_image(val, B: int, dtype, name: str, device):
+    """A host scalar (one value for the batch, stride 0) or a CUDA ``[B]`` tensor (stride 1)."""
+    if torch.is_tensor(val):
+        val = _req(val.reshape(-1), dtype, name)
+        if val.numel() not in (1, B):
+            raise RuntimeError(f"{name} must have 1 or {B} elements, got {val.numel()}")
+        return val, 0 if val.numel() == 1 else 1
+    return torch.full((1,), val, dtype=dtype, device=device), 0
+
+
+def _batch_size(gt, mask, sigma_n, seeds) -> int:
+    """Images in a simulator call: gt's batch, else the length of seeds / sigma_n / mask, else 1."""
+    H, W = gt.shape[-2:]
+    if gt.dim() > 2:
+        return gt.numel() // (H * W)
+    if torch.is_tensor(seeds):
+        return seeds.numel()
+    if torch.is_tensor(sigma_n) and sigma_n.numel() > 1:
+        return sigma_n.numel()
+    return max(1, mask.numel() // (H * W)) if mask is not None else 1
+
+
+def simulate_measurements(gt, mask, sigma_n, seeds, aty0: bool = True, out=None):
+    """Undersampled, noisy k-space measurements of fully-sampled images (``pnp_simulate_measurements``, definition in
+    include/pnp_b200.h): ``y0 = mask . (fft_c(gt) + sigma_n/255 (n_r + i n_i))``, ``ATy0 = ifft_c(y0)``, ``x0 = max(ATy0, 0)``
+    componentwise.
+
+    ``gt`` fp32 ``[B,1,H,W]`` / ``[B,H,W]`` or one shared ``[H,W]``; ``mask`` bool/uint8 ``[B or 1, ..., H, W]``;
+    ``sigma_n`` a float or fp32 ``[B]``; ``seeds`` int64 ``[B]`` or an int ``s0`` meaning ``s0 + arange(B)``.  CUDA tensors
+    only.  Returns complex64 ``[B,1,H,W]`` tensors ``(y0, x0, ATy0)`` (``ATy0`` is None with ``aty0=False``), written into
+    ``out=(y0, x0, aty0)`` when given."""
+    gt = _req(gt, torch.float32, "gt")
+    H, W = gt.shape[-2:]
+    B = _batch_size(gt, mask, sigma_n, seeds)
+    gt_stride = H * W if gt.numel() == B * H * W else 0
+    if gt.numel() not in (B * H * W, H * W):
+        raise RuntimeError(f"gt has {gt.numel()} elements, expected {B * H * W} or {H * W}")
+    mask = _mask_u8(mask)
+    if mask.numel() not in (B * H * W, H * W):
+        raise IndexError(f"mask with {mask.numel()} elements does not match {B} images of {H}x{W}")
+    mstride = H * W if mask.numel() == B * H * W else 0
+    sig, sstride = _per_image(sigma_n, B, torch.float32, "sigma_n", gt.device)
+    seeds = _seed_tensor(seeds, B, gt.device)
+    if out is None:
+        y0 = torch.empty(B, 1, H, W, dtype=torch.complex64, device=gt.device)
+        x0 = torch.empty_like(y0)
+        at = torch.empty_like(y0) if aty0 else None
+    else:
+        y0, x0, at = out
+        for t in (y0, x0) + ((at,) if at is not None else ()):
+            if not t.is_cuda or t.dtype != torch.complex64 or not t.is_contiguous() or t.numel() != B * H * W:
+                raise RuntimeError(f"out tensors must be contiguous complex64 CUDA tensors with {B * H * W} elements")
+    check(_lib.lib().pnp_simulate_measurements(gt.data_ptr(), gt_stride, mask.data_ptr(), mstride, sig.data_ptr(), sstride,
+                                               seeds.data_ptr(), y0.data_ptr(), x0.data_ptr(),
+                                               at.data_ptr() if at is not None else None, B, H, W, _lib.stream_ptr()),
+          "pnp_simulate_measurements")
+    return y0, x0, at
+
+
+def cartesian_masks(B: int, H: int, W: int, accel, seeds, acs_frac: float = 0.08, out=None) -> torch.Tensor:
+    """Seeded Cartesian masks (``pnp_cartesian_masks``): uint8 ``[B,H,W]`` on the current CUDA device with
+    ``synth.cartesian_mask``'s structure - a centred ACS band of ``max(1, round(acs_frac W))`` columns plus random columns
+    up to ``max(1, W // accel)``.  ``accel`` an int or int32 ``[B]`` CUDA tensor; ``seeds`` as in ``simulate_measurements``."""
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if not torch.is_tensor(accel) and int(accel) < 1:
+        raise ValueError(f"accel must be >= 1, got {accel}")
+    acc, astride = _per_image(accel if torch.is_tensor(accel) else int(accel), B, torch.int32, "accel", dev)
+    seeds = _seed_tensor(seeds, B, dev)
+    acs_cols = max(1, int(round(acs_frac * W)))
+    if out is None:
+        out = torch.empty(B, H, W, dtype=torch.uint8, device=dev)
+    elif not out.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous() or out.numel() != B * H * W:
+        raise RuntimeError(f"out must be a contiguous uint8 CUDA tensor with {B * H * W} elements")
+    check(_lib.lib().pnp_cartesian_masks(acc.data_ptr(), astride, seeds.data_ptr(), acs_cols, out.data_ptr(), B, H, W,
+                                         _lib.stream_ptr()), "pnp_cartesian_masks")
+    return out
+
+
+def make_items(gt, sigma_n, seeds, mask=None, accel=None) -> dict:
+    """A batch of episode items on the device with ``synth.make_batch``'s keys, shapes and dtypes (``x0, y0, ATy0`` fp32
+    ``[B,1,H,W,2]``, ``mask`` uint8 ``[B,H,W]``, ``gt`` fp32 ``[B,1,H,W]``), ready for ``PnPEnv.reset`` / ``PnPEngine.reset``.
+    Pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``) and ``accel`` (Cartesian masks drawn with ``seeds``)."""
+    if (mask is None) == (accel is None):
+        raise ValueError("pass exactly one of mask / accel")
+    gt = _req(gt, torch.float32, "gt")
+    H, W = gt.shape[-2:]
+    B = _batch_size(gt, mask, sigma_n, seeds)
+    if mask is None:
+        mask = cartesian_masks(B, H, W, accel, seeds)
+    else:
+        mask = _mask_u8(mask).ne(0).to(torch.uint8).reshape(-1, H, W).expand(B, H, W).contiguous()
+    y0, x0, aty0 = simulate_measurements(gt, mask, sigma_n, seeds)
+    return {"x0": torch.view_as_real(x0), "y0": torch.view_as_real(y0), "ATy0": torch.view_as_real(aty0), "mask": mask,
+            "gt": gt.reshape(-1, 1, H, W).expand(B, 1, H, W).contiguous()}
+
+
 def residual_real(z: torch.Tensor, u: torch.Tensor) -> torch.Tensor:
     """``Re(z - u)`` as fp32 (env.py:85-86)."""
     z = _req(z, torch.complex64, "z")

@@ -67,6 +67,41 @@ int pnp_ssim(const float* x, const float* gt, long long gt_batch_stride, float* 
  * is mixed-radix, so the reference accepts them).  dst may alias src. */
 int pnp_fft2c(const void* src_c64, void* dst_c64, int B, int H, int W, int inverse, void* stream);
 
+/* Episode generation on the device: undersampled, noisy k-space measurements of fully-sampled images (what the reference
+ * loads from precomputed .mat items, dataset/datasets.py:148-168; synth.make_item is the host-side NumPy version).
+ * Per image b, with fft_c / ifft_c the centred orthonormal transforms (transformations.py:6-19), and every index (i, j) in
+ * the centred k-space layout of y0:
+ *   p = i*W + j
+ *   (w0, w1, _, _) = philox4x32_10(counter = (p, 0, 0, 0), key = (lo32(seed[b]), hi32(seed[b])))
+ *   u1 = (w0 + 0.5) * 2^-32,   u2 = (w1 + 0.5) * 2^-32
+ *   n_r = sqrt(-2 ln u1) * cos(2 pi u2),   n_i = sqrt(-2 ln u1) * sin(2 pi u2)
+ *   y0[b,i,j]   = mask[b,i,j] != 0 ? fft_c(gt[b])[i,j] + (sigma_n[b] / 255) * (n_r + i*n_i) : 0
+ *   ATy0[b]     = ifft_c(y0[b])
+ *   x0[b]       = (max(Re ATy0, 0), max(Im ATy0, 0))          # datasets.py:160,199 / synth.make_item
+ * philox4x32_10 is the Random123 generator: 10 rounds of
+ *   (c0, c1, c2, c3) -> (hi(M1*c2) ^ c1 ^ k0, lo(M1*c2), hi(M0*c0) ^ c3 ^ k1, lo(M0*c0)),  M0 = 0xD2511F53, M1 = 0xCD9E8D57,
+ * with the key bumped by (0x9E3779B9, 0xBB67AE85) between rounds.  The noise depends only on (seed, H, W, i, j): not on the
+ * mask, the batch position or the other images.  With sigma_n[b] == 0, y0 = mask . fft_c(gt).
+ * gt: fp32 [B,H,W] with gt_batch_stride = H*W, or one [H,W] with stride 0; mask: uint8 likewise; sigma_n: device fp32,
+ * sigma_n[b*sigma_stride] (0 = one value for the batch); seeds: device uint64 [B].  Outputs c64 [B,H,W]; aty0_out may be
+ * NULL.  H, W in 2..1024 (radix kernels for powers of two in 32..512, dense DFT otherwise); no workspace; outputs must not
+ * overlap each other, gt or mask.  Results are bitwise reproducible and independent of the batch position. */
+int pnp_simulate_measurements(const float* gt, long long gt_batch_stride, const uint8_t* mask, long long mask_batch_stride,
+                              const float* sigma_n, int sigma_stride, const unsigned long long* seeds,
+                              void* y0_out_c64, void* x0_out_c64, void* aty0_out_c64, int B, int H, int W, void* stream);
+
+/* Seeded Cartesian undersampling masks (the structure of synth.cartesian_mask, drawn with the generator above).  Per image b:
+ *   n_keep = max(1, W / accel[b]) (integer division);  n_acs = min(n_keep, acs_cols);  c0 = W/2 - n_acs/2
+ *   columns [c0, c0 + n_acs) are sampled (ACS band);
+ *   key_j = philox4x32_10(counter = (j, 1, 0, 0), key = seed split as above).w0  for every column j;
+ *   the n_keep - n_acs non-ACS columns with the smallest (key_j, j), compared lexicographically, are sampled;
+ *   mask[b, i, j] = 1 for every row i of a sampled column, else 0.
+ * accel: device int32, accel[b*accel_stride] (accel < 1 samples every column); seeds: device uint64 [B]; mask_out: uint8
+ * [B,H,W].  H, W in 2..1024, acs_cols >= 1 (synth.cartesian_mask uses max(1, round(0.08 W))).  These masks depend on the
+ * column index only, so pnp_prox_prepare routes them to the row-only prox kernel. */
+int pnp_cartesian_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_cols, uint8_t* mask_out,
+                        int B, int H, int W, void* stream);
+
 /* v = Re(z - u): the denoiser input of PnPEnv.step (env.py:85-86). */
 int pnp_residual_real(const void* z_c64, const void* u_c64, float* v, long long n, void* stream);
 
