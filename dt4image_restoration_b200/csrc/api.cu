@@ -122,13 +122,13 @@ int pnp_fft2c(const void* src, void* dst, int B, int H, int W, int inverse, void
                                  cudaStream_t(stream)), "pnp_fft2c");
 }
 
-// Byte ranges [lo, hi) of the buffers of pnp_simulate_measurements, for the overlap test.
+// Byte ranges [lo, hi) of the buffers of pnp_simulate_measurements / pnp_radial_masks, for the overlap test.
 static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
   const uintptr_t pa = reinterpret_cast<uintptr_t>(a), pb = reinterpret_cast<uintptr_t>(b);
   return a && b && pa < pb + nb && pb < pa + na;
 }
 
-// The argument checks of the two simulator entry points come before REQUIRE_INIT, so a bad call is refused with its own
+// The argument checks of the simulator and mask entry points come before REQUIRE_INIT, so a bad call is refused with its own
 // message whether or not pnp_init has run.
 int pnp_simulate_measurements(const float* gt, long long gt_batch_stride, const uint8_t* mask, long long mask_batch_stride,
                               const float* sigma_n, int sigma_stride, const unsigned long long* seeds, void* y0_out,
@@ -169,6 +169,22 @@ int pnp_cartesian_masks(const int* accel, int accel_stride, const unsigned long 
   REQUIRE_INIT();
   return fail_cuda(cartesian_masks(accel, accel_stride, seeds, acs_cols, mask_out, B, H, W, cudaStream_t(stream)),
                    "pnp_cartesian_masks");
+}
+
+int pnp_radial_masks(const double* frac, int frac_stride, const unsigned long long* seeds, uint8_t* mask_out,
+                     int* lines_out, int B, int H, int W, void* stream) {
+  if (!frac || !mask_out) { set_error("pnp_radial_masks: null pointer"); return -1; }
+  if (B <= 0 || frac_stride < 0) { set_error("pnp_radial_masks: need B > 0 and frac_stride >= 0"); return -1; }
+  if (!fft_any_shape_supported(H, W)) { set_error("pnp_radial_masks: H and W must be in [2, 1024]"); return -2; }
+  const size_t nmask = size_t(B) * H * W, nlines = size_t(B) * sizeof(int);
+  const size_t nfrac = (size_t(B - 1) * frac_stride + 1) * sizeof(double), nseeds = size_t(B) * sizeof(unsigned long long);
+  const bool bad = ranges_overlap(lines_out, nlines, mask_out, nmask) || ranges_overlap(mask_out, nmask, frac, nfrac) ||
+                   ranges_overlap(mask_out, nmask, seeds, nseeds) || ranges_overlap(lines_out, nlines, frac, nfrac) ||
+                   ranges_overlap(lines_out, nlines, seeds, nseeds);
+  if (bad) { set_error("pnp_radial_masks: outputs overlap each other, frac or seeds"); return -1; }
+  REQUIRE_INIT();
+  return fail_cuda(radial_masks(frac, frac_stride, seeds, mask_out, lines_out, B, H, W, cudaStream_t(stream)),
+                   "pnp_radial_masks");
 }
 
 int pnp_residual_real(const void* z, const void* u, float* v, long long n, void* stream) {

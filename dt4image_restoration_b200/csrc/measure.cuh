@@ -1,5 +1,6 @@
-// Measurement simulator: undersampled, noisy k-space measurements of fully-sampled images, and seeded Cartesian masks
-// (pnp_simulate_measurements / pnp_cartesian_masks; the definition is in include/pnp_b200.h).  Per image b:
+// Measurement simulator: undersampled, noisy k-space measurements of fully-sampled images, and seeded Cartesian and radial
+// masks (pnp_simulate_measurements / pnp_cartesian_masks / pnp_radial_masks; the definitions are in include/pnp_b200.h).
+// Per image b:
 //
 //     y0   = mask ? fft_c(gt) + sigma_n / 255 * (n_r + i n_i) : 0      (n_r, n_i: Philox4x32-10 + Box-Muller at (i, j))
 //     ATy0 = ifft_c(y0),   x0 = (max(Re ATy0, 0), max(Im ATy0, 0))
@@ -310,6 +311,94 @@ __global__ void __launch_bounds__(kMaskThreads) cartesian_mask_kernel(const int*
   for (size_t e = head + 16 * nvec + threadIdx.x; e < n; e += kMaskThreads) img[e] = col[e % W];
 }
 
+// ---------------------------------------------------------------- golden-angle radial masks: one CTA per image
+// Lines are drawn in order because the stopping rule reads the sampled count after every line.  The image is a bitmap in
+// dynamic shared memory (one spare zero word past the end for the two-word reads of the write-out); a point sets its bit
+// with atomicOr and is new when the old word lacked the bit, so a line's new pixels are counted exactly whatever the order
+// of its points, and a pixel two t of one line round to is counted once.  sin / cos of kRadialThreads consecutive lines are
+// computed together (one line per thread) into a table, instead of by every thread for every line: the FP64 pipe then does
+// one sincos per line, and the table costs one extra barrier per kRadialThreads lines.
+constexpr int kRadialThreads = 512;
+constexpr int kRadialWarps = kRadialThreads / 32;
+constexpr int kRadialPoints = 3;        // points per thread and line: 2R + 1 = 1453 <= 3 * 512 at 1024x1024 (R = 726)
+__host__ __device__ constexpr size_t radial_smem_bytes(int H, int W) {
+  return (size_t(H) * W / 32 + 2) * sizeof(unsigned);
+}
+
+__global__ void __launch_bounds__(kRadialThreads) radial_mask_kernel(const double* frac, int frac_stride,
+                                                                     const unsigned long long* seeds, uint8_t* out,
+                                                                     int* lines_out, int H, int W) {
+  extern __shared__ unsigned radial_bits[];
+  __shared__ double2 sc[kRadialThreads];                  // (sin, cos) of lines n0 .. n0 + kRadialThreads - 1
+  __shared__ int warp_new[2][kRadialWarps];               // new pixels per warp, double-buffered by line parity
+  const int b = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int n_words = int(radial_smem_bytes(H, W) / sizeof(unsigned));
+  for (int w = tid; w < n_words; w += kRadialThreads) radial_bits[w] = 0u;
+  constexpr double kGolden = 0x1.f10d6bc8e0e35p+0;       // pi (sqrt 5 - 1) / 2 as NumPy computes it in float64
+  const double phi = seeds ? __dmul_rn(double(philox4x32_10(make_uint4(0u, 2u, 0u, 0u), seed_key(seeds[b])).x),
+                                       0x1.921fb54442d18p-31)      // pi * 2^-32: phi in [0, pi)
+                           : 0.0;
+  const double target = __dmul_rn(__dmul_rn(frac[size_t(b) * frac_stride], double(H)), double(W));   // NaN: no line
+  const int s2 = H * H + W * W;
+  int r = int(sqrt(double(s2)) * 0.5);                     // never above the smallest r with 4 r^2 >= s2
+  while (4 * r * r < s2) ++r;
+  const int R = r + 1, cap = 8 * max(H, W);
+  const double cy = double(H / 2), cx = double(W / 2);
+  double tv[kRadialPoints];                                // this thread's t: tid - R + k * kRadialThreads <= R
+  int npts = 0;
+#pragma unroll
+  for (int k = 0; k < kRadialPoints; ++k) {
+    tv[k] = double(tid - R + k * kRadialThreads);
+    npts += tid - R + k * kRadialThreads <= R;
+  }
+  __syncthreads();                                         // the bitmap is zeroed
+  int count = 0, n = 0;
+  while (n < cap && double(count) < target) {             // the same values in every thread: a uniform loop
+    if ((n & (kRadialThreads - 1)) == 0) {                 // the old table was last read before the previous barrier
+      double s, c;
+      sincos(__dadd_rn(__dmul_rn(double(n + tid), kGolden), phi), &s, &c);
+      sc[tid] = make_double2(s, c);
+      __syncthreads();
+    }
+    const double2 l = sc[n & (kRadialThreads - 1)];
+    int fresh = 0;
+#pragma unroll
+    for (int k = 0; k < kRadialPoints; ++k) {
+      // __double2int_rn is rint (half to even) and the conversion to int in one instruction (|value| < 2^11)
+      const int y = __double2int_rn(__dadd_rn(cy, __dmul_rn(tv[k], l.x)));
+      const int x = __double2int_rn(__dadd_rn(cx, __dmul_rn(tv[k], l.y)));
+      if (k < npts && unsigned(y) < unsigned(H) && unsigned(x) < unsigned(W)) {
+        const unsigned p = unsigned(y) * unsigned(W) + unsigned(x), bit = 1u << (p & 31);
+        fresh += (atomicOr(&radial_bits[p >> 5], bit) & bit) == 0u;
+      }
+    }
+    fresh = __reduce_add_sync(0xFFFFFFFFu, fresh);
+    if (lane == 0) warp_new[n & 1][warp] = fresh;          // this slot was last read before the previous line's barrier
+    __syncthreads();
+#pragma unroll
+    for (int w = 0; w < kRadialWarps; ++w) count += warp_new[n & 1][w];
+    ++n;
+  }
+  if (lines_out && tid == 0) lines_out[b] = n;
+  // the last barrier (the last line's, or the one after zeroing) orders every atomicOr before these reads.  Rows of the
+  // image as one flat run of H*W bytes: 16-byte stores between an unaligned head and tail
+  const size_t npx = size_t(H) * W;
+  uint8_t* img = out + size_t(b) * npx;
+  const size_t head = min(size_t((16 - (reinterpret_cast<uintptr_t>(img) & 15)) & 15), npx);
+  const size_t nvec = (npx - head) / 16;
+  for (size_t e = tid; e < head; e += kRadialThreads) img[e] = (radial_bits[e >> 5] >> (e & 31)) & 1u;
+  for (size_t q = tid; q < nvec; q += kRadialThreads) {
+    const size_t p0 = head + 16 * q;
+    const unsigned w0 = radial_bits[p0 >> 5], w1 = radial_bits[(p0 >> 5) + 1];
+    const unsigned bits = __funnelshift_r(w0, w1, unsigned(p0 & 31));   // pixels p0 .. p0 + 15 in the low 16 bits
+    unsigned v[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) v[k] = (((bits >> (4 * k)) & 0xFu) * 0x00204081u) & 0x01010101u;   // 4 bits -> 4 bytes
+    reinterpret_cast<uint4*>(img + p0)[0] = make_uint4(v[0], v[1], v[2], v[3]);
+  }
+  for (size_t e = head + 16 * nvec + tid; e < npx; e += kRadialThreads) img[e] = (radial_bits[e >> 5] >> (e & 31)) & 1u;
+}
+
 // ---------------------------------------------------------------- host side
 // Launch `fn(q, nb)` over batch chunks of at most 65535 images (grid.y limit), q's pointers advanced to the chunk.
 template <typename F>
@@ -398,6 +487,20 @@ int cartesian_masks(const int* accel, int accel_stride, const unsigned long long
                     int B, int H, int W, cudaStream_t st) {
   if (!any_shape_supported(H, W)) return -2;
   cartesian_mask_kernel<<<B, kMaskThreads, 0, st>>>(accel, accel_stride, seeds, acs_cols, mask, H, W);
+  return int(cudaGetLastError());
+}
+
+int radial_masks(const double* frac, int frac_stride, const unsigned long long* seeds, uint8_t* mask, int* lines_out,
+                 int B, int H, int W, cudaStream_t st) {
+  if (!any_shape_supported(H, W)) return -2;
+  static bool attr_done = false;
+  if (!attr_done) {
+    cudaError_t e = cudaFuncSetAttribute(radial_mask_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         int(radial_smem_bytes(kAnyMaxN, kAnyMaxN)));
+    if (e != cudaSuccess) return int(e);
+    attr_done = true;
+  }
+  radial_mask_kernel<<<B, kRadialThreads, radial_smem_bytes(H, W), st>>>(frac, frac_stride, seeds, mask, lines_out, H, W);
   return int(cudaGetLastError());
 }
 

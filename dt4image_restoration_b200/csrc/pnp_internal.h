@@ -43,6 +43,8 @@ int simulate_measurements(const float* gt, long long gt_bstride, const uint8_t* 
                           float2* aty0, int B, int H, int W, cudaStream_t st);
 int cartesian_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_cols, uint8_t* mask,
                     int B, int H, int W, cudaStream_t st);
+int radial_masks(const double* frac, int frac_stride, const unsigned long long* seeds, uint8_t* mask, int* lines_out,
+                 int B, int H, int W, cudaStream_t st);
 
 // policy.cu
 size_t policy_packed_floats(int n_time, int n_task);

@@ -85,18 +85,21 @@ class PnPEngine:
         self.prepare()
         self.iters = 0
 
-    def reset_from_gt(self, gt, sigma_n, seeds, mask=None, accel=None):
+    def reset_from_gt(self, gt, sigma_n, seeds, mask=None, accel=None, radial=None):
         """Start B new trajectories from fully-sampled images, simulating the measurements straight into the engine's
         buffers (``ops.simulate_measurements``; no host<->device copy of image data): ``y0``, ``z`` = x0, ``x`` = ``v`` =
-        Re x0, ``u`` = 0, ``mask``, ``gt``.  Same state as ``reset(ops.make_items(gt, sigma_n, seeds, mask, accel))``.
+        Re x0, ``u`` = 0, ``mask``, ``gt``.  Same state as ``reset(ops.make_items(gt, sigma_n, seeds, mask, accel, radial))``.
         ``gt`` fp32 CUDA ``[B,1,H,W]`` / ``[B,H,W]`` / ``[H,W]``; pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H,
-        W]``, CUDA) and ``accel`` (Cartesian masks drawn with ``seeds``)."""
-        if (mask is None) == (accel is None):
-            raise ValueError("pass exactly one of mask / accel")
+        W]``, CUDA), ``accel`` (Cartesian masks drawn with ``seeds``) and ``radial`` (radial masks with this sampled fraction,
+        rotated by ``seeds``)."""
+        if sum(m is not None for m in (mask, accel, radial)) != 1:
+            raise ValueError("pass exactly one of mask / accel / radial")
         B, H, W = self.B, self.H, self.W
         seeds = ops._seed_tensor(seeds, B, self.device)
-        if mask is None:
+        if accel is not None:
             ops.cartesian_masks(B, H, W, accel, seeds, out=self.mask)
+        elif radial is not None:
+            ops.radial_masks(B, H, W, radial, seeds, out=self.mask)
         else:
             m = ops._mask_u8(mask).reshape(-1, 1, H, W)
             self.mask.copy_(m.ne(0).expand(B, 1, H, W))

@@ -178,17 +178,42 @@ def cartesian_masks(B: int, H: int, W: int, accel, seeds, acs_frac: float = 0.08
     return out
 
 
-def make_items(gt, sigma_n, seeds, mask=None, accel=None) -> dict:
+def radial_masks(B: int, H: int, W: int, frac, seeds=None, out=None, lines_out=None) -> torch.Tensor:
+    """Golden-angle radial masks (``pnp_radial_masks``): uint8 ``[B,H,W]`` on the current CUDA device.  Lines through the
+    k-space centre are added until the sampled fraction reaches ``frac`` (a float or float64 ``[B]`` CUDA tensor).  With
+    ``seeds=None`` every mask is ``synth.radial_mask(H, W, frac)``; with ``seeds`` (as in ``simulate_measurements``) image b's
+    lines are rotated by a Philox draw of its seed.  The number of lines of each image goes to ``lines_out`` (int32 ``[B]``,
+    CUDA) when given."""
+    dev = torch.device("cuda", torch.cuda.current_device())
+    fr, fstride = _per_image(frac if torch.is_tensor(frac) else float(frac), B, torch.float64, "frac", dev)
+    seeds = _seed_tensor(seeds, B, dev) if seeds is not None else None
+    if out is None:
+        out = torch.empty(B, H, W, dtype=torch.uint8, device=dev)
+    elif not out.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous() or out.numel() != B * H * W:
+        raise _lib.PnpError(f"out must be a contiguous uint8 CUDA tensor with {B * H * W} elements")
+    if lines_out is not None and (not lines_out.is_cuda or lines_out.dtype != torch.int32 or not lines_out.is_contiguous()
+                                  or lines_out.numel() != B):
+        raise _lib.PnpError(f"lines_out must be a contiguous int32 CUDA tensor with {B} elements")
+    check(_lib.lib().pnp_radial_masks(fr.data_ptr(), fstride, seeds.data_ptr() if seeds is not None else None,
+                                      out.data_ptr(), lines_out.data_ptr() if lines_out is not None else None, B, H, W,
+                                      _lib.stream_ptr()), "pnp_radial_masks")
+    return out
+
+
+def make_items(gt, sigma_n, seeds, mask=None, accel=None, radial=None) -> dict:
     """A batch of episode items on the device with ``synth.make_batch``'s keys, shapes and dtypes (``x0, y0, ATy0`` fp32
     ``[B,1,H,W,2]``, ``mask`` uint8 ``[B,H,W]``, ``gt`` fp32 ``[B,1,H,W]``), ready for ``PnPEnv.reset`` / ``PnPEngine.reset``.
-    Pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``) and ``accel`` (Cartesian masks drawn with ``seeds``)."""
-    if (mask is None) == (accel is None):
-        raise ValueError("pass exactly one of mask / accel")
+    Pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``), ``accel`` (Cartesian masks drawn with ``seeds``) and
+    ``radial`` (the sampled fraction of radial masks rotated by ``seeds``, see ``radial_masks``)."""
+    if sum(m is not None for m in (mask, accel, radial)) != 1:
+        raise ValueError("pass exactly one of mask / accel / radial")
     gt = _req(gt, torch.float32, "gt")
     H, W = gt.shape[-2:]
     B = _batch_size(gt, mask, sigma_n, seeds)
-    if mask is None:
+    if accel is not None:
         mask = cartesian_masks(B, H, W, accel, seeds)
+    elif radial is not None:
+        mask = radial_masks(B, H, W, radial, seeds)
     else:
         mask = _mask_u8(mask).ne(0).to(torch.uint8).reshape(-1, H, W).expand(B, H, W).contiguous()
     y0, x0, aty0 = simulate_measurements(gt, mask, sigma_n, seeds)

@@ -102,6 +102,26 @@ int pnp_simulate_measurements(const float* gt, long long gt_batch_stride, const 
 int pnp_cartesian_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_cols, uint8_t* mask_out,
                         int B, int H, int W, void* stream);
 
+/* Seeded golden-angle radial masks (synth.radial_mask's lines, rotated per image).  Per image b, in float64:
+ *   cy = H / 2, cx = W / 2 (integer division);  R = 1 + the smallest integer r with 4 r^2 >= H^2 + W^2
+ *   golden = 0x1.f10d6bc8e0e35p+0 (pi (sqrt 5 - 1) / 2 as NumPy computes it)
+ *   phi = 0 if seeds == NULL, else double(philox4x32_10(counter = (0, 2, 0, 0), key = seed[b] split as above).w0)
+ *         * 0x1.921fb54442d18p-31 (pi * 2^-32, so phi is in [0, pi))
+ *   target = (frac[b*frac_stride] * H) * W;  count = 0, n = 0
+ *   while count < target and n < 8 * max(H, W):
+ *       ang = n * golden + phi                                    (two roundings, no FMA)
+ *       for t in -R .. R:  y = rint(cy + t sin(ang)),  x = rint(cx + t cos(ang))   (each op rounded, no FMA; rint rounds
+ *           half to even);  if 0 <= y < H and 0 <= x < W: mask[b, y, x] = 1
+ *       count = number of sampled pixels of image b;  n += 1
+ *   lines_out[b] = n
+ * With seeds == NULL the mask is exactly synth.radial_mask(H, W, frac).  frac <= 0 or NaN draws no line; frac > 1 runs to the
+ * 8 max(H, W) line cap.  Counter word 1 = 2 keeps this stream apart from the noise (word 1 = 0) and the Cartesian column
+ * keys (word 1 = 1).  frac: device float64 (0 stride = one value for the batch); seeds: device uint64 [B] or NULL;
+ * mask_out: uint8 [B,H,W]; lines_out: device int32 [B] or NULL.  H, W in 2..1024; the outputs must not overlap each other,
+ * frac or seeds.  Results are bitwise reproducible and independent of the batch position. */
+int pnp_radial_masks(const double* frac, int frac_stride, const unsigned long long* seeds, uint8_t* mask_out,
+                     int* lines_out, int B, int H, int W, void* stream);
+
 /* v = Re(z - u): the denoiser input of PnPEnv.step (env.py:85-86). */
 int pnp_residual_real(const void* z_c64, const void* u_c64, float* v, long long n, void* stream);
 
