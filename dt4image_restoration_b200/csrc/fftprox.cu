@@ -11,7 +11,8 @@
 // computed as conj(FFT(conj(.))) so a single forward FFT core serves both directions.
 //
 // Sizes that are not powers of two in 32..512 take the dense-DFT path of fftprox_any.cuh (any H, W in 2..1024).
-// This file is the general (any power-of-two H, W in 32..512) three-launch path:
+// This file is the general (any power-of-two H, W in 32..512) three-launch path, the ops ProxRowsIn / ProxColsBlend /
+// ProxRowsOut on the radix line passes of line_passes.cuh:
 //   rows  : load D.(x+u)            -> row FFTs                      -> T (c64 workspace)
 //   cols  : load 8..64 columns of T -> col FFT -> blend -> col FFT   -> T (in place)
 //   rows  : load T                  -> row FFTs -> z, u', v'          (epilogue)
@@ -38,196 +39,112 @@ void init_fft_tables() {
 #include "fftprox_sep.cuh"
 #include "fftprox_cl.cuh"
 #include "fftprox_cl128.cuh"
+#include "line_passes.cuh"
 #include "fftprox_any.cuh"
 #include "measure.cuh"
 namespace pnp {
 
-enum { ROWS_LOAD_XU = 0, ROWS_LOAD_C = 1 };
-enum { ROWS_STORE_C = 0, ROWS_STORE_PROX = 1 };
-
-struct RowsParams {
-  int H, W;
-  int load_mode, store_mode;
-  int load_sign;            // multiply loaded value by D[i,j]
-  int load_conj;
-  const float* x;           // [B,H,W]      (LOAD_XU, STORE_PROX)
-  const float2* u;          // [B,H,W]
-  const float2* src;        // [B,H,W]      (LOAD_C)
-  float2* dst;              // [B,H,W]      (STORE_C)
-  int store_sign, store_conj;
-  float store_scale;
-  float2* z_out;            // STORE_PROX
-  float2* u_out;
-  float* v_out;             // may be null
+// ---- radix ops of the general path (the centring signs D and s as in the header; blend and epilogue in fftprox_any.cuh)
+// rows in: D.(x + u) -> row FFTs -> work
+struct ProxRowsIn : LineOp {
+  const float* x;
+  const float2* u;
+  float2* work;
   const int* skip_flag;     // optional: != 0 -> the row-only kernel handles this batch, do nothing
-  const uint8_t* active;    // optional [B], STORE_PROX only: 0 = leave the image's z, u, v untouched
+  __device__ bool skip() const { return skip_flag && *skip_flag != 0; }
+  __device__ float2 load(const LineElem& e) const {
+    const float2 uu = u[e.g];
+    float2 v = make_float2(x[e.g] + uu.x, uu.y);
+    if ((e.i + e.j) & 1) { v.x = -v.x; v.y = -v.y; }
+    return v;
+  }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { work[e.g] = v; }
 };
 
-template <int N>
-__global__ void __launch_bounds__(256) fft_rows_kernel(const RowsParams p) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int P = fft_pitch(N);
-  if (p.skip_flag && *p.skip_flag != 0) return;
-  __shared__ float2 tw[kTwTotal];
-  extern __shared__ float2 rows_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  fft_load_twiddles(tw, g_tw512);
-  __syncthreads();
-  const int b = blockIdx.y;
-  const int row0 = (blockIdx.x * 8 + warp) * G;
-  if (row0 >= p.H) return;
-  float2* mine = rows_smem + warp * G * P;
-  const size_t img = size_t(b) * p.H * p.W;
-#pragma unroll 1
-  for (int g = 0; g < G; ++g) {
-    const int i = row0 + g;
-    const size_t base = img + size_t(i) * N;
-    for (int j = lane; j < N; j += 32) {
-      float2 v;
-      if (p.load_mode == ROWS_LOAD_XU) {
-        const float2 uu = p.u[base + j];
-        v = make_float2(p.x[base + j] + uu.x, uu.y);
-      } else {
-        v = p.src[base + j];
-      }
-      if (p.load_conj) v.y = -v.y;
-      if (p.load_sign && ((i + j) & 1)) { v.x = -v.x; v.y = -v.y; }
-      mine[g * P + fpad(j)] = v;
+// columns: col FFT -> / sqrt(HW) -> blend with s.D.y0 -> conj -> col FFT (the inverse, conjugated) -> work
+struct ProxColsBlend : ProxBlendOp {
+  float2* work;
+  float norm;               // 1 / sqrt(HW)
+  float sgn;                // s
+  const int* skip_flag;
+  __device__ bool skip() const { return skip_flag && *skip_flag != 0; }
+  __device__ float2 load(const LineElem& e) const { return work[e.g]; }
+  __device__ float2 middle(const BlendImage& m, const LineElem& e, float2 Z) const {
+    Z.x *= norm; Z.y *= norm;
+    if (m.mk[e.o]) {
+      const float2 y = y0[e.g];
+      const float sg = ((e.i + e.j) & 1) ? -sgn : sgn;
+      Z = blend(m, Z, make_float2(sg * y.x, sg * y.y));
     }
+    return make_float2(Z.x, -Z.y);   // conj -> forward FFT == inverse
   }
-  __syncwarp();
-  fft_warp_rows<N>(mine, P, tw, lane);
-#pragma unroll 1
-  for (int g = 0; g < G; ++g) {
-    const int i = row0 + g;
-    const size_t base = img + size_t(i) * N;
-    // the epilogue's u, x loads are plain (u_out may alias u) and stay behind the preceding stores, so the loads of KB
-    // elements are issued ahead of their stores by hand (load -> store -> load chains cost 25 % in the row-only kernels)
-    constexpr int KB = (N / 32 < 4) ? N / 32 : 4;
-    const bool prox_store = p.store_mode != ROWS_STORE_C;
-    if (prox_store && p.active && p.active[b] == 0) continue;
-    for (int j0 = lane; j0 < N; j0 += 32 * KB) {
-      float2 uu[KB];
-      float xx[KB];
-      if (prox_store) {
-#pragma unroll
-        for (int q = 0; q < KB; ++q) {
-          uu[q] = p.u[base + j0 + 32 * q];
-          xx[q] = p.x[base + j0 + 32 * q];
-        }
-      }
-#pragma unroll
-      for (int q = 0; q < KB; ++q) {
-        const int j = j0 + 32 * q;
-        float2 v = mine[g * P + fpad(j)];
-        v.x *= p.store_scale; v.y *= p.store_scale;
-        if (p.store_conj) v.y = -v.y;
-        if (p.store_sign && ((i + j) & 1)) { v.x = -v.x; v.y = -v.y; }
-        if (!prox_store) {
-          p.dst[base + j] = v;
-        } else {
-          const float2 un = make_float2(uu[q].x + xx[q] - v.x, uu[q].y - v.y);   // u' = u + x - z
-          p.z_out[base + j] = v;
-          p.u_out[base + j] = un;
-          if (p.v_out) p.v_out[base + j] = v.x - un.x;                            // Re(z - u')
-        }
-      }
-    }
-  }
-}
+  __device__ void store(const LineElem& e, float2 v, Pre) const { work[e.g] = v; }
+};
 
-struct ColsParams {
-  int H, W;
-  float2* t;                // [B,H,W] in/out (or src -> dst)
+// rows out: row FFTs -> z = D.conj(.) / sqrt(HW) -> z, u', v'
+struct ProxRowsOut : ProxDualOp {
+  // left alone, ptxas gives the epilogue the registers of one CTA per SM at these lengths
+  template <int N> static constexpr int kRowCtas = N == 32 ? 8 : N == 256 ? 6 : 0;
+  const float2* work;
+  float norm;               // 1 / sqrt(HW)
+  const int* skip_flag;
+  __device__ bool skip() const { return skip_flag && *skip_flag != 0; }
+  __device__ float2 load(const LineElem& e) const { return work[e.g]; }
+  __device__ void store(const LineElem& e, float2 v, const Pre& p) const {
+    v.x *= norm; v.y *= norm;
+    v.y = -v.y;
+    if ((e.i + e.j) & 1) { v.x = -v.x; v.y = -v.y; }
+    store_dual(e.g, v, p);
+  }
+};
+
+// pnp_fft2c: rows D.w (conj(w) for the inverse) -> row FFTs -> dst; columns col FFT -> s.D / sqrt(HW) (conj) -> dst
+struct Fft2cRows : LineOp {
   const float2* src;
-  int blend;                // 1: blend with y0 then second FFT of the conjugate
-  const float2* y0;         // [B,H,W]
-  const uint8_t* mask;      // [mask_B,H,W]
-  long long mask_bstride;   // 0 when one mask is shared by the batch
-  const float* mu;          // [B] or [1]
-  int mu_stride;
-  float scale1;             // applied to the first FFT's output (1/sqrt(HW))
-  float sgn;                // s = (-1)^((H+W)/2)
-  int store_sign, store_conj;
-  float store_scale;
-  int load_sign, load_conj, load_neg;   // loaded value: conj if load_conj, times D[i,j] if load_sign, times -1 if load_neg
-  const int* skip_flag;     // optional: != 0 -> do nothing (see RowsParams)
-  const int* skip_unless_flag;   // optional: == 0 -> do nothing
+  float2* dst;
+  int inv;
+  __device__ float2 load(const LineElem& e) const {
+    float2 v = src[e.g];
+    if (inv) v.y = -v.y;
+    if ((e.i + e.j) & 1) { v.x = -v.x; v.y = -v.y; }
+    return v;
+  }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { dst[e.g] = v; }
 };
 
-// N = H (transform length), CTA owns NCOL = 8*G adjacent columns of one image.
-template <int N>
-__global__ void __launch_bounds__(256) fft_cols_kernel(const ColsParams p) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int NCOL = 8 * G;
-  constexpr int P = fft_pitch(N) + ((fft_pitch(N) % 16 == 0) ? 4 : 0);   // de-conflict the transposed fill
-  if (p.skip_flag && *p.skip_flag != 0) return;
-  if (p.skip_unless_flag && *p.skip_unless_flag == 0) return;
-  __shared__ float2 tw[kTwTotal];
-  extern __shared__ float2 cols_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  fft_load_twiddles(tw, g_tw512);
-  const int b = blockIdx.y;
-  const int c0 = blockIdx.x * NCOL;
-  const size_t img = size_t(b) * p.H * p.W;
-  // load: consecutive threads walk the NCOL contiguous columns of a row
-  for (int e = threadIdx.x; e < N * NCOL; e += blockDim.x) {
-    const int c = e % NCOL, i = e / NCOL;
-    float2 v = (c0 + c < p.W) ? p.src[img + size_t(i) * p.W + c0 + c] : make_float2(0.f, 0.f);
-    if (p.load_conj) v.y = -v.y;
-    if ((p.load_sign && ((i + c0 + c) & 1)) != (p.load_neg != 0)) { v.x = -v.x; v.y = -v.y; }
-    cols_smem[c * P + fpad(i)] = v;
+struct Fft2cCols : LineOp {
+  float2* dst;
+  float norm;               // s / sqrt(HW)
+  int inv;
+  __device__ float2 load(const LineElem& e) const { return dst[e.g]; }
+  __device__ void store(const LineElem& e, float2 v, Pre) const {
+    v.x *= norm; v.y *= norm;
+    if (inv) v.y = -v.y;
+    if ((e.i + e.j) & 1) { v.x = -v.x; v.y = -v.y; }
+    dst[e.g] = v;
   }
-  __syncthreads();
-  float2* mine = cols_smem + warp * G * P;
-  fft_warp_rows<N>(mine, P, tw, lane);
-  if (p.blend) {
-    __syncthreads();
-    const float mu = p.mu[size_t(b) * p.mu_stride];
-    const float inv1mu = 1.f / (1.f + mu);
-    const uint8_t* mk = p.mask + size_t(b) * p.mask_bstride;
-    for (int e = threadIdx.x; e < N * NCOL; e += blockDim.x) {
-      const int c = e % NCOL, i = e / NCOL;
-      if (c0 + c >= p.W) continue;
-      const size_t g = size_t(i) * p.W + c0 + c;
-      float2 Z = cols_smem[c * P + fpad(i)];
-      Z.x *= p.scale1; Z.y *= p.scale1;
-      if (mk[g]) {
-        float2 y = p.y0[img + g];
-        const float sg = ((i + c0 + c) & 1) ? -p.sgn : p.sgn;
-        Z.x = (mu * Z.x + sg * y.x) * inv1mu;
-        Z.y = (mu * Z.y + sg * y.y) * inv1mu;
-      }
-      cols_smem[c * P + fpad(i)] = make_float2(Z.x, -Z.y);   // conj -> forward FFT == inverse
-    }
-    __syncthreads();
-    fft_warp_rows<N>(mine, P, tw, lane);
-  }
-  __syncthreads();
-  for (int e = threadIdx.x; e < N * NCOL; e += blockDim.x) {
-    const int c = e % NCOL, i = e / NCOL;
-    if (c0 + c >= p.W) continue;
-    float2 v = cols_smem[c * P + fpad(i)];
-    v.x *= p.store_scale; v.y *= p.store_scale;
-    if (p.store_conj) v.y = -v.y;
-    if (p.store_sign && ((i + c0 + c) & 1)) { v.x = -v.x; v.y = -v.y; }
-    p.t[img + size_t(i) * p.W + c0 + c] = v;
-  }
-}
+};
 
-template <int N> static void launch_rows(const RowsParams& p, int B, cudaStream_t st) {
-  constexpr int G = FftPlan<N>::G;
-  const size_t smem = size_t(8) * G * fft_pitch(N) * sizeof(float2);
-  dim3 grid((p.H + 8 * G - 1) / (8 * G), B);
-  fft_rows_kernel<N><<<grid, 256, smem, st>>>(p);
-}
-template <int N> static void launch_cols(const ColsParams& p, int B, cudaStream_t st) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int P = fft_pitch(N) + ((fft_pitch(N) % 16 == 0) ? 4 : 0);
-  const size_t smem = size_t(8) * G * P * sizeof(float2);
-  dim3 grid((p.W + 8 * G - 1) / (8 * G), B);
-  fft_cols_kernel<N><<<grid, 256, smem, st>>>(p);
-}
+// prox_prepare: Yt = Fc^-1(s.D.y0) = conj(FFT_col(conj(s.D.y0))) / sqrt(H), read only by the row-only kernels
+struct PrepareYt : LineOp {
+  const float2* y0;
+  float2* yt;
+  float sgn;                // s
+  float norm;               // 1 / sqrt(H)
+  const int* flag;          // == 0 (not every mask is column-only) -> do nothing
+  __device__ bool skip() const { return *flag == 0; }
+  __device__ float2 load(const LineElem& e) const {
+    float2 v = y0[e.g];
+    v.y = -v.y;
+    if ((((e.i + e.j) & 1) != 0) != (sgn < 0.f)) { v.x = -v.x; v.y = -v.y; }
+    return v;
+  }
+  __device__ void store(const LineElem& e, float2 v, Pre) const {
+    v.x *= norm; v.y *= norm;
+    v.y = -v.y;
+    yt[e.g] = v;
+  }
+};
 
 static int launch_cl(const ClParams& p, cudaStream_t st) { return launch_cl_t<16>(p, st); }
 
@@ -246,17 +163,8 @@ static int prox_prepare_cl128(const float2* y0, const uint8_t* mask, long long m
 
 static bool pow2_ok(int n) { return n == 32 || n == 64 || n == 128 || n == 256 || n == 512; }
 
-#define DISPATCH_N(n, fn, ...)                         \
-  switch (n) {                                         \
-    case 32: fn<32>(__VA_ARGS__); break;               \
-    case 64: fn<64>(__VA_ARGS__); break;               \
-    case 128: fn<128>(__VA_ARGS__); break;             \
-    case 256: fn<256>(__VA_ARGS__); break;             \
-    default: fn<512>(__VA_ARGS__); break;              \
-  }
-
 int fft_shape_supported(int H, int W) { return pow2_ok(H) && pow2_ok(W); }
-// every shape some kernel serves: the radix kernels above or the dense-DFT path (fftprox_any.cuh, 2..1024)
+// every shape some kernel serves: the radix passes or the dense-DFT pass (line_passes.cuh, 2..1024)
 int fft_any_shape_supported(int H, int W) { return fft_shape_supported(H, W) || any_shape_supported(H, W); }
 
 // Layout of the prepared buffers (pnp_prox_prepared_bytes), nb = B (per-image masks) or 1:
@@ -305,13 +213,7 @@ int prox_prepare(const float2* y0, const uint8_t* mask, long long mask_bstride, 
     cudaMemcpyAsync(y0p, y0, n * sizeof(float2), cudaMemcpyDeviceToDevice, st);
     cudaMemcpyAsync(maskp, mask, size_t(nb) * H * W, cudaMemcpyDeviceToDevice, st);
   }
-  ColsParams c{};
-  c.H = H; c.W = W; c.t = y0p + n; c.src = y0; c.blend = 0;
-  c.load_sign = 1; c.load_conj = 1; c.load_neg = (((H + W) / 2) & 1) ? 1 : 0;
-  c.store_conj = 1; c.store_scale = 1.0f / sqrtf(float(H));
-  c.skip_unless_flag = flag;                                          // Yt is only read by the row-only kernels
-  DISPATCH_N(H, launch_cols, c, B, st);
-  return int(cudaGetLastError());
+  return radix_cols(PrepareYt{{}, y0, y0p + n, centre_sign(H, W), 1.0f / sqrtf(float(H)), flag}, H, W, B, st);
 }
 
 // The structure flag written by prox_prepare (device int32: != 0 = every mask of the batch depends on the column index only).
@@ -346,15 +248,12 @@ int prox_dual_prepared(const float* x, const float2* u_in, const float2* y0p, co
     return launch_cl128(cp, st);
   }
   if (kind != 0) {
-  SepGenParams gp{x, u_in, y0p + n, rowmask, mask_bstride ? 1 : 0, flag, mu, mu_stride, z_out, u_out, v_out, H, 0, active};
-  switch (W) {
-    case 32: gp.groups_total = B * H / FftPlan<32>::G; launch_sep_generic<32>(gp, num_sms(), st); break;
-    case 64: gp.groups_total = B * H / FftPlan<64>::G; launch_sep_generic<64>(gp, num_sms(), st); break;
-    case 128: gp.groups_total = B * H / FftPlan<128>::G; launch_sep_generic<128>(gp, num_sms(), st); break;
-    case 256: gp.groups_total = B * H / FftPlan<256>::G; launch_sep_generic<256>(gp, num_sms(), st); break;
-    default: gp.groups_total = B * H / FftPlan<512>::G; launch_sep_generic<512>(gp, num_sms(), st); break;
-  }
-  if (kind == 1) return int(cudaGetLastError());
+    SepGenParams gp{x, u_in, y0p + n, rowmask, mask_bstride ? 1 : 0, flag, mu, mu_stride, z_out, u_out, v_out, H, 0, active};
+    with_pow2(W, [&](auto w) {
+      gp.groups_total = B * H / FftPlan<decltype(w)::value>::G;
+      launch_sep_generic<decltype(w)::value>(gp, num_sms(), st);
+    });
+    if (kind == 1) return int(cudaGetLastError());
   }
   // any other mask: the general three-launch path on the copies, gated by the same flag
   return prox_dual_general_impl(x, u_in, y0p, maskp, mask_bstride, mu, mu_stride, z_out, u_out, v_out,
@@ -397,37 +296,22 @@ static int prox_dual_general_impl(const float* x, const float2* u_in, const floa
     }
   }
   const float inv = 1.0f / sqrtf(float(H) * float(W));
-  RowsParams r1{};
-  r1.H = H; r1.W = W; r1.load_mode = ROWS_LOAD_XU; r1.store_mode = ROWS_STORE_C; r1.load_sign = 1;
-  r1.x = x; r1.u = u_in; r1.dst = work; r1.store_scale = 1.f; r1.skip_flag = skip_flag;
-  DISPATCH_N(W, launch_rows, r1, B, st);
-  ColsParams c{};
-  c.H = H; c.W = W; c.t = work; c.src = work; c.blend = 1; c.y0 = y0; c.mask = mask; c.mask_bstride = mask_bstride;
-  c.mu = mu; c.mu_stride = mu_stride; c.scale1 = inv; c.sgn = (((H + W) / 2) & 1) ? -1.f : 1.f;
-  c.store_scale = 1.f; c.skip_flag = skip_flag;
-  DISPATCH_N(H, launch_cols, c, B, st);
-  RowsParams r2{};
-  r2.H = H; r2.W = W; r2.load_mode = ROWS_LOAD_C; r2.store_mode = ROWS_STORE_PROX; r2.src = work;
-  r2.x = x; r2.u = u_in; r2.store_scale = inv; r2.store_conj = 1; r2.store_sign = 1;
-  r2.z_out = z_out; r2.u_out = u_out; r2.v_out = v_out; r2.skip_flag = skip_flag; r2.active = active;
-  DISPATCH_N(W, launch_rows, r2, B, st);
-  return int(cudaGetLastError());
+  int rc = radix_rows(ProxRowsIn{{}, x, u_in, work, skip_flag}, H, W, B, st);
+  if (rc == 0)
+    rc = radix_cols(ProxColsBlend{{{}, y0, mask, mask_bstride, mu, mu_stride}, work, inv, centre_sign(H, W), skip_flag},
+                    H, W, B, st);
+  if (rc == 0)
+    rc = radix_rows(ProxRowsOut{{{}, x, u_in, z_out, u_out, v_out, active}, work, inv, skip_flag}, H, W, B, st);
+  return rc;
 }
 
 // Stand-alone centred orthonormal 2-D transform (mirror of transformations.py fft / ifft). dst may equal src.
 int fft2c_general(const float2* src, float2* dst, int B, int H, int W, int inverse, cudaStream_t st) {
   if (!fft_shape_supported(H, W)) return fft2c_any(src, dst, B, H, W, inverse, st);
   const float inv = 1.0f / sqrtf(float(H) * float(W));
-  const float s = (((H + W) / 2) & 1) ? -1.f : 1.f;
-  RowsParams r{};
-  r.H = H; r.W = W; r.load_mode = ROWS_LOAD_C; r.store_mode = ROWS_STORE_C; r.load_sign = 1; r.load_conj = inverse;
-  r.src = src; r.dst = dst; r.store_scale = 1.f;
-  DISPATCH_N(W, launch_rows, r, B, st);
-  ColsParams c{};
-  c.H = H; c.W = W; c.t = dst; c.src = dst; c.blend = 0; c.store_scale = inv * s; c.store_sign = 1;
-  c.store_conj = inverse;
-  DISPATCH_N(H, launch_cols, c, B, st);
-  return int(cudaGetLastError());
+  int rc = radix_rows(Fft2cRows{{}, src, dst, inverse}, H, W, B, st);
+  if (rc == 0) rc = radix_cols(Fft2cCols{{}, dst, inv * centre_sign(H, W), inverse}, H, W, B, st);
+  return rc;
 }
 
 }  // namespace pnp

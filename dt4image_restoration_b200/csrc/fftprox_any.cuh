@@ -7,230 +7,135 @@
 // is, for EVERY N (even or odd: ifftshift rolls by -h, fftshift by +h),
 //     fft_c(w)[k] = 1/sqrt(N) * sum_m w[m] * omega^((m - h)(k - h)),   omega = exp(-2 pi i / N),
 // and ifft_c (transformations.py:14-19) is the same sum with conj(omega): a dense N x N matrix whose entries are looked up
-// in an N-entry table by the exponent (m - h)(k - h) mod N, walked incrementally.  O(N^2) per line instead of O(N log N):
-// this is the compatibility path (a 130x130 image-iteration is ~35 MFLOP), not the throughput path; k-space coordinates
-// need no rotation and the mask / y0 are read in place (no prepared constants).
+// in an N-entry table by the exponent (m - h)(k - h) mod N, walked incrementally (any_dft_lines, line_passes.cuh).
+// O(N^2) per line instead of O(N log N): this is the compatibility path (a 130x130 image-iteration is ~35 MFLOP), not the
+// throughput path; k-space coordinates need no rotation and the mask / y0 are read in place (no prepared constants).
 //
-// Three launches like the radix general path (fftprox.cu): rows -> work; columns: DFT, blend, inverse DFT in shared
-// memory -> work; rows inverse + dual-update epilogue.  A CTA owns kAnyLines lines (adjacent columns are read as 64-byte
-// row segments); both operand buffers are padded to an odd pitch so that the eight lines of a warp hit distinct banks.
+// Three dense line passes (dense_lines_kernel) like the radix general path (fftprox.cu): rows -> work; columns: DFT,
+// blend, inverse DFT in shared memory -> work; rows inverse + dual-update epilogue.  The blend and the epilogue below are
+// shared with the radix ops of fftprox.cu, which add the centring signs.
 #pragma once
 #include "common.cuh"
+#include "line_passes.cuh"
 
 namespace pnp {
 
-constexpr int kAnyMaxN = 1024;
-constexpr int kAnyLines = 8;
-constexpr int kAnyThreads = 256;
-
-enum { ANY_LOAD_XU = 0, ANY_LOAD_C = 1 };
-enum { ANY_STORE_C = 0, ANY_STORE_PROX = 1 };
-
-struct AnyParams {
-  int H, W;
-  int along_rows;           // 1: a line is an image row (transform over the column index), 0: a line is a column
-  int load_mode, store_mode;
-  int inverse;              // direction of the first transform
-  int blend;                // columns only: forward DFT -> masked k-space solve -> inverse DFT
-  float scale;              // applied to the first transform's output
-  float scale2;             // applied to the second transform's output (blend)
-  const float* x;
-  const float2* u;
-  const float2* src;
-  float2* dst;
-  const float2* y0;
-  const uint8_t* mask;
-  long long mask_bstride;
-  const float* mu;
-  int mu_stride;
-  float2* z_out;
-  float2* u_out;
-  float* v_out;
-  const uint8_t* active;
+// One image's blend constants.
+struct BlendImage {
+  float mu, inv1mu;
+  const uint8_t* mk;
 };
 
-__host__ __device__ inline int any_pitch(int N) { return N | 1; }
-inline size_t any_smem_bytes(int N) { return (size_t(N) + 2 * size_t(kAnyLines) * any_pitch(N)) * sizeof(float2); }
+// Column passes of the prox: blend(Z) = (mu Z + y) / (1 + mu) under the mask, Z elsewhere (env.py:88-90).
+struct ProxBlendOp : LineOp {
+  static constexpr bool kMiddle = true;
+  const float2* y0;         // [B,H,W]
+  const uint8_t* mask;      // [mask_B,H,W]
+  long long mask_bstride;   // 0 when one mask is shared by the batch
+  const float* mu;          // [B] or [1]
+  int mu_stride;
+  __device__ BlendImage middle_begin(int b) const {
+    const float m = mu[size_t(b) * mu_stride];
+    return {m, 1.f / (1.f + m), mask + size_t(b) * mask_bstride};
+  }
+  // y: y0 at the sample, times the centring sign where the transform leaves one
+  __device__ static float2 blend(const BlendImage& m, float2 Z, float2 y) {
+    return make_float2((m.mu * Z.x + y.x) * m.inv1mu, (m.mu * Z.y + y.y) * m.inv1mu);
+  }
+};
 
-// out[l][k] = scale * sum_m in[l][m] * tw[((m - h)(k - h)) mod N]  (tw holds the conjugates for the inverse direction)
-__device__ __forceinline__ void any_dft_lines(const float2* __restrict__ in, float2* __restrict__ out,
-                                              const float2* __restrict__ tw, int N, int P, int nl, float scale) {
-  const int h = N / 2;
-  for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-    const int l = e % kAnyLines, k = e / kAnyLines;
-    if (l >= nl) continue;
-    const int step = (k >= h) ? (k - h) : (k - h + N);                       // (k - h) mod N
-    int ex = int((long long)(N - h) % N * step % N);                          // (0 - h)(k - h) mod N
-    const float2* a = in + l * P;
-    float2 acc0 = make_float2(0.f, 0.f), acc1 = make_float2(0.f, 0.f);
-    int m = 0;
-    for (; m + 1 < N; m += 2) {
-      const float2 w0 = tw[ex];
-      ex += step; if (ex >= N) ex -= N;
-      const float2 w1 = tw[ex];
-      ex += step; if (ex >= N) ex -= N;
-      const float2 v0 = a[m], v1 = a[m + 1];
-      acc0.x = fmaf(v0.x, w0.x, acc0.x); acc0.x = fmaf(-v0.y, w0.y, acc0.x);
-      acc0.y = fmaf(v0.x, w0.y, acc0.y); acc0.y = fmaf(v0.y, w0.x, acc0.y);
-      acc1.x = fmaf(v1.x, w1.x, acc1.x); acc1.x = fmaf(-v1.y, w1.y, acc1.x);
-      acc1.y = fmaf(v1.x, w1.y, acc1.y); acc1.y = fmaf(v1.y, w1.x, acc1.y);
-    }
-    if (m < N) {
-      const float2 w0 = tw[ex];
-      const float2 v0 = a[m];
-      acc0.x = fmaf(v0.x, w0.x, acc0.x); acc0.x = fmaf(-v0.y, w0.y, acc0.x);
-      acc0.y = fmaf(v0.x, w0.y, acc0.y); acc0.y = fmaf(v0.y, w0.x, acc0.y);
-    }
-    out[l * P + k] = make_float2((acc0.x + acc1.x) * scale, (acc0.y + acc1.y) * scale);
+// Row-out stores of the prox: z, u' = u + x - z (env.py:93), v' = Re(z - u') (the next denoiser input).  u and x are
+// plain loads (u_out may alias u), fetched by preload().
+struct ProxDualOp : LineOp {
+  const float* x;           // [B,H,W]
+  const float2* u;          // [B,H,W]
+  float2* z_out;
+  float2* u_out;
+  float* v_out;             // may be null
+  const uint8_t* active;    // optional [B]: 0 = leave the image's z, u, v untouched
+  struct Pre {
+    float2 u;
+    float x;
+  };
+  __device__ bool image_active(int b) const { return !(active && active[b] == 0); }
+  __device__ Pre preload(const LineElem& e) const { return {u[e.g], x[e.g]}; }
+  __device__ void store_dual(size_t g, float2 z, const Pre& p) const {
+    const float2 un = make_float2(p.u.x + p.x - z.x, p.u.y - z.y);
+    z_out[g] = z;
+    u_out[g] = un;
+    if (v_out) v_out[g] = z.x - un.x;
   }
-}
+};
 
-__global__ void __launch_bounds__(kAnyThreads) dft_any_kernel(const AnyParams p) {
-  extern __shared__ float2 any_sm[];
-  const int N = p.along_rows ? p.W : p.H;              // transform length
-  const int nlines = p.along_rows ? p.H : p.W;
-  const int P = any_pitch(N);
-  float2* tw = any_sm;                                 // forward table exp(-2 pi i k / N)
-  float2* bufa = tw + N;
-  float2* bufc = bufa + kAnyLines * P;
-  const int b = blockIdx.y, l0 = blockIdx.x * kAnyLines;
-  const int nl = min(kAnyLines, nlines - l0);
-  const size_t img = size_t(b) * p.H * p.W;
-  const bool inv1 = p.inverse != 0;
-  for (int k = threadIdx.x; k < N; k += kAnyThreads) {
-    float s, c;
-    sincospif(2.0f * float(k) / float(N), &s, &c);
-    tw[k] = make_float2(c, inv1 ? s : -s);
+// ---- dense ops: the transforms are centred and scaled inside any_dft_lines
+struct ProxAnyRowsIn : LineOp {
+  static constexpr bool kRows = true;
+  const float* x;
+  const float2* u;
+  float2* work;
+  float norm;               // 1 / sqrt(W)
+  __device__ bool inverse() const { return false; }
+  __device__ float scale(int) const { return norm; }
+  __device__ float2 load(const LineElem& e) const {
+    const float2 uu = u[e.g];
+    return make_float2(x[e.g] + uu.x, uu.y);
   }
-  // ---- load: consecutive threads walk memory-contiguous elements ----
-  for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-    int l, m;
-    size_t g;
-    if (p.along_rows) { l = e / N; m = e % N; g = img + size_t(l0 + l) * p.W + m; }
-    else              { l = e % kAnyLines; m = e / kAnyLines; g = img + size_t(m) * p.W + l0 + l; }
-    if (l >= nl) continue;
-    float2 v;
-    if (p.load_mode == ANY_LOAD_XU) {
-      const float2 uu = p.u[g];
-      v = make_float2(p.x[g] + uu.x, uu.y);
-    } else {
-      v = p.src[g];
-    }
-    bufa[l * P + m] = v;
-  }
-  __syncthreads();
-  any_dft_lines(bufa, bufc, tw, N, P, nl, p.scale);
-  __syncthreads();
-  const float2* res = bufc;
-  if (p.blend) {                                       // lines are columns: element (l, k) is k-space sample (row k, column l0 + l)
-    const float mu = p.mu[size_t(b) * p.mu_stride];
-    const float inv1mu = 1.f / (1.f + mu);
-    const uint8_t* mk = p.mask + size_t(b) * p.mask_bstride;
-    for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-      const int l = e % kAnyLines, k = e / kAnyLines;
-      if (l >= nl) continue;
-      const size_t g = size_t(k) * p.W + l0 + l;
-      if (mk[g]) {
-        const float2 y = p.y0[img + g];
-        float2 Z = bufc[l * P + k];
-        Z.x = (mu * Z.x + y.x) * inv1mu;               // env.py:88-90
-        Z.y = (mu * Z.y + y.y) * inv1mu;
-        bufc[l * P + k] = Z;
-      }
-    }
-    for (int k = threadIdx.x; k < N; k += kAnyThreads) tw[k].y = -tw[k].y;   // own entries only: no barrier needed before
-    __syncthreads();
-    any_dft_lines(bufc, bufa, tw, N, P, nl, p.scale2);
-    __syncthreads();
-    res = bufa;
-  }
-  // ---- store ----
-  const bool act = !(p.active && p.active[b] == 0);
-  for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-    int l, m;
-    size_t g;
-    if (p.along_rows) { l = e / N; m = e % N; g = img + size_t(l0 + l) * p.W + m; }
-    else              { l = e % kAnyLines; m = e / kAnyLines; g = img + size_t(m) * p.W + l0 + l; }
-    if (l >= nl) continue;
-    const float2 v = res[l * P + m];
-    if (p.store_mode == ANY_STORE_C) {
-      p.dst[g] = v;
-    } else if (act) {
-      const float2 uu = p.u[g];
-      const float xx = p.x[g];
-      const float2 un = make_float2(uu.x + xx - v.x, uu.y - v.y);            // u' = u + x - z   (env.py:93)
-      p.z_out[g] = v;
-      p.u_out[g] = un;
-      if (p.v_out) p.v_out[g] = v.x - un.x;                                  // Re(z - u'): the next denoiser input
-    }
-  }
-}
+  __device__ void store(const LineElem& e, float2 v, Pre) const { work[e.g] = v; }
+};
 
-inline bool any_shape_supported(int H, int W) { return H >= 2 && W >= 2 && H <= kAnyMaxN && W <= kAnyMaxN; }
+struct ProxAnyColsBlend : ProxBlendOp {
+  static constexpr bool kRows = false;
+  float2* work;
+  float norm;               // 1 / sqrt(H)
+  __device__ bool inverse() const { return false; }
+  __device__ float scale(int) const { return norm; }
+  __device__ float2 load(const LineElem& e) const { return work[e.g]; }
+  __device__ float2 middle(const BlendImage& m, const LineElem& e, float2 Z) const {
+    return m.mk[e.o] ? blend(m, Z, y0[e.g]) : Z;
+  }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { work[e.g] = v; }
+};
 
-static int launch_any(const AnyParams& p, int B, cudaStream_t st) {
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(dft_any_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         int(any_smem_bytes(kAnyMaxN)));
-    if (e != cudaSuccess) return int(e);
-    attr_done = true;
-  }
-  const int N = p.along_rows ? p.W : p.H, nlines = p.along_rows ? p.H : p.W;
-  for (int b0 = 0; b0 < B; b0 += 65535) {              // grid.y limit
-    AnyParams q = p;
-    const size_t off = size_t(b0) * p.H * p.W;
-    if (q.x) q.x += off;
-    if (q.u) q.u += off;
-    if (q.src) q.src += off;
-    if (q.dst) q.dst += off;
-    if (q.y0) q.y0 += off;
-    if (q.mask) q.mask += size_t(b0) * p.mask_bstride;
-    if (q.mu) q.mu += size_t(b0) * p.mu_stride;
-    if (q.z_out) q.z_out += off;
-    if (q.u_out) q.u_out += off;
-    if (q.v_out) q.v_out += off;
-    if (q.active) q.active += b0;
-    const int nb = (B - b0 < 65535) ? (B - b0) : 65535;
-    dft_any_kernel<<<dim3((nlines + kAnyLines - 1) / kAnyLines, nb), kAnyThreads, any_smem_bytes(N), st>>>(q);
-  }
-  return int(cudaGetLastError());
-}
+struct ProxAnyRowsOut : ProxDualOp {
+  static constexpr bool kRows = true;
+  const float2* work;
+  float norm;               // 1 / sqrt(W)
+  __device__ bool inverse() const { return true; }
+  __device__ float scale(int) const { return norm; }
+  __device__ float2 load(const LineElem& e) const { return work[e.g]; }
+  __device__ void store(const LineElem& e, float2 v, const Pre& p) const { store_dual(e.g, v, p); }
+};
+
+template <bool ROWS> struct Fft2cAny : LineOp {
+  static constexpr bool kRows = ROWS;
+  const float2* src;
+  float2* dst;
+  float norm;               // 1 / sqrt(length)
+  int inv;
+  __device__ bool inverse() const { return inv != 0; }
+  __device__ float scale(int) const { return norm; }
+  __device__ float2 load(const LineElem& e) const { return src[e.g]; }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { dst[e.g] = v; }
+};
 
 // z = ifft_c(blend(fft_c(x + u))), u' = u + x - z, v' = Re(z - u') for any H, W in 2..1024; `work` = c64 [B,H,W] scratch.
 static int prox_dual_any(const float* x, const float2* u_in, const float2* y0, const uint8_t* mask, long long mask_bstride,
                          const float* mu, int mu_stride, float2* z_out, float2* u_out, float* v_out, float2* work, int B,
                          int H, int W, cudaStream_t st, const uint8_t* active) {
   if (!any_shape_supported(H, W)) return -2;
-  AnyParams r1{};
-  r1.H = H; r1.W = W; r1.along_rows = 1; r1.load_mode = ANY_LOAD_XU; r1.store_mode = ANY_STORE_C;
-  r1.x = x; r1.u = u_in; r1.dst = work; r1.scale = 1.0f / sqrtf(float(W));
-  int rc = launch_any(r1, B, st);
-  if (rc) return rc;
-  AnyParams c{};
-  c.H = H; c.W = W; c.along_rows = 0; c.load_mode = ANY_LOAD_C; c.store_mode = ANY_STORE_C; c.blend = 1;
-  c.src = work; c.dst = work; c.scale = 1.0f / sqrtf(float(H)); c.scale2 = c.scale;
-  c.y0 = y0; c.mask = mask; c.mask_bstride = mask_bstride; c.mu = mu; c.mu_stride = mu_stride;
-  rc = launch_any(c, B, st);
-  if (rc) return rc;
-  AnyParams r2{};
-  r2.H = H; r2.W = W; r2.along_rows = 1; r2.load_mode = ANY_LOAD_C; r2.store_mode = ANY_STORE_PROX; r2.inverse = 1;
-  r2.src = work; r2.x = x; r2.u = u_in; r2.scale = 1.0f / sqrtf(float(W));
-  r2.z_out = z_out; r2.u_out = u_out; r2.v_out = v_out; r2.active = active;
-  return launch_any(r2, B, st);
+  const float nw = 1.0f / sqrtf(float(W)), nh = 1.0f / sqrtf(float(H));
+  int rc = dense_lines(ProxAnyRowsIn{{}, x, u_in, work, nw}, H, W, B, st);
+  if (rc == 0) rc = dense_lines(ProxAnyColsBlend{{{}, y0, mask, mask_bstride, mu, mu_stride}, work, nh}, H, W, B, st);
+  if (rc == 0) rc = dense_lines(ProxAnyRowsOut{{{}, x, u_in, z_out, u_out, v_out, active}, work, nw}, H, W, B, st);
+  return rc;
 }
 
 // Stand-alone centred orthonormal 2-D transform for any H, W in 2..1024 (dst may equal src).
 static int fft2c_any(const float2* src, float2* dst, int B, int H, int W, int inverse, cudaStream_t st) {
   if (!any_shape_supported(H, W)) return -2;
-  AnyParams r{};
-  r.H = H; r.W = W; r.along_rows = 1; r.load_mode = ANY_LOAD_C; r.store_mode = ANY_STORE_C; r.inverse = inverse;
-  r.src = src; r.dst = dst; r.scale = 1.0f / sqrtf(float(W));
-  int rc = launch_any(r, B, st);
-  if (rc) return rc;
-  AnyParams c = r;
-  c.along_rows = 0; c.src = dst; c.scale = 1.0f / sqrtf(float(H));
-  return launch_any(c, B, st);
+  int rc = dense_lines(Fft2cAny<true>{{}, src, dst, 1.0f / sqrtf(float(W)), inverse}, H, W, B, st);
+  if (rc == 0) rc = dense_lines(Fft2cAny<false>{{}, dst, dst, 1.0f / sqrtf(float(H)), inverse}, H, W, B, st);
+  return rc;
 }
 
 }  // namespace pnp

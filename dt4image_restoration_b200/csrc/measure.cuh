@@ -11,14 +11,15 @@
 //   cols : load columns of T -> col FFT -> s.D / sqrt(HW) = K -> noise, mask -> y0 (stored)
 //          -> conj(D.y0) -> col FFT                                                          -> T
 //   rows : load T -> row FFTs -> conj, s.D / sqrt(HW) = ATy0 -> x0 (and ATy0)
-// with D[i,j] = (-1)^(i+j), s = (-1)^((H+W)/2) as in fftprox.cu.  Powers of two in 32..512 take the radix kernels below
-// (fft_core.cuh); every other H, W in 2..1024 takes the dense-DFT kernel (any_dft_lines, fftprox_any.cuh), which computes
-// the centred transforms directly.  The noise of a sample depends only on (seed, H, W, i, j), never on the mask or the batch
+// with D[i,j] = (-1)^(i+j), s = (-1)^((H+W)/2) as in fftprox.cu.  The passes are ops on the line passes of
+// line_passes.cuh: powers of two in 32..512 take the radix passes (SimRowsFwd, SimCols, SimRowsInv); every other H, W in
+// 2..1024 takes the dense-DFT pass (SimAnyRowsFwd, SimAnyCols, SimAnyRowsInv), which computes the centred transforms
+// directly.  The noise of a sample depends only on (seed, H, W, i, j), never on the mask or the batch
 // position, and nothing is accumulated across CTAs, so every output is bitwise reproducible.
 #pragma once
 #include "common.cuh"
 #include "fft_core.cuh"
-#include "fftprox_any.cuh"
+#include "line_passes.cuh"
 
 namespace pnp {
 
@@ -58,203 +59,126 @@ __device__ __forceinline__ float2 measure_sample(float2 K, bool sampled, int i, 
   return make_float2(fmaf(sig, n.x, K.x), fmaf(sig, n.y, K.y));
 }
 
-struct SimParams {
-  int H, W;
-  const float* gt;              // [B or 1, H, W]
-  long long gt_bstride;         // H*W, or 0 for one shared gt
+// ---------------------------------------------------------------- ops of the three line passes (line_passes.cuh)
+// Column passes: K -> y0 at k-space sample (i, j), stored; the y0 the second transform starts from.
+struct SimSampleOp : LineOp {
+  static constexpr bool kMiddle = true;
   const uint8_t* mask;          // [B or 1, H, W]
   long long mask_bstride;
   const float* sigma;           // sigma_n[b * sigma_stride]
   int sigma_stride;
   const unsigned long long* seeds;   // [B]
   float2* y0;                   // [B, H, W]
-  float2* x0;                   // [B, H, W]; holds T between the passes
-  float2* aty0;                 // [B, H, W] or null
-  float kscale;                 // radix: s / sqrt(HW)
-  int gt_vec4;                  // radix rows pass: every image's gt is 16-byte aligned
+  int W;
+  struct Mid {
+    float sig;
+    uint2 key;
+    const uint8_t* mk;
+  };
+  __device__ Mid middle_begin(int b) const {
+    return {sigma[size_t(b) * sigma_stride] * (1.f / 255.f), seed_key(seeds[b]), mask + size_t(b) * mask_bstride};
+  }
+  __device__ float2 sample(const Mid& m, const LineElem& e, float2 K) const {
+    const float2 y = measure_sample(K, m.mk[e.o] != 0, e.i, e.j, W, m.sig, m.key);
+    y0[e.g] = y;
+    return y;
+  }
 };
 
-// ---------------------------------------------------------------- radix path (H, W powers of two in 32..512)
-// Pass 1: D.gt -> row FFTs -> T.  N = W; a warp owns G consecutive rows (G*N contiguous floats).
-template <int N>
-__global__ void __launch_bounds__(256) sim_rows_fwd_kernel(const SimParams p) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int P = fft_pitch(N);
-  __shared__ float2 tw[kTwTotal];
-  extern __shared__ float2 sim_rows_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  fft_load_twiddles(tw, g_tw512);
-  __syncthreads();
-  const int b = blockIdx.y;
-  const int row0 = (blockIdx.x * 8 + warp) * G;
-  if (row0 >= p.H) return;
-  float2* mine = sim_rows_smem + warp * G * P;
-  const float* g = p.gt + size_t(b) * p.gt_bstride + size_t(row0) * N;
-  if (p.gt_vec4) {
+// radix path (H, W powers of two in 32..512).  Pass 1: D.gt -> row FFTs -> T.
+struct SimRowsFwd : LineOp {
+  template <int N> static constexpr int kRowCtas = N == 128 ? 8 : 0;   // left alone, ptxas spills at N = 128
+  const float* gt;              // [B or 1, H, W]
+  long long gt_bstride;         // H*W, or 0 for one shared gt
+  float2* t;                    // x0
+  int gt_vec4;                  // every image's gt is 16-byte aligned
+  // float4 loads: a warp's G rows are G*N contiguous floats
+  template <int N> __device__ bool load_rows(float2* rows, int b, int row0, int lane) const {
+    if (!gt_vec4) return false;
+    constexpr int G = FftPlan<N>::G, P = fft_pitch(N);
+    const float* g = gt + size_t(b) * gt_bstride + size_t(row0) * N;
     for (int q = lane; q < G * N / 4; q += 32) {
       const float4 v = reinterpret_cast<const float4*>(g)[q];
       const int r = (4 * q) / N, j = (4 * q) % N;
       const float s = ((row0 + r) & 1) ? -1.f : 1.f;     // D at the even column j
-      float2* d = mine + r * P;
+      float2* d = rows + r * P;
       d[fpad(j)] = make_float2(s * v.x, 0.f);
       d[fpad(j + 1)] = make_float2(-s * v.y, 0.f);
       d[fpad(j + 2)] = make_float2(s * v.z, 0.f);
       d[fpad(j + 3)] = make_float2(-s * v.w, 0.f);
     }
-  } else {
-    for (int e = lane; e < G * N; e += 32) {
-      const int r = e / N, j = e % N;
-      const float v = g[e];
-      mine[r * P + fpad(j)] = make_float2(((row0 + r + j) & 1) ? -v : v, 0.f);
-    }
+    return true;
   }
-  __syncwarp();
-  fft_warp_rows<N>(mine, P, tw, lane);
-  float2* t = p.x0 + size_t(b) * p.H * N + size_t(row0) * N;
-  for (int e = lane; e < G * N; e += 32) t[e] = mine[(e / N) * P + fpad(e % N)];
-}
+  __device__ float2 load(const LineElem& e) const {
+    const float v = gt[size_t(e.b) * gt_bstride + e.o];
+    return make_float2(((e.i + e.j) & 1) ? -v : v, 0.f);
+  }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { t[e.g] = v; }
+};
 
-// Pass 2: columns of T -> col FFT -> K -> y0 -> conj(D.y0) -> col FFT -> T.  N = H; a CTA owns NCOL = 8*G adjacent
-// columns of one image, so the loads and the y0 / T stores walk NCOL contiguous elements of a row.
-template <int N>
-__global__ void __launch_bounds__(256) sim_cols_kernel(const SimParams p) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int NCOL = 8 * G;
-  constexpr int P = fft_pitch(N) + ((fft_pitch(N) % 16 == 0) ? 4 : 0);   // de-conflict the transposed fill
-  __shared__ float2 tw[kTwTotal];
-  extern __shared__ float2 sim_cols_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  fft_load_twiddles(tw, g_tw512);
-  const int b = blockIdx.y, W = p.W;
-  const int c0 = blockIdx.x * NCOL;
-  float2* t = p.x0 + size_t(b) * N * W;
-  for (int e = threadIdx.x; e < N * NCOL; e += blockDim.x) {
-    const int c = e % NCOL, i = e / NCOL;
-    sim_cols_smem[c * P + fpad(i)] = (c0 + c < W) ? t[size_t(i) * W + c0 + c] : make_float2(0.f, 0.f);
+// Pass 2: columns of T -> col FFT -> K = s.D / sqrt(HW) -> y0 -> conj(D.y0) -> col FFT -> T.
+struct SimCols : SimSampleOp {
+  float2* t;
+  float kscale;                 // s / sqrt(HW)
+  __device__ float2 load(const LineElem& e) const { return t[e.g]; }
+  __device__ float2 middle(const Mid& m, const LineElem& e, float2 Z) const {
+    const float d = ((e.i + e.j) & 1) ? -kscale : kscale;
+    const float2 y = sample(m, e, make_float2(Z.x * d, Z.y * d));
+    const float dy = ((e.i + e.j) & 1) ? -1.f : 1.f;
+    return make_float2(dy * y.x, -dy * y.y);   // conj(D.y0): forward FFT == inverse
   }
-  __syncthreads();
-  float2* mine = sim_cols_smem + warp * G * P;
-  fft_warp_rows<N>(mine, P, tw, lane);
-  __syncthreads();
-  const float sig = p.sigma[size_t(b) * p.sigma_stride] * (1.f / 255.f);
-  const uint2 key = seed_key(p.seeds[b]);
-  const uint8_t* mk = p.mask + size_t(b) * p.mask_bstride;
-  float2* y0 = p.y0 + size_t(b) * N * W;
-  for (int e = threadIdx.x; e < N * NCOL; e += blockDim.x) {
-    const int c = e % NCOL, i = e / NCOL, j = c0 + c;
-    if (j >= W) continue;
-    const float d = ((i + j) & 1) ? -p.kscale : p.kscale;
-    const float2 Z = sim_cols_smem[c * P + fpad(i)];
-    const float2 y = measure_sample(make_float2(Z.x * d, Z.y * d), mk[size_t(i) * W + j] != 0, i, j, W, sig, key);
-    y0[size_t(i) * W + j] = y;
-    const float dy = ((i + j) & 1) ? -1.f : 1.f;
-    sim_cols_smem[c * P + fpad(i)] = make_float2(dy * y.x, -dy * y.y);   // conj(D.y0): forward FFT == inverse
-  }
-  __syncthreads();
-  fft_warp_rows<N>(mine, P, tw, lane);
-  __syncthreads();
-  for (int e = threadIdx.x; e < N * NCOL; e += blockDim.x) {
-    const int c = e % NCOL, i = e / NCOL;
-    if (c0 + c < W) t[size_t(i) * W + c0 + c] = sim_cols_smem[c * P + fpad(i)];
-  }
-}
+  __device__ void store(const LineElem& e, float2 v, Pre) const { t[e.g] = v; }
+};
 
-// Pass 3: T -> row FFTs -> ATy0 = s.D.conj(.) / sqrt(HW) -> x0 = max(ATy0, 0) (and ATy0).  N = W.
-template <int N>
-__global__ void __launch_bounds__(256) sim_rows_inv_kernel(const SimParams p) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int P = fft_pitch(N);
-  __shared__ float2 tw[kTwTotal];
-  extern __shared__ float2 sim_rows_smem[];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  fft_load_twiddles(tw, g_tw512);
-  __syncthreads();
-  const int b = blockIdx.y;
-  const int row0 = (blockIdx.x * 8 + warp) * G;
-  if (row0 >= p.H) return;
-  float2* mine = sim_rows_smem + warp * G * P;
-  const size_t base = size_t(b) * p.H * N + size_t(row0) * N;
-  for (int e = lane; e < G * N; e += 32) mine[(e / N) * P + fpad(e % N)] = p.x0[base + e];
-  __syncwarp();
-  fft_warp_rows<N>(mine, P, tw, lane);
-  for (int e = lane; e < G * N; e += 32) {
-    const int r = e / N, j = e % N;
-    const float2 v = mine[r * P + fpad(j)];
-    const float d = ((row0 + r + j) & 1) ? -p.kscale : p.kscale;
+// Pass 3: T -> row FFTs -> ATy0 = s.D.conj(.) / sqrt(HW) -> x0 = max(ATy0, 0) (and ATy0).
+struct SimRowsInv : LineOp {
+  float2* x0;                   // [B, H, W]; holds T between the passes
+  float2* aty0;                 // [B, H, W] or null
+  float kscale;
+  __device__ float2 load(const LineElem& e) const { return x0[e.g]; }
+  __device__ void store(const LineElem& e, float2 v, Pre) const {
+    const float d = ((e.i + e.j) & 1) ? -kscale : kscale;
     const float2 a = make_float2(v.x * d, -v.y * d);
-    if (p.aty0) p.aty0[base + e] = a;
-    p.x0[base + e] = make_float2(fmaxf(a.x, 0.f), fmaxf(a.y, 0.f));
+    if (aty0) aty0[e.g] = a;
+    x0[e.g] = make_float2(fmaxf(a.x, 0.f), fmaxf(a.y, 0.f));
   }
-}
+};
 
-// ---------------------------------------------------------------- dense-DFT path (every other H, W in 2..1024)
-// PASS 0: gt rows -> fft_c along rows -> T;  PASS 1: columns of T -> fft_c -> y0 -> ifft_c -> T;
-// PASS 2: rows of T -> ifft_c along rows -> x0, ATy0.  A CTA owns kAnyLines lines, as dft_any_kernel.
-template <int PASS>
-__global__ void __launch_bounds__(kAnyThreads) sim_any_kernel(const SimParams p) {
-  extern __shared__ float2 sim_any_smem[];
-  constexpr bool kRows = PASS != 1;
-  const int W = p.W;
-  const int N = kRows ? W : p.H;
-  const int nlines = kRows ? p.H : W;
-  const int P = any_pitch(N);
-  float2* tw = sim_any_smem;
-  float2* bufa = tw + N;
-  float2* bufc = bufa + kAnyLines * P;
-  const int b = blockIdx.y, l0 = blockIdx.x * kAnyLines;
-  const int nl = min(kAnyLines, nlines - l0);
-  const size_t img = size_t(b) * p.H * W;
-  const float scale = rsqrtf(float(N));
-  for (int k = threadIdx.x; k < N; k += kAnyThreads) {
-    float s, c;
-    sincospif(2.0f * float(k) / float(N), &s, &c);
-    tw[k] = make_float2(c, PASS == 2 ? s : -s);
+// dense-DFT path (every other H, W in 2..1024): gt rows -> fft_c along rows -> T; columns of T -> fft_c -> y0 -> ifft_c
+// -> T; rows of T -> ifft_c along rows -> x0, ATy0.
+struct SimAnyRowsFwd : LineOp {
+  static constexpr bool kRows = true;
+  const float* gt;
+  long long gt_bstride;
+  float2* t;
+  __device__ bool inverse() const { return false; }
+  __device__ float scale(int N) const { return rsqrtf(float(N)); }
+  __device__ float2 load(const LineElem& e) const { return make_float2(gt[size_t(e.b) * gt_bstride + e.o], 0.f); }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { t[e.g] = v; }
+};
+
+struct SimAnyCols : SimSampleOp {
+  static constexpr bool kRows = false;
+  float2* t;
+  __device__ bool inverse() const { return false; }
+  __device__ float scale(int N) const { return rsqrtf(float(N)); }
+  __device__ float2 load(const LineElem& e) const { return t[e.g]; }
+  __device__ float2 middle(const Mid& m, const LineElem& e, float2 K) const { return sample(m, e, K); }
+  __device__ void store(const LineElem& e, float2 v, Pre) const { t[e.g] = v; }
+};
+
+struct SimAnyRowsInv : LineOp {
+  static constexpr bool kRows = true;
+  float2* x0;
+  float2* aty0;
+  __device__ bool inverse() const { return true; }
+  __device__ float scale(int N) const { return rsqrtf(float(N)); }
+  __device__ float2 load(const LineElem& e) const { return x0[e.g]; }
+  __device__ void store(const LineElem& e, float2 v, Pre) const {
+    if (aty0) aty0[e.g] = v;
+    x0[e.g] = make_float2(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f));
   }
-  for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-    int l, m;
-    size_t g;
-    if (kRows) { l = e / N; m = e % N; g = size_t(l0 + l) * W + m; }
-    else       { l = e % kAnyLines; m = e / kAnyLines; g = size_t(m) * W + l0 + l; }
-    if (l >= nl) continue;
-    bufa[l * P + m] = (PASS == 0) ? make_float2(p.gt[size_t(b) * p.gt_bstride + g], 0.f) : p.x0[img + g];
-  }
-  __syncthreads();
-  any_dft_lines(bufa, bufc, tw, N, P, nl, scale);
-  __syncthreads();
-  const float2* res = bufc;
-  if (PASS == 1) {                                     // element (l, k) is k-space sample (row k, column l0 + l)
-    const float sig = p.sigma[size_t(b) * p.sigma_stride] * (1.f / 255.f);
-    const uint2 key = seed_key(p.seeds[b]);
-    const uint8_t* mk = p.mask + size_t(b) * p.mask_bstride;
-    for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-      const int l = e % kAnyLines, k = e / kAnyLines;
-      if (l >= nl) continue;
-      const size_t g = size_t(k) * W + l0 + l;
-      const float2 y = measure_sample(bufc[l * P + k], mk[g] != 0, k, l0 + l, W, sig, key);
-      p.y0[img + g] = y;
-      bufc[l * P + k] = y;
-    }
-    for (int k = threadIdx.x; k < N; k += kAnyThreads) tw[k].y = -tw[k].y;   // own entries only: no barrier needed before
-    __syncthreads();
-    any_dft_lines(bufc, bufa, tw, N, P, nl, scale);
-    __syncthreads();
-    res = bufa;
-  }
-  for (int e = threadIdx.x; e < kAnyLines * N; e += kAnyThreads) {
-    int l, m;
-    size_t g;
-    if (kRows) { l = e / N; m = e % N; g = size_t(l0 + l) * W + m; }
-    else       { l = e % kAnyLines; m = e / kAnyLines; g = size_t(m) * W + l0 + l; }
-    if (l >= nl) continue;
-    const float2 v = res[l * P + m];
-    if (PASS != 2) {
-      p.x0[img + g] = v;
-    } else {
-      if (p.aty0) p.aty0[img + g] = v;
-      p.x0[img + g] = make_float2(fmaxf(v.x, 0.f), fmaxf(v.y, 0.f));
-    }
-  }
-}
+};
 
 // ---------------------------------------------------------------- Cartesian masks: one CTA per image
 constexpr int kMaskThreads = 256;
@@ -400,87 +324,23 @@ __global__ void __launch_bounds__(kRadialThreads) radial_mask_kernel(const doubl
 }
 
 // ---------------------------------------------------------------- host side
-// Launch `fn(q, nb)` over batch chunks of at most 65535 images (grid.y limit), q's pointers advanced to the chunk.
-template <typename F>
-static void for_batch_chunks(const SimParams& p, int B, F&& fn) {
-  for (int b0 = 0; b0 < B; b0 += 65535) {
-    SimParams q = p;
-    const size_t off = size_t(b0) * p.H * p.W;
-    q.gt += size_t(b0) * p.gt_bstride;
-    q.mask += size_t(b0) * p.mask_bstride;
-    q.sigma += size_t(b0) * p.sigma_stride;
-    q.seeds += b0;
-    q.y0 += off;
-    q.x0 += off;
-    if (q.aty0) q.aty0 += off;
-    fn(q, (B - b0 < 65535) ? (B - b0) : 65535);
-  }
-}
-
-template <int N> static void sim_launch_rows_fwd(const SimParams& p, int B, cudaStream_t st) {
-  constexpr int G = FftPlan<N>::G;
-  const size_t smem = size_t(8) * G * fft_pitch(N) * sizeof(float2);
-  for_batch_chunks(p, B, [&](const SimParams& q, int nb) {
-    sim_rows_fwd_kernel<N><<<dim3((p.H + 8 * G - 1) / (8 * G), nb), 256, smem, st>>>(q);
-  });
-}
-template <int N> static void sim_launch_rows_inv(const SimParams& p, int B, cudaStream_t st) {
-  constexpr int G = FftPlan<N>::G;
-  const size_t smem = size_t(8) * G * fft_pitch(N) * sizeof(float2);
-  for_batch_chunks(p, B, [&](const SimParams& q, int nb) {
-    sim_rows_inv_kernel<N><<<dim3((p.H + 8 * G - 1) / (8 * G), nb), 256, smem, st>>>(q);
-  });
-}
-template <int N> static void sim_launch_cols(const SimParams& p, int B, cudaStream_t st) {
-  constexpr int G = FftPlan<N>::G;
-  constexpr int P = fft_pitch(N) + ((fft_pitch(N) % 16 == 0) ? 4 : 0);
-  const size_t smem = size_t(8) * G * P * sizeof(float2);
-  for_batch_chunks(p, B, [&](const SimParams& q, int nb) {
-    sim_cols_kernel<N><<<dim3((p.W + 8 * G - 1) / (8 * G), nb), 256, smem, st>>>(q);
-  });
-}
-
-template <int PASS> static int sim_launch_any(const SimParams& p, int B, cudaStream_t st) {
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(sim_any_kernel<PASS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         int(any_smem_bytes(kAnyMaxN)));
-    if (e != cudaSuccess) return int(e);
-    attr_done = true;
-  }
-  const int N = (PASS != 1) ? p.W : p.H, nlines = (PASS != 1) ? p.H : p.W;
-  for_batch_chunks(p, B, [&](const SimParams& q, int nb) {
-    sim_any_kernel<PASS><<<dim3((nlines + kAnyLines - 1) / kAnyLines, nb), kAnyThreads, any_smem_bytes(N), st>>>(q);
-  });
-  return int(cudaGetLastError());
-}
-
-#define SIM_DISPATCH_N(n, fn, ...)                     \
-  switch (n) {                                         \
-    case 32: fn<32>(__VA_ARGS__); break;               \
-    case 64: fn<64>(__VA_ARGS__); break;               \
-    case 128: fn<128>(__VA_ARGS__); break;             \
-    case 256: fn<256>(__VA_ARGS__); break;             \
-    default: fn<512>(__VA_ARGS__); break;              \
-  }
-
 int simulate_measurements(const float* gt, long long gt_bstride, const uint8_t* mask, long long mask_bstride,
                           const float* sigma, int sigma_stride, const unsigned long long* seeds, float2* y0, float2* x0,
                           float2* aty0, int B, int H, int W, cudaStream_t st) {
   if (!any_shape_supported(H, W)) return -2;
-  SimParams p{H, W, gt, gt_bstride, mask, mask_bstride, sigma, sigma_stride, seeds, y0, x0, aty0, 0.f, 0};
+  const SimSampleOp smp{{}, mask, mask_bstride, sigma, sigma_stride, seeds, y0, W};
   if (!fft_shape_supported(H, W)) {
-    int rc = sim_launch_any<0>(p, B, st);
-    if (rc == 0) rc = sim_launch_any<1>(p, B, st);
-    if (rc == 0) rc = sim_launch_any<2>(p, B, st);
+    int rc = dense_lines(SimAnyRowsFwd{{}, gt, gt_bstride, x0}, H, W, B, st);
+    if (rc == 0) rc = dense_lines(SimAnyCols{smp, x0}, H, W, B, st);
+    if (rc == 0) rc = dense_lines(SimAnyRowsInv{{}, x0, aty0}, H, W, B, st);
     return rc;
   }
-  p.kscale = ((((H + W) / 2) & 1) ? -1.f : 1.f) / sqrtf(float(H) * float(W));
-  p.gt_vec4 = (reinterpret_cast<uintptr_t>(gt) % 16 == 0) && (gt_bstride % 4 == 0);
-  SIM_DISPATCH_N(W, sim_launch_rows_fwd, p, B, st);
-  SIM_DISPATCH_N(H, sim_launch_cols, p, B, st);
-  SIM_DISPATCH_N(W, sim_launch_rows_inv, p, B, st);
-  return int(cudaGetLastError());
+  const float kscale = centre_sign(H, W) / sqrtf(float(H) * float(W));
+  const int gt_vec4 = (reinterpret_cast<uintptr_t>(gt) % 16 == 0) && (gt_bstride % 4 == 0);
+  int rc = radix_rows(SimRowsFwd{{}, gt, gt_bstride, x0, gt_vec4}, H, W, B, st);
+  if (rc == 0) rc = radix_cols(SimCols{smp, x0, kscale}, H, W, B, st);
+  if (rc == 0) rc = radix_rows(SimRowsInv{{}, x0, aty0, kscale}, H, W, B, st);
+  return rc;
 }
 
 int cartesian_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_cols, uint8_t* mask,
@@ -503,7 +363,5 @@ int radial_masks(const double* frac, int frac_stride, const unsigned long long* 
   radial_mask_kernel<<<B, kRadialThreads, radial_smem_bytes(H, W), st>>>(frac, frac_stride, seeds, mask, lines_out, H, W);
   return int(cudaGetLastError());
 }
-
-#undef SIM_DISPATCH_N
 
 }  // namespace pnp

@@ -99,6 +99,29 @@ def test_fft2c_any_size_more_images_than_one_grid_dimension():
     assert (got[-1] - ref[-1]).abs().max().item() < 1e-5 and (got[65535] - ref[65535]).abs().max().item() < 1e-5
 
 
+def test_radix_passes_more_images_than_one_grid_dimension():
+    """More images than gridDim.y holds (65535) at a radix size: the radix line passes walk the batch in slices too, and an
+    image's result does not depend on the slice it lands in."""
+    B, H, W = 65537, 32, 32
+    g = torch.Generator(device=DEV).manual_seed(13)
+    cz = lambda: torch.complex(torch.randn(B, 1, H, W, device=DEV, generator=g),
+                               torch.randn(B, 1, H, W, device=DEV, generator=g))
+    z = cz()
+    got = ops.fft2c(z)
+    for b in (0, 65536):
+        assert torch.equal(got[b], ops.fft2c(z[b:b + 1])[0])
+    del got
+    x = torch.rand(B, 1, H, W, device=DEV, generator=g)
+    u, y0 = z, cz()
+    mask = torch.rand(B, 1, H, W, device=DEV, generator=g) < 0.3
+    mu = torch.tensor([0.4], device=DEV)
+    zz, uu, vv = ops.prox_dual(x, u, y0, mask, mu)
+    for b in (0, 65536):
+        s = slice(b, b + 1)
+        z1, u1, v1 = ops.prox_dual(x[s], u[s], y0[s], mask[s], mu)
+        assert torch.equal(zz[s], z1) and torch.equal(uu[s], u1) and torch.equal(vv[s], v1)
+
+
 def test_fft2c_rejects_sizes_outside_2_1024():
     from dt4image_restoration_b200._lib import PnpError
     for (h, w) in ((1025, 16), (16, 2048), (1, 64)):

@@ -113,7 +113,8 @@ def passes(B, H, W, iters=50):
             ops.simulate_measurements(gt, mask, 10.0, 0, out=out)
         torch.cuda.synchronize()
     px = B * H * W
-    pass_bytes = {"sim_rows_fwd": 12, "sim_cols": 25, "sim_rows_inv": 24}   # B/pixel each pass moves (ATy0 written)
+    # B/pixel each pass moves (ATy0 written); the op type names the pass: radix_rows_kernel<N, SimRowsFwd> etc.
+    pass_bytes = {"SimRowsFwd": 12, "SimCols": 25, "SimRowsInv": 24}
     for ev in prof.key_averages():
         for k, nb in pass_bytes.items():
             if k in ev.key:
