@@ -35,6 +35,8 @@ SIGNATURES = {
                                           c_void_p, c_int, c_int, c_int, c_void_p]),
     "pnp_cartesian_masks": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p]),
     "pnp_radial_masks": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
+    "pnp_variable_density_masks": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int,
+                                           c_void_p]),
     "pnp_residual_real": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_void_p]),
     "pnp_prox_workspace_bytes": (c_size_t, [c_int, c_int, c_int]),
     "pnp_prox_dual": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_void_p, c_int, c_void_p, c_void_p,

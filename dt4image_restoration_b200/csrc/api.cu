@@ -122,7 +122,7 @@ int pnp_fft2c(const void* src, void* dst, int B, int H, int W, int inverse, void
                                  cudaStream_t(stream)), "pnp_fft2c");
 }
 
-// Byte ranges [lo, hi) of the buffers of pnp_simulate_measurements / pnp_radial_masks, for the overlap test.
+// Byte ranges [lo, hi) of the buffers of pnp_simulate_measurements and the mask calls, for the overlap test.
 static bool ranges_overlap(const void* a, size_t na, const void* b, size_t nb) {
   const uintptr_t pa = reinterpret_cast<uintptr_t>(a), pb = reinterpret_cast<uintptr_t>(b);
   return a && b && pa < pb + nb && pb < pa + na;
@@ -185,6 +185,26 @@ int pnp_radial_masks(const double* frac, int frac_stride, const unsigned long lo
   REQUIRE_INIT();
   return fail_cuda(radial_masks(frac, frac_stride, seeds, mask_out, lines_out, B, H, W, cudaStream_t(stream)),
                    "pnp_radial_masks");
+}
+
+int pnp_variable_density_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_h, int acs_w,
+                               int power, uint8_t* mask_out, int B, int H, int W, void* stream) {
+  if (!accel || !seeds || !mask_out) { set_error("pnp_variable_density_masks: null pointer"); return -1; }
+  if (B <= 0 || accel_stride < 0) { set_error("pnp_variable_density_masks: need B > 0 and accel_stride >= 0"); return -1; }
+  if (!fft_any_shape_supported(H, W)) { set_error("pnp_variable_density_masks: H and W must be in [2, 1024]"); return -2; }
+  if (acs_h < 0 || acs_h > H || acs_w < 0 || acs_w > W || power < 0 || power > 16) {
+    set_error("pnp_variable_density_masks: need 0 <= acs_h <= H, 0 <= acs_w <= W and 0 <= power <= 16");
+    return -1;
+  }
+  const size_t nmask = size_t(B) * H * W, nseeds = size_t(B) * sizeof(unsigned long long);
+  const size_t naccel = (size_t(B - 1) * accel_stride + 1) * sizeof(int);
+  if (ranges_overlap(mask_out, nmask, accel, naccel) || ranges_overlap(mask_out, nmask, seeds, nseeds)) {
+    set_error("pnp_variable_density_masks: mask_out overlaps accel or seeds");
+    return -1;
+  }
+  REQUIRE_INIT();
+  return fail_cuda(variable_density_masks(accel, accel_stride, seeds, acs_h, acs_w, power, mask_out, B, H, W,
+                                          cudaStream_t(stream)), "pnp_variable_density_masks");
 }
 
 int pnp_residual_real(const void* z, const void* u, float* v, long long n, void* stream) {

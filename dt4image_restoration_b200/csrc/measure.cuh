@@ -1,6 +1,6 @@
-// Measurement simulator: undersampled, noisy k-space measurements of fully-sampled images, and seeded Cartesian and radial
-// masks (pnp_simulate_measurements / pnp_cartesian_masks / pnp_radial_masks; the definitions are in include/pnp_b200.h).
-// Per image b:
+// Measurement simulator: undersampled, noisy k-space measurements of fully-sampled images, and seeded Cartesian, radial and
+// variable-density masks (pnp_simulate_measurements / pnp_cartesian_masks / pnp_radial_masks / pnp_variable_density_masks;
+// the definitions are in include/pnp_b200.h).  Per image b:
 //
 //     y0   = mask ? fft_c(gt) + sigma_n / 255 * (n_r + i n_i) : 0      (n_r, n_i: Philox4x32-10 + Box-Muller at (i, j))
 //     ATy0 = ifft_c(y0),   x0 = (max(Re ATy0, 0), max(Im ATy0, 0))
@@ -323,6 +323,227 @@ __global__ void __launch_bounds__(kRadialThreads) radial_mask_kernel(const doubl
   for (size_t e = head + 16 * nvec + tid; e < npx; e += kRadialThreads) img[e] = (radial_bits[e >> 5] >> (e & 31)) & 1u;
 }
 
+// ---------------------------------------------------------------- variable-density random masks: one cluster per image
+// Image b's mask is the ACS block plus the `extra` non-ACS pixels with the smallest 51-bit words (float_bits(key) << 20 | p):
+// keys are positive floats, which order like their bits, and p < 2^20, so the integer order is the (key, p) order and the
+// extra-th smallest word is a unique threshold.  It is found by radix selection over the cluster, 11 bits at a time
+// (digits 50..40, 39..29, 28..18, 17..7, 6..0).  Each CTA owns a slice of `slice` consecutive pixels (a multiple of 32) and
+// keeps its part of the mask as a bitmap in shared memory.  A pass counts the digit of the words whose higher bits equal the
+// prefix P chosen so far into a shared histogram; one cluster barrier later every CTA sums the cluster's histograms
+// through DSMEM (double-buffered by pass parity, so one barrier per pass) and picks the same bin and remaining rank.  The
+// selection stops as soon as the chosen bin holds exactly the remaining rank; then a word is sampled iff (word >> L) <= P.
+// A pass either recomputes the keys of the whole slice (and sets the bitmap bits of the words already below the prefix) or,
+// once they fit, reads the slice's words of the current bin from a candidate list in shared memory: the recompute pass
+// after which a CTA's share of the chosen bin is at most `cap` also writes that list.  Small slices fit from the first
+// pass; large ones take two key computations per pixel and then passes over the list (an 11-bit bin of positive floats
+// holds at most 1/8 of the slice in expectation, so cap >= slice / 8 is almost always enough; if not, a CTA recomputes
+// once more, with the same code).  The key path uses only __dadd_rn / __dsub_rn / __dmul_rn / __ddiv_rn / __dsqrt_rn /
+// __double2float_rn, so it is bit for bit the definition's, and integer counts make every mask independent of the cluster
+// size and the batch position.
+constexpr int kVdThreads = 512;
+constexpr int kVdWarps = kVdThreads / 32;
+constexpr int kVdDigit = 11;
+constexpr int kVdBins = 1 << kVdDigit;                   // 4 per thread in the scan
+constexpr int kVdMaxSlice = 131072;                      // pixels per CTA at most: 1024^2 on an 8-CTA cluster
+__host__ __device__ constexpr size_t vd_bitmap_offset(int H, int W) {
+  return 2 * kVdBins * sizeof(unsigned) + size_t(H + W) * sizeof(double);
+}
+__host__ __device__ constexpr size_t vd_cand_offset(int H, int W, int slice) {
+  return (vd_bitmap_offset(H, W) + (size_t(slice) / 32 + 1) * sizeof(unsigned) + 7) / 8 * 8;
+}
+__host__ __device__ constexpr size_t vd_smem_bytes(int H, int W, int slice, int cap) {
+  return vd_cand_offset(H, W, slice) + size_t(cap) * sizeof(unsigned long long);
+}
+
+__device__ __forceinline__ uint4 ld_dsmem_v4(const void* local, unsigned rank) {
+  uint32_t a;
+  uint4 v;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(smem_u32(local)), "r"(rank));
+  asm volatile("ld.shared::cluster.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(a)
+               : "memory");
+  return v;
+}
+
+// key = float32(u / w) at pixel p = i*W + j, with ky2 = ky*ky and kx2 = kx*kx of its row and column (definition in
+// include/pnp_b200.h): every operation rounded on its own, no FMA.
+__device__ __forceinline__ float vd_key(double ky2, double kx2, int power, unsigned p, uint2 seed_k) {
+  const double r = __dsqrt_rn(__dmul_rn(0.5, __dadd_rn(ky2, kx2)));
+  const double q = __dsub_rn(1.0, r);
+  double w = 1.0;
+  for (int k = 0; k < power; ++k) w = __dmul_rn(w, q);
+  const unsigned w0 = philox4x32_10(make_uint4(p, 3u, 0u, 0u), seed_k).x;
+  const double u = __dmul_rn(__dadd_rn(double(w0), 0.5), 0x1p-32);
+  return __double2float_rn(__ddiv_rn(u, w));                // w = 0: +inf
+}
+
+__global__ void __launch_bounds__(kVdThreads) vd_mask_kernel(const int* accel, int accel_stride,
+                                                             const unsigned long long* seeds, int acs_h, int acs_w,
+                                                             int power, uint8_t* out, int H, int W, int slice, int cap) {
+  extern __shared__ __align__(16) unsigned char vd_smem[];
+  unsigned* hist = reinterpret_cast<unsigned*>(vd_smem);                      // [2][kVdBins], by pass parity
+  double* sq = reinterpret_cast<double*>(vd_smem + 2 * kVdBins * sizeof(unsigned));   // ky^2 of the rows, kx^2 of the columns
+  unsigned* bm = reinterpret_cast<unsigned*>(vd_smem + vd_bitmap_offset(H, W));      // the slice's mask, bit e = pixel s0 + e
+  unsigned long long* cand = reinterpret_cast<unsigned long long*>(vd_smem + vd_cand_offset(H, W, slice));
+  __shared__ unsigned warp_total[kVdWarps];
+  __shared__ unsigned chosen[4];                           // bin, rank left in it, its population: cluster, this CTA
+  __shared__ unsigned n_cand;
+  unsigned cs, crank;
+  asm volatile("mov.u32 %0, %%cluster_nctarank;" : "=r"(cs));
+  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(crank));
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int b = blockIdx.x / int(cs);
+  const int HW = H * W;
+  const int s0 = min(HW, int(crank) * slice), s1 = min(HW, s0 + slice);
+  const int nq = (s1 - s0 + 31) >> 5;                      // 32-pixel groups of the slice: bitmap words
+  const int cy = H / 2, cx = W / 2, r0 = cy - acs_h / 2, c0 = cx - acs_w / 2;
+  const int a = accel[size_t(b) * accel_stride];
+  const int n_keep = a >= 1 ? max(1, HW / a) : HW;
+  const int n_acs = acs_h * acs_w;
+  const int extra = max(0, n_keep - n_acs);
+  const uint2 seed_k = seed_key(seeds[b]);
+  for (int t = tid; t < H + W; t += kVdThreads) {
+    const int c = t < H ? cy : cx;
+    const double k = __ddiv_rn(double((t < H ? t : t - H) - c), double(c));
+    sq[t] = __dmul_rn(k, k);
+  }
+  if (tid == 0) n_cand = 0u;
+  __syncthreads();
+
+  // bits of group q (32 consecutive pixels of the slice, one group per thread): the ACS pixels, and each other pixel for
+  // which take(word) holds (take is not called when keys = false)
+  auto group = [&](int q, bool keys, auto&& take) -> unsigned {
+    int p = s0 + (q << 5);
+    int i = p / W, j = p - i * W;
+    const int n = min(32, s1 - p);
+    unsigned bits = 0u;
+    for (int e = 0; e < n; ++e, ++p) {
+      if (unsigned(i - r0) < unsigned(acs_h) && unsigned(j - c0) < unsigned(acs_w)) {
+        bits |= 1u << e;
+      } else if (keys) {
+        const float key = vd_key(sq[i], sq[H + j], power, unsigned(p), seed_k);
+        if (take((static_cast<unsigned long long>(__float_as_uint(key)) << 20) | unsigned(p))) bits |= 1u << e;
+      }
+      if (++j == W) { j = 0; ++i; }
+    }
+    return bits;
+  };
+  auto mark = [&](unsigned long long w) {                 // a listed word is sampled
+    const unsigned e = unsigned(w & 0xFFFFFu) - unsigned(s0);
+    atomicOr(&bm[e >> 5], 1u << (e & 31));
+  };
+
+  const bool all = extra == HW - n_acs;                    // every pixel is sampled (accel <= 1)
+  const bool select = extra != 0 && !all;                  // the same in every CTA of the cluster
+  if (!select) {                                           // no key, no DSMEM access
+    for (int q = tid; q < nq; q += kVdThreads) {
+      const unsigned bits = group(q, false, [](unsigned long long) { return false; });
+      const int n = min(32, s1 - s0 - (q << 5));
+      bm[q] = all ? (n == 32 ? ~0u : (1u << n) - 1u) : bits;
+    }
+  } else {
+    int L = 51;                                            // the words in play have (w >> L) == P
+    unsigned long long P = 0ull;
+    unsigned k = unsigned(extra);                          // rank of the threshold among them
+    bool listed = false;                                   // cand[] holds this CTA's words in play
+    bool collect = s1 - s0 <= cap;                         // this pass writes cand[]
+    for (int pass = 0;; ++pass) {
+      unsigned* h = hist + (pass & 1) * kVdBins;           // peers last read this buffer before the previous barrier
+      for (int d = tid; d < kVdBins; d += kVdThreads) h[d] = 0u;
+      __syncthreads();
+      const int Ln = max(L - kVdDigit, 0);
+      const unsigned dmask = (1u << (L - Ln)) - 1u;
+      if (listed) {
+        for (unsigned c = tid; c < n_cand; c += kVdThreads) {
+          const unsigned long long w = cand[c], t = w >> L;
+          if (t < P) mark(w);
+          else if (t == P) atomicAdd(&h[unsigned(w >> Ln) & dmask], 1u);
+        }
+      } else {
+        for (int q = tid; q < nq; q += kVdThreads) {
+          bm[q] = group(q, true, [&](unsigned long long w) {
+            const unsigned long long t = w >> L;
+            if (t == P) {
+              atomicAdd(&h[unsigned(w >> Ln) & dmask], 1u);
+              if (collect) {                               // warp-aggregated append
+                const unsigned act = __activemask();
+                const int leader = __ffs(act) - 1;
+                unsigned base = 0u;
+                if (lane == leader) base = atomicAdd(&n_cand, unsigned(__popc(act)));
+                base = __shfl_sync(act, base, leader);
+                cand[base + __popc(act & ((1u << lane) - 1u))] = w;
+              }
+            }
+            return t < P;
+          });
+        }
+      }
+      asm volatile("barrier.cluster.arrive.release;\n\tbarrier.cluster.wait.acquire;" ::: "memory");
+      // bins 4 tid .. 4 tid + 3 summed over the cluster; a block scan finds the bin that holds rank k
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      for (unsigned r = 0; r < cs; ++r) {
+        const uint4 x = ld_dsmem_v4(h + 4 * tid, r);
+        v = make_uint4(v.x + x.x, v.y + x.y, v.z + x.z, v.w + x.w);
+      }
+      const unsigned s = v.x + v.y + v.z + v.w;
+      unsigned incl = s;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const unsigned y = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+        if (lane >= o) incl += y;
+      }
+      if (lane == 31) warp_total[warp] = incl;
+      __syncthreads();
+      unsigned before = incl - s;
+      for (int w2 = 0; w2 < warp; ++w2) before += warp_total[w2];
+      if (before < k && k <= before + s) {
+        const unsigned c4[4] = {v.x, v.y, v.z, v.w};
+        for (int m = 0; m < 4; ++m) {
+          if (k <= before + c4[m]) {
+            chosen[0] = unsigned(4 * tid + m);
+            chosen[1] = k - before;
+            chosen[2] = c4[m];
+            chosen[3] = h[4 * tid + m];
+            break;
+          }
+          before += c4[m];
+        }
+      }
+      __syncthreads();
+      P = (P << (L - Ln)) | chosen[0];
+      L = Ln;
+      k = chosen[1];
+      listed |= collect;
+      collect = !listed && chosen[3] <= unsigned(cap);
+      if (chosen[2] == k || L == 0) break;                 // the whole bin is sampled (at L = 0 it holds one word)
+    }
+    asm volatile("barrier.cluster.arrive.release;" ::: "memory");    // the last DSMEM reads are done
+    if (listed) {
+      for (unsigned c = tid; c < n_cand; c += kVdThreads)
+        if ((cand[c] >> L) <= P) mark(cand[c]);
+    } else {
+      for (int q = tid; q < nq; q += kVdThreads)
+        bm[q] = group(q, true, [&](unsigned long long w) { return (w >> L) <= P; });
+    }
+  }
+  __syncthreads();
+  // the slice as one flat run of bytes: 16-byte stores between an unaligned head and tail (bits from two bitmap words)
+  const int n = s1 - s0;
+  uint8_t* img = out + size_t(b) * HW + s0;
+  const int head = min(int((16 - (reinterpret_cast<uintptr_t>(img) & 15)) & 15), n);
+  const int nvec = (n - head) / 16;
+  for (int e = tid; e < head; e += kVdThreads) img[e] = (bm[e >> 5] >> (e & 31)) & 1u;
+  for (int q = tid; q < nvec; q += kVdThreads) {
+    const int p0 = head + 16 * q;
+    const unsigned bits = __funnelshift_r(bm[p0 >> 5], bm[(p0 >> 5) + 1], unsigned(p0 & 31));
+    unsigned v[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) v[k] = (((bits >> (4 * k)) & 0xFu) * 0x00204081u) & 0x01010101u;   // 4 bits -> 4 bytes
+    reinterpret_cast<uint4*>(img + p0)[0] = make_uint4(v[0], v[1], v[2], v[3]);
+  }
+  for (int e = head + 16 * nvec + tid; e < n; e += kVdThreads) img[e] = (bm[e >> 5] >> (e & 31)) & 1u;
+  if (select) asm volatile("barrier.cluster.wait.acquire;" ::: "memory");   // no peer reads this CTA's histograms any more
+}
+
 // ---------------------------------------------------------------- host side
 int simulate_measurements(const float* gt, long long gt_bstride, const uint8_t* mask, long long mask_bstride,
                           const float* sigma, int sigma_stride, const unsigned long long* seeds, float2* y0, float2* x0,
@@ -362,6 +583,41 @@ int radial_masks(const double* frac, int frac_stride, const unsigned long long* 
   }
   radial_mask_kernel<<<B, kRadialThreads, radial_smem_bytes(H, W), st>>>(frac, frac_stride, seeds, mask, lines_out, H, W);
   return int(cudaGetLastError());
+}
+
+// Cluster size: enough CTAs that a slice is at most kVdMaxSlice pixels (8 at 1024^2), then more (up to 16, a non-portable
+// size) while the batch leaves SMs idle and slices keep >= 4096 pixels; the masks do not depend on it.  The candidate list
+// holds max(slice / 8, slice up to 4096) words.
+int variable_density_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_h, int acs_w,
+                           int power, uint8_t* mask, int B, int H, int W, cudaStream_t st) {
+  if (!any_shape_supported(H, W)) return -2;
+  static bool attr_done = false;
+  if (!attr_done) {
+    cudaError_t e = cudaFuncSetAttribute(vd_mask_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         int(vd_smem_bytes(kAnyMaxN, kAnyMaxN, kVdMaxSlice, kVdMaxSlice / 8)));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(vd_mask_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    if (e != cudaSuccess) return int(e);
+    attr_done = true;
+  }
+  const int hw = H * W;
+  int cs = 1;
+  while (cs < 16 && ((hw + cs - 1) / cs > kVdMaxSlice || ((long long)B * cs < num_sms() && hw / (2 * cs) >= 4096))) cs *= 2;
+  const int slice = ((hw + cs - 1) / cs + 31) / 32 * 32;
+  const int cap = max(slice / 8, min(slice, 4096));
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(unsigned(B) * unsigned(cs));
+  cfg.blockDim = dim3(kVdThreads);
+  cfg.dynamicSmemBytes = vd_smem_bytes(H, W, slice, cap);
+  cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = unsigned(cs);
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  return int(cudaLaunchKernelEx(&cfg, vd_mask_kernel, accel, accel_stride, seeds, acs_h, acs_w, power, mask, H, W, slice,
+                                cap));
 }
 
 }  // namespace pnp

@@ -45,6 +45,8 @@ int cartesian_masks(const int* accel, int accel_stride, const unsigned long long
                     int B, int H, int W, cudaStream_t st);
 int radial_masks(const double* frac, int frac_stride, const unsigned long long* seeds, uint8_t* mask, int* lines_out,
                  int B, int H, int W, cudaStream_t st);
+int variable_density_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_h, int acs_w,
+                           int power, uint8_t* mask, int B, int H, int W, cudaStream_t st);
 
 // policy.cu
 size_t policy_packed_floats(int n_time, int n_task);

@@ -85,21 +85,24 @@ class PnPEngine:
         self.prepare()
         self.iters = 0
 
-    def reset_from_gt(self, gt, sigma_n, seeds, mask=None, accel=None, radial=None):
+    def reset_from_gt(self, gt, sigma_n, seeds, mask=None, accel=None, radial=None, vd=None):
         """Start B new trajectories from fully-sampled images, simulating the measurements straight into the engine's
         buffers (``ops.simulate_measurements``; no host<->device copy of image data): ``y0``, ``z`` = x0, ``x`` = ``v`` =
-        Re x0, ``u`` = 0, ``mask``, ``gt``.  Same state as ``reset(ops.make_items(gt, sigma_n, seeds, mask, accel, radial))``.
-        ``gt`` fp32 CUDA ``[B,1,H,W]`` / ``[B,H,W]`` / ``[H,W]``; pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H,
-        W]``, CUDA), ``accel`` (Cartesian masks drawn with ``seeds``) and ``radial`` (radial masks with this sampled fraction,
-        rotated by ``seeds``)."""
-        if sum(m is not None for m in (mask, accel, radial)) != 1:
-            raise ValueError("pass exactly one of mask / accel / radial")
+        Re x0, ``u`` = 0, ``mask``, ``gt``.  Same state as
+        ``reset(ops.make_items(gt, sigma_n, seeds, mask, accel, radial, vd))``.  ``gt`` fp32 CUDA ``[B,1,H,W]`` / ``[B,H,W]``
+        / ``[H,W]``; pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``, CUDA), ``accel`` (Cartesian masks
+        drawn with ``seeds``), ``radial`` (radial masks with this sampled fraction, rotated by ``seeds``) and ``vd`` (the
+        acceleration of variable-density masks drawn with ``seeds``)."""
+        if sum(m is not None for m in (mask, accel, radial, vd)) != 1:
+            raise ValueError("pass exactly one of mask / accel / radial / vd")
         B, H, W = self.B, self.H, self.W
         seeds = ops._seed_tensor(seeds, B, self.device)
         if accel is not None:
             ops.cartesian_masks(B, H, W, accel, seeds, out=self.mask)
         elif radial is not None:
             ops.radial_masks(B, H, W, radial, seeds, out=self.mask)
+        elif vd is not None:
+            ops.variable_density_masks(B, H, W, vd, seeds, out=self.mask)
         else:
             m = ops._mask_u8(mask).reshape(-1, 1, H, W)
             self.mask.copy_(m.ne(0).expand(B, 1, H, W))

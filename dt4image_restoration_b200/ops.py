@@ -200,13 +200,36 @@ def radial_masks(B: int, H: int, W: int, frac, seeds=None, out=None, lines_out=N
     return out
 
 
-def make_items(gt, sigma_n, seeds, mask=None, accel=None, radial=None) -> dict:
+def variable_density_masks(B: int, H: int, W: int, accel, seeds, power: int = 3, acs_frac: float = 0.08,
+                           out=None) -> torch.Tensor:
+    """Seeded 2-D variable-density random masks (``pnp_variable_density_masks``): uint8 ``[B,H,W]`` on the current CUDA
+    device.  A centred ACS block of ``max(1, round(acs_frac H))`` x ``max(1, round(acs_frac W))`` pixels plus the other
+    pixels with the smallest Philox key / ``(1 - r)^power`` (r the normalised k-space radius), up to exactly
+    ``max(1, H*W // accel)`` sampled pixels.  ``accel`` an int or int32 ``[B]`` CUDA tensor; ``seeds`` as in
+    ``simulate_measurements``; ``power`` in 0..16 (0: uniform)."""
+    dev = torch.device("cuda", torch.cuda.current_device())
+    if not torch.is_tensor(accel) and int(accel) < 1:
+        raise ValueError(f"accel must be >= 1, got {accel}")
+    acc, astride = _per_image(accel if torch.is_tensor(accel) else int(accel), B, torch.int32, "accel", dev)
+    seeds = _seed_tensor(seeds, B, dev)
+    acs_h, acs_w = max(1, int(round(acs_frac * H))), max(1, int(round(acs_frac * W)))
+    if out is None:
+        out = torch.empty(B, H, W, dtype=torch.uint8, device=dev)
+    elif not out.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous() or out.numel() != B * H * W:
+        raise _lib.PnpError(f"out must be a contiguous uint8 CUDA tensor with {B * H * W} elements")
+    check(_lib.lib().pnp_variable_density_masks(acc.data_ptr(), astride, seeds.data_ptr(), acs_h, acs_w, int(power),
+                                                out.data_ptr(), B, H, W, _lib.stream_ptr()), "pnp_variable_density_masks")
+    return out
+
+
+def make_items(gt, sigma_n, seeds, mask=None, accel=None, radial=None, vd=None) -> dict:
     """A batch of episode items on the device with ``synth.make_batch``'s keys, shapes and dtypes (``x0, y0, ATy0`` fp32
     ``[B,1,H,W,2]``, ``mask`` uint8 ``[B,H,W]``, ``gt`` fp32 ``[B,1,H,W]``), ready for ``PnPEnv.reset`` / ``PnPEngine.reset``.
-    Pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``), ``accel`` (Cartesian masks drawn with ``seeds``) and
-    ``radial`` (the sampled fraction of radial masks rotated by ``seeds``, see ``radial_masks``)."""
-    if sum(m is not None for m in (mask, accel, radial)) != 1:
-        raise ValueError("pass exactly one of mask / accel / radial")
+    Pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``), ``accel`` (Cartesian masks drawn with ``seeds``),
+    ``radial`` (the sampled fraction of radial masks rotated by ``seeds``, see ``radial_masks``) and ``vd`` (the
+    acceleration of variable-density masks drawn with ``seeds``, default power and ACS of ``variable_density_masks``)."""
+    if sum(m is not None for m in (mask, accel, radial, vd)) != 1:
+        raise ValueError("pass exactly one of mask / accel / radial / vd")
     gt = _req(gt, torch.float32, "gt")
     H, W = gt.shape[-2:]
     B = _batch_size(gt, mask, sigma_n, seeds)
@@ -214,6 +237,8 @@ def make_items(gt, sigma_n, seeds, mask=None, accel=None, radial=None) -> dict:
         mask = cartesian_masks(B, H, W, accel, seeds)
     elif radial is not None:
         mask = radial_masks(B, H, W, radial, seeds)
+    elif vd is not None:
+        mask = variable_density_masks(B, H, W, vd, seeds)
     else:
         mask = _mask_u8(mask).ne(0).to(torch.uint8).reshape(-1, H, W).expand(B, H, W).contiguous()
     y0, x0, aty0 = simulate_measurements(gt, mask, sigma_n, seeds)

@@ -122,6 +122,31 @@ int pnp_cartesian_masks(const int* accel, int accel_stride, const unsigned long 
 int pnp_radial_masks(const double* frac, int frac_stride, const unsigned long long* seeds, uint8_t* mask_out,
                      int* lines_out, int B, int H, int W, void* stream);
 
+/* Seeded 2-D variable-density random masks (Lustig, Donoho and Pauly, 2007): dense near the k-space centre, sparser
+ * towards the edge, with exactly max(n_keep, |ACS|) sampled pixels.  Per image b, for every index (i, j) in the centred
+ * k-space layout, in float64 with every operation rounded on its own (no FMA):
+ *   cy = H / 2,  cx = W / 2                                   (integer division; H, W >= 2 so both >= 1)
+ *   ky = (i - cy) / cy,   kx = (j - cx) / cx                  (both in [-1, 1])
+ *   r  = sqrt(0.5 * (ky*ky + kx*kx))                          (in [0, 1]; r = 1 only where |ky| = |kx| = 1)
+ *   w  = 1; repeat `power` times: w = w * (1 - r)             (power 0: w = 1, uniform sampling)
+ *   p  = i*W + j
+ *   u  = (philox4x32_10(counter = (p, 3, 0, 0), key = (lo32(seed[b]), hi32(seed[b]))).w0 + 0.5) * 2^-32
+ *   key[p] = float32(u / w)                                   (round to nearest; w = 0 or overflow gives +inf)
+ *   n_keep = accel[b] >= 1 ? max(1, (H*W) / accel[b]) : H*W  (integer division; same rule as pnp_cartesian_masks)
+ *   ACS    = rows [cy - acs_h/2, cy - acs_h/2 + acs_h) x columns [cx - acs_w/2, cx - acs_w/2 + acs_w)
+ *   mask[b] = 1 on ACS, plus on the max(0, n_keep - |ACS|) pixels outside ACS with the smallest (key[p], p),
+ *             compared lexicographically; 0 elsewhere
+ * Selecting the smallest u/w is Bernoulli sampling of pixel p when u_p <= t w_p, with the threshold t that makes the count
+ * exact: the density (1 - r)^power, scaled to the sample budget.  Counter word 1 = 3 keeps this stream apart from the
+ * noise (0), the Cartesian column keys (1) and the radial rotation (2).  The key uses only + - * /, sqrt and the double ->
+ * float rounding, so a NumPy restatement reproduces the masks bit for bit.  accel: device int32, accel[b*accel_stride]
+ * (0 stride = one value for the batch); seeds: device uint64 [B]; mask_out: uint8 [B,H,W], must not overlap accel or
+ * seeds.  H, W in 2..1024, 0 <= acs_h <= H, 0 <= acs_w <= W, 0 <= power <= 16.  Results are bitwise reproducible and
+ * independent of the batch position.  These masks are general (not column-only, unless every pixel is sampled), so
+ * pnp_prox_prepare routes them to the cluster prox kernel. */
+int pnp_variable_density_masks(const int* accel, int accel_stride, const unsigned long long* seeds, int acs_h, int acs_w,
+                               int power, uint8_t* mask_out, int B, int H, int W, void* stream);
+
 /* v = Re(z - u): the denoiser input of PnPEnv.step (env.py:85-86). */
 int pnp_residual_real(const void* z_c64, const void* u_c64, float* v, long long n, void* stream);
 
