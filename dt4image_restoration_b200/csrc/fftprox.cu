@@ -146,19 +146,42 @@ struct PrepareYt : LineOp {
   }
 };
 
-static int launch_cl(const ClParams& p, cudaStream_t st) { return launch_cl_t<16>(p, st); }
+// The three radix passes of the general path.  skip_flag: optional device flag, != 0 -> the row-only kernel handles this
+// batch; active as in ClParams.
+static int prox_radix3(const float* x, const float2* u_in, const float2* y0, const uint8_t* mask, long long mask_bstride,
+                       const float* mu, int mu_stride, float2* z_out, float2* u_out, float* v_out, float2* work, int B, int H,
+                       int W, const int* skip_flag, const uint8_t* active, cudaStream_t st) {
+  const float inv = 1.0f / sqrtf(float(H) * float(W));
+  int rc = radix_rows(ProxRowsIn{{}, x, u_in, work, skip_flag}, H, W, B, st);
+  if (rc == 0)
+    rc = radix_cols(ProxColsBlend{{{}, y0, mask, mask_bstride, mu, mu_stride}, work, inv, centre_sign(H, W), skip_flag},
+                    H, W, B, st);
+  if (rc == 0)
+    rc = radix_rows(ProxRowsOut{{{}, x, u_in, z_out, u_out, v_out, active}, work, inv, skip_flag}, H, W, B, st);
+  return rc;
+}
 
-static int prox_prepare_cl(const float2* y0, const uint8_t* mask, long long mask_bstride, float2* y0R, uint16_t* mpack,
-                           int B, cudaStream_t st, const int* skip_flag = nullptr) {
-  prox_prepare_cl_kernel<<<dim3(kClN, B), 256, 0, st>>>(y0, mask, mask_bstride, y0R, mpack, mask_bstride ? B : 1, skip_flag);
+// Shapes with a single-launch cluster kernel: 256x256 (fftprox_cl.cuh) and 128x128 (fftprox_cl128.cuh).
+static bool cluster_shape(int H, int W) { return H == W && (H == kClN || H == kC128N); }
+
+// The cluster kernel's trajectory constants y0R and packed rotated mask (fftprox_cl.cuh "Algebra") at a cluster shape.
+static int prepare_cluster(const float2* y0, const uint8_t* mask, long long mask_bstride, float2* y0R, uint16_t* mpack,
+                           int B, int H, const int* skip_flag, cudaStream_t st) {
+  const int nb = mask_bstride ? B : 1;
+  if (H == kClN)
+    prox_prepare_cl_kernel<<<dim3(kClN, B), 256, 0, st>>>(y0, mask, mask_bstride, y0R, mpack, nb, skip_flag);
+  else
+    prox_prepare_cl128_kernel<<<dim3(kC128N, B), kC128N, 0, st>>>(y0, mask, mask_bstride, y0R, mpack, nb, skip_flag);
   return int(cudaGetLastError());
 }
 
-static int prox_prepare_cl128(const float2* y0, const uint8_t* mask, long long mask_bstride, float2* y0R, uint16_t* mpack,
-                              int B, cudaStream_t st, const int* skip_flag = nullptr) {
-  prox_prepare_cl128_kernel<<<dim3(kC128N, B), kC128N, 0, st>>>(y0, mask, mask_bstride, y0R, mpack, mask_bstride ? B : 1,
-                                                                 skip_flag);
-  return int(cudaGetLastError());
+// One cluster-kernel prox + dual update on the constants of prepare_cluster.
+static int launch_cluster(const float* x, const float2* u_in, const float2* y0R, const uint16_t* mpack, bool per_image_mask,
+                          const float* mu, int mu_stride, float2* z_out, float2* u_out, float* v_out, int B, int H,
+                          const int* skip_flag, const uint8_t* active, cudaStream_t st) {
+  const long long mpack_bstride = !per_image_mask ? 0 : H == kClN ? 16 * kClN : 8 * kC128N;
+  const ClParams cp{x, u_in, y0R, mpack, mpack_bstride, mu, mu_stride, z_out, u_out, v_out, B, skip_flag, active};
+  return H == kClN ? launch_cl(cp, st) : launch_cl128(cp, st);
 }
 
 static bool pow2_ok(int n) { return n == 32 || n == 64 || n == 128 || n == 256 || n == 512; }
@@ -182,11 +205,6 @@ void prox_prepared_bytes(int B, int H, int W, size_t* y0p_bytes, size_t* maskp_b
   *maskp_bytes = maskp_flag_off(B, H, W) + 16;
 }
 
-static int prox_dual_general_impl(const float* x, const float2* u_in, const float2* y0, const uint8_t* mask,
-                                  long long mask_bstride, const float* mu, int mu_stride, float2* z_out, float2* u_out,
-                                  float* v_out, float2* work, int B, int H, int W, const int* skip_flag, cudaStream_t st,
-                                  const uint8_t* active = nullptr);
-
 // Full preparation: copies for the general kernels, the column-only-mask test (device flag), the row mask and
 // Yt = Fc^-1 (s*D.y0) for the row-only kernels (fftprox_sep.cuh).  Once per trajectory.
 int prox_prepare(const float2* y0, const uint8_t* mask, long long mask_bstride, float2* y0p, uint8_t* maskp, int B, int H,
@@ -199,17 +217,14 @@ int prox_prepare(const float2* y0, const uint8_t* mask, long long mask_bstride, 
   int* flag = reinterpret_cast<int*>(maskp + maskp_flag_off(nb, H, W));
   cudaMemsetAsync(flag, 1, sizeof(int), st);                        // bytes 01 01 01 01: non-zero = "column-only so far"
   sep_check_kernel<<<dim3(nb, kSepCheckSlices), 256, 0, st>>>(mask, mask_bstride, H, W, mpack, flag);
-  // copies for the general kernels (the 256x256 transposes are skipped on the device when the masks are column-only)
-  if (is256) {
-    int rc = prox_prepare_cl(y0, mask, mask_bstride, y0p, reinterpret_cast<uint16_t*>(maskp), B, st, flag);
-    if (rc) return rc;
-  } else if (H == 128 && W == 128) {
-    // 128x128: the cluster kernel serves EVERY mask (measured faster than the generic row-only kernel even for column-only
-    // masks: 0.41-0.48 vs 0.34-0.42 of the HBM roofline, profiles/r02_config5_sweep_n1.txt), so it is always prepared
-    int rc = prox_prepare_cl128(y0, mask, mask_bstride, y0p, reinterpret_cast<uint16_t*>(maskp), B, st, nullptr);
-    if (rc) return rc;
-    return int(cudaGetLastError());
-  } else {
+  if (cluster_shape(H, W)) {
+    // the 256x256 constants are skipped on the device when the masks are column-only; 128x128: the cluster kernel serves
+    // EVERY mask (measured faster than the generic row-only kernel even for column-only masks: 0.41-0.48 vs 0.34-0.42 of
+    // the HBM roofline, profiles/r02_config5_sweep_n1.txt), so it is always prepared and needs no Yt
+    int rc = prepare_cluster(y0, mask, mask_bstride, y0p, reinterpret_cast<uint16_t*>(maskp), B, H, is256 ? flag : nullptr,
+                             st);
+    if (rc || !is256) return rc;
+  } else {                                                            // copies for the general kernels
     cudaMemcpyAsync(y0p, y0, n * sizeof(float2), cudaMemcpyDeviceToDevice, st);
     cudaMemcpyAsync(maskp, mask, size_t(nb) * H * W, cudaMemcpyDeviceToDevice, st);
   }
@@ -238,15 +253,12 @@ int prox_dual_prepared(const float* x, const float2* u_in, const float2* y0p, co
       int rc = launch_sep(sp, num_sms(), st);
       if (rc || kind == 1) return rc;
     }
-    ClParams cp{x, u_in, y0p, reinterpret_cast<const uint16_t*>(maskp), mask_bstride ? 16 * kClN : 0, mu, mu_stride,
-                z_out, u_out, v_out, B, flag, active};
-    return launch_cl(cp, st);
+    return launch_cluster(x, u_in, y0p, reinterpret_cast<const uint16_t*>(maskp), mask_bstride != 0, mu, mu_stride, z_out,
+                          u_out, v_out, B, H, flag, active, st);
   }
-  if (H == 128 && W == 128) {                             // every mask at 128x128: the 4-CTA cluster kernel (see prox_prepare)
-    ClParams cp{x, u_in, y0p, reinterpret_cast<const uint16_t*>(maskp), mask_bstride ? 8 * kC128N : 0, mu, mu_stride,
-                z_out, u_out, v_out, B, nullptr, active};
-    return launch_cl128(cp, st);
-  }
+  if (H == 128 && W == 128)                               // every mask at 128x128: the 4-CTA cluster kernel (see prox_prepare)
+    return launch_cluster(x, u_in, y0p, reinterpret_cast<const uint16_t*>(maskp), mask_bstride != 0, mu, mu_stride, z_out,
+                          u_out, v_out, B, H, nullptr, active, st);
   if (kind != 0) {
     SepGenParams gp{x, u_in, y0p + n, rowmask, mask_bstride ? 1 : 0, flag, mu, mu_stride, z_out, u_out, v_out, H, 0, active};
     with_pow2(W, [&](auto w) {
@@ -256,53 +268,25 @@ int prox_dual_prepared(const float* x, const float2* u_in, const float2* y0p, co
     if (kind == 1) return int(cudaGetLastError());
   }
   // any other mask: the general three-launch path on the copies, gated by the same flag
-  return prox_dual_general_impl(x, u_in, y0p, maskp, mask_bstride, mu, mu_stride, z_out, u_out, v_out,
-                                const_cast<float2*>(y0p) + 2 * n, B, H, W, flag, st, active);
+  return prox_radix3(x, u_in, y0p, maskp, mask_bstride, mu, mu_stride, z_out, u_out, v_out, const_cast<float2*>(y0p) + 2 * n,
+                     B, H, W, flag, active, st);
 }
 
-// General three-launch prox + dual update.  `work` is a c64 [B,H,W] scratch buffer.
+// Unprepared prox + dual update.  `work` is a c64 [B,H,W] scratch buffer; at 256x256 and 128x128 the cluster kernel's
+// constants go there first.
 int prox_dual_general(const float* x, const float2* u_in, const float2* y0, const uint8_t* mask,
                       long long mask_bstride, const float* mu, int mu_stride, float2* z_out, float2* u_out,
                       float* v_out, float2* work, int B, int H, int W, cudaStream_t st) {
-  return prox_dual_general_impl(x, u_in, y0, mask, mask_bstride, mu, mu_stride, z_out, u_out, v_out, work, B, H, W,
-                                nullptr, st);
-}
-
-static int prox_dual_general_impl(const float* x, const float2* u_in, const float2* y0, const uint8_t* mask,
-                                  long long mask_bstride, const float* mu, int mu_stride, float2* z_out, float2* u_out,
-                                  float* v_out, float2* work, int B, int H, int W, const int* skip_flag, cudaStream_t st,
-                                  const uint8_t* active) {
   if (!fft_shape_supported(H, W))
-    return (skip_flag == nullptr) ? prox_dual_any(x, u_in, y0, mask, mask_bstride, mu, mu_stride, z_out, u_out, v_out, work,
-                                                   B, H, W, st, active)
-                                  : -2;
-  if (skip_flag == nullptr) {
-    // single-launch cluster kernels (256x256, 128x128): y0R and the packed mask go to the workspace first
-    if (H == 128 && W == 128) {
-      float2* y0R = work;
-      uint16_t* mpack = reinterpret_cast<uint16_t*>(work + size_t(B) * H * W);
-      int rc = prox_prepare_cl128(y0, mask, mask_bstride, y0R, mpack, B, st);
-      if (rc) return rc;
-      ClParams cp{x, u_in, y0R, mpack, mask_bstride ? 8 * kC128N : 0, mu, mu_stride, z_out, u_out, v_out, B, nullptr, nullptr};
-      return launch_cl128(cp, st);
-    }
-    if (H == 256 && W == 256) {
-      float2* y0R = work;
-      uint16_t* mpack = reinterpret_cast<uint16_t*>(work + size_t(B) * H * W);
-      int rc = prox_prepare_cl(y0, mask, mask_bstride, y0R, mpack, B, st);
-      if (rc) return rc;
-      ClParams cp{x, u_in, y0R, mpack, mask_bstride ? 16 * kClN : 0, mu, mu_stride, z_out, u_out, v_out, B, nullptr, nullptr};
-      return launch_cl(cp, st);
-    }
+    return prox_dual_any(x, u_in, y0, mask, mask_bstride, mu, mu_stride, z_out, u_out, v_out, work, B, H, W, st, nullptr);
+  if (cluster_shape(H, W)) {
+    uint16_t* mpack = reinterpret_cast<uint16_t*>(work + size_t(B) * H * W);
+    int rc = prepare_cluster(y0, mask, mask_bstride, work, mpack, B, H, nullptr, st);
+    if (rc) return rc;
+    return launch_cluster(x, u_in, work, mpack, mask_bstride != 0, mu, mu_stride, z_out, u_out, v_out, B, H, nullptr, nullptr,
+                          st);
   }
-  const float inv = 1.0f / sqrtf(float(H) * float(W));
-  int rc = radix_rows(ProxRowsIn{{}, x, u_in, work, skip_flag}, H, W, B, st);
-  if (rc == 0)
-    rc = radix_cols(ProxColsBlend{{{}, y0, mask, mask_bstride, mu, mu_stride}, work, inv, centre_sign(H, W), skip_flag},
-                    H, W, B, st);
-  if (rc == 0)
-    rc = radix_rows(ProxRowsOut{{{}, x, u_in, z_out, u_out, v_out, active}, work, inv, skip_flag}, H, W, B, st);
-  return rc;
+  return prox_radix3(x, u_in, y0, mask, mask_bstride, mu, mu_stride, z_out, u_out, v_out, work, B, H, W, nullptr, nullptr, st);
 }
 
 // Stand-alone centred orthonormal 2-D transform (mirror of transformations.py fft / ifft). dst may equal src.

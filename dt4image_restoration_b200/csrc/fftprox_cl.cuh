@@ -443,35 +443,31 @@ template <int CL> __global__ void __launch_bounds__(ClCfg<CL>::THREADS) cl_occup
   if (p) p[0] = probe_sm[0];
 }
 
-template <int CL>
-static int launch_cl_t(const ClParams& p, cudaStream_t st) {
-  constexpr size_t kSmem = ClCfg<CL>::SMEM;
+// Launch of a persistent cluster kernel (one image per cluster at a time) with every cluster that can be resident, at
+// most one per image.  `Probe` stands in for `Kernel` in the occupancy query (see cl_occupancy_probe).
+template <void (*Kernel)(ClParams), void (*Probe)(int*)>
+static int launch_resident_clusters(const ClParams& p, int cl, int threads, size_t smem, cudaStream_t st) {
   static bool attr_done = false;
   if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(fftprox_cl_kernel<CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kSmem));
-    if (e != cudaSuccess) return int(e);
-    e = cudaFuncSetAttribute(cl_occupancy_probe<CL>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kSmem));
-    if (e != cudaSuccess) return int(e);
-    if (CL > 8) {
-      e = cudaFuncSetAttribute(fftprox_cl_kernel<CL>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
-      if (e != cudaSuccess) return int(e);
-      e = cudaFuncSetAttribute(cl_occupancy_probe<CL>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
+    for (const void* f : {reinterpret_cast<const void*>(Kernel), reinterpret_cast<const void*>(Probe)}) {
+      cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+      if (e == cudaSuccess && cl > 8) e = cudaFuncSetAttribute(f, cudaFuncAttributeNonPortableClusterSizeAllowed, 1);
       if (e != cudaSuccess) return int(e);
     }
     attr_done = true;
   }
   cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(CL);
-  cfg.blockDim = dim3(ClCfg<CL>::THREADS);
-  cfg.dynamicSmemBytes = kSmem;
+  cfg.gridDim = dim3(cl * 64);
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem;
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL;
+  attr[0].val.clusterDim.x = cl;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
-  // (default cluster scheduling policy: load balancing reports a 15th 16-CTA cluster that never becomes resident with this
-  // kernel's register use, and the launch falls off a wave cliff - profiles/r02_prox_cl_steps.txt)
+  // (default cluster scheduling policy: load balancing reports a 15th 16-CTA cluster that never becomes resident with the
+  // 256x256 kernel's register use, and the launch falls off a wave cliff - profiles/r02_prox_cl_steps.txt)
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[1].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
@@ -479,8 +475,7 @@ static int launch_cl_t(const ClParams& p, cudaStream_t st) {
   static int max_clusters = 0;
   if (max_clusters == 0) {
     int n = 0;
-    cfg.gridDim = dim3(CL * 64);
-    if (cudaOccupancyMaxActiveClusters(&n, cl_occupancy_probe<CL>, &cfg) != cudaSuccess || n < 1) {
+    if (cudaOccupancyMaxActiveClusters(&n, Probe, &cfg) != cudaSuccess || n < 1) {
       (void)cudaGetLastError();
       n = 1;
     }
@@ -490,10 +485,16 @@ static int launch_cl_t(const ClParams& p, cudaStream_t st) {
   if (clusters < 1) clusters = 1;
   // all resident clusters are used even when the last round is partial (evening the rounds out - the smallest cluster count
   // with the same number of rounds - was right for the unpipelined kernel; now the clusters of a partial last round run with
-  // less contention: B = 20: 21.6 vs 27.8 us, B = 100: 84.2 vs 89.9 us, B = 64: 59.0 vs 59.8 us)
-  cfg.gridDim = dim3(clusters * CL);
+  // less contention, all resident vs evened out: 256x256 B = 20: 21.6 vs 27.8 us, B = 100: 84.2 vs 89.9 us, B = 64: 59.0 vs
+  // 59.8 us; 128x128 B = 100: 21.8 vs 28.7 us, B = 1024: 192.0 vs 197.3 us)
+  cfg.gridDim = dim3(clusters * cl);
   cfg.numAttrs = 2;
-  return int(cudaLaunchKernelEx(&cfg, fftprox_cl_kernel<CL>, p));
+  return int(cudaLaunchKernelEx(&cfg, Kernel, p));
+}
+
+static int launch_cl(const ClParams& p, cudaStream_t st) {
+  return launch_resident_clusters<fftprox_cl_kernel<16>, cl_occupancy_probe<16>>(p, 16, ClCfg<16>::THREADS, ClCfg<16>::SMEM,
+                                                                                  st);
 }
 
 }  // namespace pnp

@@ -292,44 +292,7 @@ __global__ void __launch_bounds__(kC128Threads) cl128_occupancy_probe(int* p) {
 }
 
 static int launch_cl128(const ClParams& p, cudaStream_t st) {
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(fftprox_cl128_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kC128Smem));
-    if (e != cudaSuccess) return int(e);
-    e = cudaFuncSetAttribute(cl128_occupancy_probe, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kC128Smem));
-    if (e != cudaSuccess) return int(e);
-    attr_done = true;
-  }
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(kC128CL * 64);
-  cfg.blockDim = dim3(kC128Threads);
-  cfg.dynamicSmemBytes = kC128Smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kC128CL;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  static int max_clusters = 0;
-  if (max_clusters == 0) {
-    int n = 0;
-    if (cudaOccupancyMaxActiveClusters(&n, cl128_occupancy_probe, &cfg) != cudaSuccess || n < 1) {
-      (void)cudaGetLastError();
-      n = 1;
-    }
-    max_clusters = n;
-  }
-  int clusters = max_clusters < p.B ? max_clusters : p.B;
-  if (clusters < 1) clusters = 1;
-  // every resident cluster is used, a partial last round included (evening the rounds out was measured slower here too:
-  // B = 100: 28.7 vs 21.8 us, B = 1024: 197.3 vs 192.0 us)
-  cfg.gridDim = dim3(clusters * kC128CL);
-  cfg.numAttrs = 2;
-  return int(cudaLaunchKernelEx(&cfg, fftprox_cl128_kernel, p));
+  return launch_resident_clusters<fftprox_cl128_kernel, cl128_occupancy_probe>(p, kC128CL, kC128Threads, kC128Smem, st);
 }
 
 }  // namespace pnp

@@ -38,29 +38,21 @@ class PnPEngine:
         self.ssim_out = torch.zeros(B, dtype=torch.float32, device=dev)
         self.ssim_work = ops.aligned_empty(_lib.lib().pnp_ssim_workspace_bytes(B, H, W), dev, align=16)
         self.work = torch.empty(_lib.lib().pnp_prox_workspace_bytes(B, H, W), dtype=torch.uint8, device=dev)
-        # shapes with a prepared single-launch prox kernel keep transposed, sign-folded copies of y0 / mask
-        self.prepared = bool(_lib.lib().pnp_prox_prepared_supported(H, W))
+        # shapes with a prepared prox path keep the trajectory constants derived from y0 / mask (ops.ProxPrepared)
+        self.prepared = ops.ProxPrepared.supported(H, W)
         if self.prepared:
-            import ctypes as C
-            n_y, n_m = C.c_size_t(0), C.c_size_t(0)
-            check(_lib.lib().pnp_prox_prepared_bytes(B, H, W, C.byref(n_y), C.byref(n_m)), "pnp_prox_prepared_bytes")
-            # y0T: transposed y0 + column-transformed y0; maskT: transposed mask + packed row mask + structure flag
-            self.y0T = torch.zeros(n_y.value // 8, dtype=torch.complex64, device=dev)
-            self.maskT = torch.zeros(n_m.value, dtype=torch.uint8, device=dev)
+            self.prep = ops.ProxPrepared.empty(B, H, W, dev)
         self.iters = 0
+
+    # the prepared buffers and the host-side mask-kind hint, under the names bench.py and tools/ncu_step.py read
+    y0T = property(lambda self: self.prep.y0p)
+    maskT = property(lambda self: self.prep.maskp)
+    probe = property(lambda self: self.prep.probe)
 
     @property
     def launches_per_step(self) -> int:
-        """Kernel launches of one step: the denoiser's op list (depends on L2 chunking) + 3 FFT-prox launches."""
-        if self.prepared:      # one prox launch once the mask kind is known on the host, else row-only + general kernels
-            known = getattr(self, "probe", None) is not None and self.probe.get() >= 0
-            single = (self.H, self.W) in ((256, 256), (128, 128))
-            n_prox = 1 if (known and (single or self.probe.get() == 1)) else (2 if single else (3 if known else 4))
-            if (self.H, self.W) == (128, 128):
-                n_prox = 1       # the 4-CTA cluster kernel serves every mask at 128x128
-        else:
-            n_prox = 3
-        return _lib.lib().pnp_unet_num_launches(self.plan.handle) + n_prox
+        """Kernel launches of one step: the denoiser's op list (depends on L2 chunking) + the FFT-prox launches."""
+        return _lib.lib().pnp_unet_num_launches(self.plan.handle) + (self.prep.launches if self.prepared else 3)
 
     def reset(self, data: dict, non_blocking: bool = False):
         """Same item dict as ``PnPEnv.reset`` (reference env.py:57-71), batch on dim 0."""
@@ -93,19 +85,9 @@ class PnPEngine:
         / ``[H,W]``; pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``, CUDA), ``accel`` (Cartesian masks
         drawn with ``seeds``), ``radial`` (radial masks with this sampled fraction, rotated by ``seeds``) and ``vd`` (the
         acceleration of variable-density masks drawn with ``seeds``)."""
-        if sum(m is not None for m in (mask, accel, radial, vd)) != 1:
-            raise ValueError("pass exactly one of mask / accel / radial / vd")
         B, H, W = self.B, self.H, self.W
         seeds = ops._seed_tensor(seeds, B, self.device)
-        if accel is not None:
-            ops.cartesian_masks(B, H, W, accel, seeds, out=self.mask)
-        elif radial is not None:
-            ops.radial_masks(B, H, W, radial, seeds, out=self.mask)
-        elif vd is not None:
-            ops.variable_density_masks(B, H, W, vd, seeds, out=self.mask)
-        else:
-            m = ops._mask_u8(mask).reshape(-1, 1, H, W)
-            self.mask.copy_(m.ne(0).expand(B, 1, H, W))
+        ops._episode_masks(B, H, W, seeds, mask, accel, radial, vd, out=self.mask)
         self.gt.copy_(ops._req(gt, torch.float32, "gt").reshape(-1, 1, H, W).expand(B, 1, H, W))
         ops.simulate_measurements(self.gt, self.mask, sigma_n, seeds, aty0=False, out=(self.y0, self.z, None))
         self.u.zero_()
@@ -117,10 +99,7 @@ class PnPEngine:
     def prepare(self):
         """Refresh the prepared copies after ``y0`` / ``mask`` changed (they are constants of a trajectory)."""
         if self.prepared:
-            check(_lib.lib().pnp_prox_prepare(self.y0.data_ptr(), self.mask.data_ptr(), self.H * self.W,
-                                              self.y0T.data_ptr(), self.maskT.data_ptr(), self.B, self.H, self.W,
-                                              _lib.stream_ptr()), "pnp_prox_prepare")
-            self.probe = ops.MaskKindProbe(self.maskT, self.H * self.W, self.B, self.H, self.W)
+            self.prep.prepare(self.y0, self.mask)
 
     def set_actions(self, sigma_d, mu):
         """Device-side action buffers: ``sigma_d`` ``[B]``, ``mu`` scalar or ``[B]`` (tensors or floats)."""
@@ -143,11 +122,11 @@ class PnPEngine:
                 active = active.reshape(-1)
                 if active.numel() != self.B or not active.is_cuda or active.dtype != torch.uint8:
                     raise RuntimeError(f"active must be a bool / uint8 CUDA tensor with {self.B} elements")
-            kind = self.probe.get() if getattr(self, "probe", None) is not None else -1
+            p = self.prep
             check(_lib.lib().pnp_step_prepared_active(self.plan.handle, self.v.data_ptr(), self.sigma.data_ptr(),
-                                                      self.u.data_ptr(), self.y0T.data_ptr(), self.maskT.data_ptr(),
-                                                      self.H * self.W, self.mu.data_ptr(), 1, self.x.data_ptr(),
-                                                      self.z.data_ptr(), self.u.data_ptr(), self.v.data_ptr(), kind,
+                                                      self.u.data_ptr(), p.y0p.data_ptr(), p.maskp.data_ptr(), p.mstride,
+                                                      self.mu.data_ptr(), 1, self.x.data_ptr(), self.z.data_ptr(),
+                                                      self.u.data_ptr(), self.v.data_ptr(), p.probe.get(),
                                                       active.data_ptr() if active is not None else None,
                                                       _lib.stream_ptr()), "pnp_step_prepared_active")
         else:

@@ -35,7 +35,6 @@ class _GraphedStep:
     references to old ones, reference mcts.py:15,18) is kept by ONE copy of the flat state into a new allocation."""
 
     def __init__(self, denoiser: UNetDenoiser2D, B: int, H: int, W: int, device):
-        import ctypes as C
         self.B, self.H, self.W, self.dev = B, H, W, device
         n = B * H * W
         self.flat = torch.zeros(n * 5, dtype=torch.float32, device=device)         # x: n floats, z: 2n, u: 2n
@@ -45,12 +44,7 @@ class _GraphedStep:
         self.v = torch.zeros(B, 1, H, W, dtype=torch.float32, device=device)
         self.sigma = torch.zeros(B, dtype=torch.float32, device=device)
         self.mu = torch.zeros(1, dtype=torch.float32, device=device)
-        l = _lib.lib()
-        n_y, n_m = C.c_size_t(0), C.c_size_t(0)
-        check(l.pnp_prox_prepared_bytes(B, H, W, C.byref(n_y), C.byref(n_m)), "pnp_prox_prepared_bytes")
-        self.y0p = torch.zeros(n_y.value // 8, dtype=torch.complex64, device=device)
-        self.maskp = torch.zeros(n_m.value, dtype=torch.uint8, device=device)
-        self.mstride = 0
+        self.prep = ops.ProxPrepared.empty(B, H, W, device)
         self.plan = denoiser.plan(B, H, W)
         self.prep_key = None
         self.last_out = None                    # (z, u) handed out by the last step and their versions
@@ -61,24 +55,19 @@ class _GraphedStep:
                (y0.data_ptr(), y0._version, mask.data_ptr(), mask._version, tuple(mask.shape)))
         if key == self.prep_key:
             return
-        m = mask.contiguous().view(torch.uint8) if mask.dtype == torch.bool else mask.contiguous()
-        mstride = self.H * self.W if m.numel() == self.B * self.H * self.W else 0
-        if m.numel() not in (self.B * self.H * self.W, self.H * self.W):
-            raise IndexError(f"mask with {m.numel()} elements does not match y0 {tuple(y0.shape)}")
-        if mstride != self.mstride and self.graph is not None:
+        mstride = self.prep.mstride
+        self.prep.prepare(y0, mask)             # IndexError for a mask that does not match
+        if self.prep.mstride != mstride:
             self.graph = None                   # the mask stride is baked into the captured launch
-        self.mstride = mstride
-        check(_lib.lib().pnp_prox_prepare(y0.contiguous().data_ptr(), m.data_ptr(), mstride, self.y0p.data_ptr(),
-                                          self.maskp.data_ptr(), self.B, self.H, self.W, _lib.stream_ptr()), "pnp_prox_prepare")
         self.prep_key, self._keep = key, (y0, mask)
 
     def _body(self):
-        l = _lib.lib()
+        l, p = _lib.lib(), self.prep
         n = self.z.numel()
         check(l.pnp_residual_real(self.z.data_ptr(), self.u.data_ptr(), self.v.data_ptr(), n, _lib.stream_ptr()),
               "pnp_residual_real")
         check(l.pnp_step_prepared_kind(self.plan.handle, self.v.data_ptr(), self.sigma.data_ptr(), self.u.data_ptr(),
-                                       self.y0p.data_ptr(), self.maskp.data_ptr(), self.mstride, self.mu.data_ptr(), 0,
+                                       p.y0p.data_ptr(), p.maskp.data_ptr(), p.mstride, self.mu.data_ptr(), 0,
                                        self.x.data_ptr(), self.z.data_ptr(), self.u.data_ptr(), None, -1,
                                        _lib.stream_ptr()), "pnp_step_prepared_kind")
 

@@ -84,10 +84,20 @@ def fft2c(x: torch.Tensor, inverse: bool = False) -> torch.Tensor:
     return out
 
 
-def _mask_u8(mask: torch.Tensor) -> torch.Tensor:
+def _mask_arg(mask: torch.Tensor, B: int, H: int, W: int):
+    """bool/uint8 mask(s) of B images or one shared image -> (uint8 CUDA tensor, batch stride ``H*W`` or 0)."""
     if mask.dtype == torch.bool:
         mask = mask.contiguous().view(torch.uint8)
-    return _req(mask, torch.uint8, "mask")
+    mask = _req(mask, torch.uint8, "mask")
+    if mask.numel() not in (B * H * W, H * W):
+        raise IndexError(f"mask with {mask.numel()} elements does not match {B} images of {H}x{W}")
+    return mask, H * W if mask.numel() == B * H * W else 0
+
+
+def _check_out(t: torch.Tensor, dtype, numel: int, name: str = "out"):
+    """A caller-provided output buffer: contiguous, on the device, of ``dtype`` and ``numel`` elements."""
+    if not t.is_cuda or t.dtype != dtype or not t.is_contiguous() or t.numel() != numel:
+        raise _lib.PnpError(f"{name} must be a contiguous {dtype} CUDA tensor with {numel} elements")
 
 
 def _seed_tensor(seeds, B: int, device) -> torch.Tensor:
@@ -137,10 +147,7 @@ def simulate_measurements(gt, mask, sigma_n, seeds, aty0: bool = True, out=None)
     gt_stride = H * W if gt.numel() == B * H * W else 0
     if gt.numel() not in (B * H * W, H * W):
         raise RuntimeError(f"gt has {gt.numel()} elements, expected {B * H * W} or {H * W}")
-    mask = _mask_u8(mask)
-    if mask.numel() not in (B * H * W, H * W):
-        raise IndexError(f"mask with {mask.numel()} elements does not match {B} images of {H}x{W}")
-    mstride = H * W if mask.numel() == B * H * W else 0
+    mask, mstride = _mask_arg(mask, B, H, W)
     sig, sstride = _per_image(sigma_n, B, torch.float32, "sigma_n", gt.device)
     seeds = _seed_tensor(seeds, B, gt.device)
     if out is None:
@@ -150,8 +157,7 @@ def simulate_measurements(gt, mask, sigma_n, seeds, aty0: bool = True, out=None)
     else:
         y0, x0, at = out
         for t in (y0, x0) + ((at,) if at is not None else ()):
-            if not t.is_cuda or t.dtype != torch.complex64 or not t.is_contiguous() or t.numel() != B * H * W:
-                raise RuntimeError(f"out tensors must be contiguous complex64 CUDA tensors with {B * H * W} elements")
+            _check_out(t, torch.complex64, B * H * W)
     check(_lib.lib().pnp_simulate_measurements(gt.data_ptr(), gt_stride, mask.data_ptr(), mstride, sig.data_ptr(), sstride,
                                                seeds.data_ptr(), y0.data_ptr(), x0.data_ptr(),
                                                at.data_ptr() if at is not None else None, B, H, W, _lib.stream_ptr()),
@@ -171,8 +177,7 @@ def cartesian_masks(B: int, H: int, W: int, accel, seeds, acs_frac: float = 0.08
     acs_cols = max(1, int(round(acs_frac * W)))
     if out is None:
         out = torch.empty(B, H, W, dtype=torch.uint8, device=dev)
-    elif not out.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous() or out.numel() != B * H * W:
-        raise RuntimeError(f"out must be a contiguous uint8 CUDA tensor with {B * H * W} elements")
+    _check_out(out, torch.uint8, B * H * W)
     check(_lib.lib().pnp_cartesian_masks(acc.data_ptr(), astride, seeds.data_ptr(), acs_cols, out.data_ptr(), B, H, W,
                                          _lib.stream_ptr()), "pnp_cartesian_masks")
     return out
@@ -189,11 +194,9 @@ def radial_masks(B: int, H: int, W: int, frac, seeds=None, out=None, lines_out=N
     seeds = _seed_tensor(seeds, B, dev) if seeds is not None else None
     if out is None:
         out = torch.empty(B, H, W, dtype=torch.uint8, device=dev)
-    elif not out.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous() or out.numel() != B * H * W:
-        raise _lib.PnpError(f"out must be a contiguous uint8 CUDA tensor with {B * H * W} elements")
-    if lines_out is not None and (not lines_out.is_cuda or lines_out.dtype != torch.int32 or not lines_out.is_contiguous()
-                                  or lines_out.numel() != B):
-        raise _lib.PnpError(f"lines_out must be a contiguous int32 CUDA tensor with {B} elements")
+    _check_out(out, torch.uint8, B * H * W)
+    if lines_out is not None:
+        _check_out(lines_out, torch.int32, B, "lines_out")
     check(_lib.lib().pnp_radial_masks(fr.data_ptr(), fstride, seeds.data_ptr() if seeds is not None else None,
                                       out.data_ptr(), lines_out.data_ptr() if lines_out is not None else None, B, H, W,
                                       _lib.stream_ptr()), "pnp_radial_masks")
@@ -215,10 +218,29 @@ def variable_density_masks(B: int, H: int, W: int, accel, seeds, power: int = 3,
     acs_h, acs_w = max(1, int(round(acs_frac * H))), max(1, int(round(acs_frac * W)))
     if out is None:
         out = torch.empty(B, H, W, dtype=torch.uint8, device=dev)
-    elif not out.is_cuda or out.dtype != torch.uint8 or not out.is_contiguous() or out.numel() != B * H * W:
-        raise _lib.PnpError(f"out must be a contiguous uint8 CUDA tensor with {B * H * W} elements")
+    _check_out(out, torch.uint8, B * H * W)
     check(_lib.lib().pnp_variable_density_masks(acc.data_ptr(), astride, seeds.data_ptr(), acs_h, acs_w, int(power),
                                                 out.data_ptr(), B, H, W, _lib.stream_ptr()), "pnp_variable_density_masks")
+    return out
+
+
+def _episode_masks(B: int, H: int, W: int, seeds, mask=None, accel=None, radial=None, vd=None, out=None) -> torch.Tensor:
+    """The uint8 ``[B,H,W]`` masks of a batch of episodes (written into ``out`` when given) from exactly one of ``mask``
+    (bool/uint8 ``[B or 1, ..., H, W]``, read as ``!= 0``; one mask serves every image), ``accel`` (``cartesian_masks``),
+    ``radial`` (``radial_masks``) and ``vd`` (``variable_density_masks``), the last three drawn with ``seeds``."""
+    if sum(m is not None for m in (mask, accel, radial, vd)) != 1:
+        raise ValueError("pass exactly one of mask / accel / radial / vd")
+    if accel is not None:
+        return cartesian_masks(B, H, W, accel, seeds, out=out)
+    if radial is not None:
+        return radial_masks(B, H, W, radial, seeds, out=out)
+    if vd is not None:
+        return variable_density_masks(B, H, W, vd, seeds, out=out)
+    mask = _mask_arg(mask, B, H, W)[0].ne(0).reshape(-1, H, W).expand(B, H, W)
+    if out is None:
+        return mask.to(torch.uint8).contiguous()
+    _check_out(out, torch.uint8, B * H * W)
+    out.view(B, H, W).copy_(mask)
     return out
 
 
@@ -228,19 +250,10 @@ def make_items(gt, sigma_n, seeds, mask=None, accel=None, radial=None, vd=None) 
     Pass exactly one of ``mask`` (bool/uint8 ``[B or 1, ..., H, W]``), ``accel`` (Cartesian masks drawn with ``seeds``),
     ``radial`` (the sampled fraction of radial masks rotated by ``seeds``, see ``radial_masks``) and ``vd`` (the
     acceleration of variable-density masks drawn with ``seeds``, default power and ACS of ``variable_density_masks``)."""
-    if sum(m is not None for m in (mask, accel, radial, vd)) != 1:
-        raise ValueError("pass exactly one of mask / accel / radial / vd")
     gt = _req(gt, torch.float32, "gt")
     H, W = gt.shape[-2:]
     B = _batch_size(gt, mask, sigma_n, seeds)
-    if accel is not None:
-        mask = cartesian_masks(B, H, W, accel, seeds)
-    elif radial is not None:
-        mask = radial_masks(B, H, W, radial, seeds)
-    elif vd is not None:
-        mask = variable_density_masks(B, H, W, vd, seeds)
-    else:
-        mask = _mask_u8(mask).ne(0).to(torch.uint8).reshape(-1, H, W).expand(B, H, W).contiguous()
+    mask = _episode_masks(B, H, W, seeds, mask, accel, radial, vd)
     y0, x0, aty0 = simulate_measurements(gt, mask, sigma_n, seeds)
     return {"x0": torch.view_as_real(x0), "y0": torch.view_as_real(y0), "ATy0": torch.view_as_real(aty0), "mask": mask,
             "gt": gt.reshape(-1, 1, H, W).expand(B, 1, H, W).contiguous()}
@@ -260,81 +273,101 @@ class MaskKindProbe:
     """Host-side view of the mask-structure flag that ``pnp_prox_prepare`` leaves on the device, WITHOUT a synchronisation:
     an asynchronous 4-byte copy into pinned memory plus an event.  ``get()`` returns -1 until the copy has landed, then
     1 (every mask depends on the column index only: row kernel) or 0 (general masks: cluster kernel) - the ``kind``
-    argument of ``pnp_prox_dual_prepared_kind`` / ``pnp_step_prepared_kind`` (-1 launches both kernels)."""
+    argument of ``pnp_prox_dual_prepared_kind`` / ``pnp_step_prepared_kind`` (-1 launches both kernels).  Without
+    ``maskp`` (nothing prepared yet) ``get()`` stays -1."""
 
-    def __init__(self, maskp: torch.Tensor, mstride: int, B: int, H: int, W: int):
+    def __init__(self, maskp: torch.Tensor | None = None, mstride: int = 0, B: int = 0, H: int = 0, W: int = 0):
+        self.kind, self.event = -1, None
+        if maskp is None:
+            return
         self.host = torch.full((1,), -1, dtype=torch.int32).pin_memory()
         check(_lib.lib().pnp_prox_prepared_kind_async(maskp.data_ptr(), mstride, B, H, W, self.host.data_ptr(),
                                                       _lib.stream_ptr()), "pnp_prox_prepared_kind_async")
         self.event = torch.cuda.Event()
         self.event.record()
-        self.kind = -1
 
     def get(self) -> int:
-        if self.kind < 0 and not torch.cuda.is_current_stream_capturing() and self.event.query():
+        if (self.kind < 0 and self.event is not None and not torch.cuda.is_current_stream_capturing()
+                and self.event.query()):
             self.kind = 1 if int(self.host[0]) != 0 else 0
         return self.kind
 
 
 class ProxPrepared:
-    """Trajectory constants of the prox step, prepared once (``pnp_prox_prepare``): see include/pnp_b200.h.
+    """Trajectory constants of the prox step (``pnp_prox_prepare``, see include/pnp_b200.h): the buffers ``y0p`` and
+    ``maskp``, their mask stride and the host-side mask-kind hint ``probe``.
 
     ``ProxPrepared(y0, mask)`` then ``prep.prox_dual(x, u, mu)`` per iteration; same results as ``prox_dual``.
-    Only for shapes with a prepared path (``supported(H, W)``: 256x256)."""
+    ``ProxPrepared.empty(B, H, W, device)`` allocates the buffers zero-filled and ``prep.prepare(y0, mask)`` (re)fills them
+    in place, so CUDA graphs that captured them stay valid for the next trajectory.
+    Only for shapes with a prepared path (``supported(H, W)``)."""
 
     @staticmethod
     def supported(H: int, W: int) -> bool:
         return bool(_lib.lib().pnp_prox_prepared_supported(H, W))
 
     def __init__(self, y0, mask):
-        import ctypes as C
         y0 = _req(y0, torch.complex64, "y0")
         H, W = y0.shape[-2:]
-        B = y0.numel() // (H * W)
-        if mask.dtype == torch.bool:
-            mask = mask.contiguous().view(torch.uint8)
-        mask = _req(mask, torch.uint8, "mask")
-        if mask.numel() == B * H * W:
-            self.mstride = H * W
-        elif mask.numel() == H * W:
-            self.mstride = 0
-        else:
-            raise IndexError(f"mask with {mask.numel()} elements does not match y0 {tuple(y0.shape)}")
-        self.B, self.H, self.W = B, H, W
-        l = _lib.lib()
+        self._allocate(y0.numel() // (H * W), H, W, y0.device)
+        self.prepare(y0, mask)
+
+    @classmethod
+    def empty(cls, B: int, H: int, W: int, device) -> "ProxPrepared":
+        prep = cls.__new__(cls)
+        prep._allocate(B, H, W, device)
+        return prep
+
+    def _allocate(self, B: int, H: int, W: int, device):
         n_y, n_m = C.c_size_t(0), C.c_size_t(0)
-        check(l.pnp_prox_prepared_bytes(B, H, W, C.byref(n_y), C.byref(n_m)), "pnp_prox_prepared_bytes")
-        self.y0p = torch.empty(n_y.value // 8, dtype=torch.complex64, device=y0.device)
-        self.maskp = torch.empty(n_m.value, dtype=torch.uint8, device=y0.device)
-        check(l.pnp_prox_prepare(y0.data_ptr(), mask.data_ptr(), self.mstride, self.y0p.data_ptr(), self.maskp.data_ptr(),
-                                 B, H, W, _lib.stream_ptr()), "pnp_prox_prepare")
+        check(_lib.lib().pnp_prox_prepared_bytes(B, H, W, C.byref(n_y), C.byref(n_m)), "pnp_prox_prepared_bytes")
+        self.B, self.H, self.W = B, H, W
+        self.y0p = torch.zeros(n_y.value // 8, dtype=torch.complex64, device=device)
+        self.maskp = torch.zeros(n_m.value, dtype=torch.uint8, device=device)
+        self.mstride = 0
+        self.probe = MaskKindProbe()
+
+    def prepare(self, y0, mask):
+        """Prepare ``y0`` (complex64, B images) and ``mask`` (bool/uint8, B masks or one for the batch) into the buffers."""
+        B, H, W = self.B, self.H, self.W
+        y0 = _req(y0, torch.complex64, "y0")
+        if y0.numel() != B * H * W:
+            raise IndexError(f"y0 with {y0.numel()} elements does not match {B} images of {H}x{W}")
+        mask, self.mstride = _mask_arg(mask, B, H, W)
+        check(_lib.lib().pnp_prox_prepare(y0.data_ptr(), mask.data_ptr(), self.mstride, self.y0p.data_ptr(),
+                                          self.maskp.data_ptr(), B, H, W, _lib.stream_ptr()), "pnp_prox_prepare")
         self.probe = MaskKindProbe(self.maskp, self.mstride, B, H, W)
 
     @property
     def column_only(self) -> bool:
         """Did the preparation find every mask of the batch to depend on the column index only? (synchronises)"""
-        nb = self.B if self.mstride else 1                   # layout documented in csrc/fftprox.cu (prox_prepared_bytes)
-        stride = 32 if (self.H == 256 and self.W == 256) else self.W
-        off = ((nb * self.H * self.W + 15) // 16 * 16 + nb * stride + 15) // 16 * 16
-        return bool(self.maskp[off:off + 4].view(torch.int32).item() != 0)
+        self.probe.event.synchronize()
+        return self.probe.get() == 1
+
+    @property
+    def launches(self) -> int:
+        """Kernel launches of one ``prox_dual`` with the current host-side hint (the routing of ``pnp_prox_dual_prepared``)."""
+        kind = self.probe.get()
+        if (self.H, self.W) == (128, 128):
+            return 1                          # the 4-CTA cluster kernel serves every mask
+        if (self.H, self.W) == (256, 256):
+            return 1 if kind >= 0 else 2      # row-only or cluster kernel; both while the kind is unknown
+        return {1: 1, 0: 3}.get(kind, 4)      # row-only kernel, the three radix passes, or both
 
     def prox_dual(self, x, u, mu, want_v: bool = True, out=None, kind: int | None = None):
         """``kind``: None = use the host-side hint once it has landed; -1 forces the both-kernels launch."""
         x = _req(x, torch.float32, "x")
         u = _req(u, torch.complex64, "u")
-        B = self.B
-        mu = _req(mu.reshape(-1).float(), torch.float32, "mu")
-        if mu.numel() not in (1, B):
-            raise RuntimeError(f"mu must have 1 or {B} elements, got {mu.numel()}")
+        mu, mu_stride = _per_image(mu.float(), self.B, torch.float32, "mu", x.device)
         if out is None:
             z, un = torch.empty_like(u), torch.empty_like(u)
             v = torch.empty_like(x) if want_v else None
         else:
             z, un, v = out
         check(_lib.lib().pnp_prox_dual_prepared_kind(x.data_ptr(), u.data_ptr(), self.y0p.data_ptr(), self.maskp.data_ptr(),
-                                                     self.mstride, mu.data_ptr(), 0 if mu.numel() == 1 else 1, z.data_ptr(),
-                                                     un.data_ptr(), v.data_ptr() if v is not None else None, B, self.H,
-                                                     self.W, self.probe.get() if kind is None else kind, _lib.stream_ptr()),
+                                                     self.mstride, mu.data_ptr(), mu_stride, z.data_ptr(), un.data_ptr(),
+                                                     v.data_ptr() if v is not None else None, self.B, self.H, self.W,
+                                                     self.probe.get() if kind is None else kind, _lib.stream_ptr()),
               "pnp_prox_dual_prepared_kind")
         return z, un, v
 
@@ -349,22 +382,8 @@ def prox_dual(x, u, y0, mask, mu, want_v: bool = True, out=None, workspace=None)
     y0 = _req(y0, torch.complex64, "y0")
     H, W = x.shape[-2:]
     B = x.numel() // (H * W)
-    if mask.dtype == torch.bool:
-        mask = mask.contiguous().view(torch.uint8)
-    mask = _req(mask, torch.uint8, "mask")
-    if mask.numel() == B * H * W:
-        mstride = H * W
-    elif mask.numel() == H * W:
-        mstride = 0
-    else:
-        raise IndexError(f"mask with {mask.numel()} elements does not match x {tuple(x.shape)}")
-    mu = _req(mu.reshape(-1).float(), torch.float32, "mu")
-    if mu.numel() == 1:
-        mu_stride = 0
-    elif mu.numel() == B:
-        mu_stride = 1
-    else:
-        raise RuntimeError(f"mu must have 1 or {B} elements, got {mu.numel()}")
+    mask, mstride = _mask_arg(mask, B, H, W)
+    mu, mu_stride = _per_image(mu.float(), B, torch.float32, "mu", x.device)
     if out is None:
         z = torch.empty_like(u)
         un = torch.empty_like(u)
