@@ -70,6 +70,8 @@ SIGNATURES = {
     "pnp_unet_set_splitk": (c_int, [c_int]),
     "pnp_unet_plan_tensor": (c_int, [c_void_p, c_char_p, C.POINTER(c_size_t), C.POINTER(c_int), C.POINTER(c_int),
                                      C.POINTER(c_int)]),
+    "pnp_unet_forward_ops": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "pnp_unet_op_describe": (c_int, [c_void_p, c_int, C.POINTER(c_ll)]),
     "pnp_conv3x3_packed_bytes": (c_size_t, [c_int, c_int]),
     "pnp_conv3x3_bf16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                  c_int, c_int, c_int, c_void_p]),

@@ -379,6 +379,23 @@ int pnp_unet_plan_tensor(const pnp_unet_plan* plan, const char* name, size_t* by
   return unet_plan_tensor(plan->impl, name, byte_offset, C, H, W);
 }
 
+static_assert(kUnetOpDescLen == PNP_UNET_OP_DESC_LEN, "descriptor length");
+
+int pnp_unet_forward_ops(pnp_unet_plan* plan, const float* v, const float* sigma, float* x_out, float* preclamp,
+                         int first_op, int end_op, void* stream) {
+  REQUIRE_INIT();
+  if (!plan || !v || !sigma || !x_out) { set_error("pnp_unet_forward_ops: null pointer"); return -1; }
+  if (plan->mb != plan->B) { set_error("pnp_unet_forward_ops: the plan is micro-batched"); return -1; }
+  return fail_cuda(unet_forward_ops(plan->impl, v, sigma, x_out, preclamp, first_op, end_op, cudaStream_t(stream)),
+                   "pnp_unet_forward_ops");
+}
+
+int pnp_unet_op_describe(const pnp_unet_plan* plan, int i, long long* desc) {
+  if (!plan || !desc) { set_error("pnp_unet_op_describe: null pointer"); return -1; }
+  if (plan->mb != plan->B) { set_error("pnp_unet_op_describe: the plan is micro-batched"); return -1; }
+  return unet_op_describe(plan->impl, i, desc);
+}
+
 size_t pnp_policy_packed_floats(int n_time, int n_task) { return policy_packed_floats(n_time, n_task); }
 
 int pnp_policy_step(const float* packed, const float* rtg, const float* emb, float* act, const long long* timesteps,

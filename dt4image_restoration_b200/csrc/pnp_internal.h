@@ -76,6 +76,10 @@ int unet_forward(UnetPlan* p, const float* v, const float* sigma, float* x_out, 
 int unet_profile(UnetPlan* p, const float* v, const float* sigma, float* x_out, cudaStream_t st, float* ms, int* kinds,
                  int* ids, int* n_inout);
 int unet_num_launches(const UnetPlan* p);
+int unet_forward_ops(UnetPlan* p, const float* v, const float* sigma, float* x_out, float* preclamp, int first, int end,
+                     cudaStream_t st);
+constexpr int kUnetOpDescLen = 21;      // PNP_UNET_OP_DESC_LEN
+int unet_op_describe(const UnetPlan* p, int i, long long* desc);
 int unet_set_splitk(int mode);
 size_t conv_packed_bytes(int Cin, int Cout);
 int conv3x3_single(const __nv_bfloat16* in0, int C0, const __nv_bfloat16* in1, int C1, const float* w_fp32,

@@ -642,6 +642,7 @@ struct Op {
   int level;                // pyramid level the op writes
   int conv;                 // index into convs (K_UMMA)
   int rev;                  // sweep direction (alternates launch by launch, see ConvParams::rev)
+  const TensorSlot *in0, *in1, *out, *pool;   // workspace tensors read / written (null: none, or not in the workspace)
 };
 
 struct UnetPlan {
@@ -762,7 +763,8 @@ int unet_plan_create(UnetPlan** out, const uint8_t* packed, uint8_t* workspace, 
     if (epi == EPI_FINAL) { cl.p.wout = flat + ow; cl.p.bout = flat + ob; }
     if (pooled) cl.p.pool_out = T(*pooled);
     P->convs.push_back(cl);
-    P->ops.push_back(Op{K_UMMA, li, lvl, int(P->convs.size()) - 1});
+    // the FINAL epilogue writes x_out / preclamp, not `o`
+    P->ops.push_back(Op{K_UMMA, li, lvl, int(P->convs.size()) - 1, 0, &in0, in1, epi == EPI_FINAL ? nullptr : &o, pooled});
   };
   {
     // first-layer weights to the host (plan creation may synchronise): fp32 [32][2][3][3] + bias[32]
@@ -786,7 +788,7 @@ int unet_plan_create(UnetPlan** out, const uint8_t* packed, uint8_t* workspace, 
     }
   }
   // MaxPool2d(2) is fused into the epilogue of the conv that produces the skip tensor
-  P->ops.push_back(Op{K_FIRST, 0, 0, -1});
+  P->ops.push_back(Op{K_FIRST, 0, 0, -1, 0, nullptr, nullptr, &P->tA[0], nullptr});
   conv(1, P->tA[0], nullptr, P->tB[0], 0);
   conv(2, P->tB[0], nullptr, P->skip[0], 0, &P->pooled[1]);
   for (int l = 1; l <= 4; ++l) {
@@ -796,7 +798,7 @@ int unet_plan_create(UnetPlan** out, const uint8_t* packed, uint8_t* workspace, 
   }
   for (int l = 3; l >= 0; --l) {                    // up1 .. up4
     const int blk = 5 + (3 - l);
-    P->ops.push_back(Op{K_UPS, 200 + l, l, -1});
+    P->ops.push_back(Op{K_UPS, 200 + l, l, -1, 0, l == 3 ? &P->skip[4] : &P->tA[l + 1], nullptr, &P->ups[l], nullptr});
     conv(blk * 3 + 0, P->skip[l], &P->ups[l], P->tA[l], l);
     conv(blk * 3 + 1, P->tA[l], nullptr, P->tB[l], l);
     conv(blk * 3 + 2, P->tB[l], nullptr, P->tA[l], l);
@@ -856,13 +858,19 @@ struct ProfileCtx {
   void end() { cudaEventRecord(ev.back(), st); }
 };
 
+// The exact-doubling upsample into level l (no pad, source at least 2x2) takes upsample2x_fast_kernel.
+static bool ups_fast(const UnetPlan* P, int l) {
+  const int h = P->Hl[l + 1], w = P->Wl[l + 1];
+  return P->Hl[l] == 2 * h && P->Wl[l] == 2 * w && h > 1 && w > 1;
+}
+
+// Runs launches [first, end) of the plan (the whole forward is [0, ops.size())).
 static int unet_forward_impl(UnetPlan* P, const float* v, const float* sigma, float* x_out, float* preclamp,
-                             cudaStream_t st, ProfileCtx* prof, const uint8_t* active = nullptr) {
-  LayerDesc L[27]; size_t ow, ob, n, pk;
-  layer_table(L, ow, ob, n, pk);
+                             cudaStream_t st, ProfileCtx* prof, const uint8_t* active, int first, int end) {
   auto T = [&](const TensorSlot& s) { return reinterpret_cast<__nv_bfloat16*>(P->ws + s.off); };
   int rc = 0;
-  for (const Op& op : P->ops) {
+  for (int i = first; i < end; ++i) {
+    const Op& op = P->ops[i];
     if (prof) prof->begin();
     switch (op.kind) {
       case K_FIRST: {
@@ -882,13 +890,13 @@ static int unet_forward_impl(UnetPlan* P, const float* v, const float* sigma, fl
       }
       case K_UPS: {
         const int l = op.level;
-        const TensorSlot& lo = (l == 3) ? P->skip[4] : P->tA[l + 1];   // previous block's output
+        const TensorSlot& lo = *op.in0;                                // previous block's output
         const int h = P->Hl[l + 1], w = P->Wl[l + 1], Ho = P->Hl[l], Wo = P->Wl[l];
         const int C8 = kCh[l + 1] / 8;
         const int dy = Ho - 2 * h, dx = Wo - 2 * w;
         const float sy = (2 * h > 1) ? float(h - 1) / float(2 * h - 1) : 0.f;
         const float sx = (2 * w > 1) ? float(w - 1) / float(2 * w - 1) : 0.f;
-        if (dy == 0 && dx == 0 && h > 1 && w > 1)
+        if (ups_fast(P, l))
         {
           const int gx = ((w + 1) * C8 + 255) / 256;
           int walk = 8;                              // long walks only while the grid still fills the machine
@@ -912,10 +920,47 @@ static int unet_forward_impl(UnetPlan* P, const float* v, const float* sigma, fl
 
 int unet_forward(UnetPlan* P, const float* v, const float* sigma, float* x_out, float* preclamp, cudaStream_t st,
                  const uint8_t* active) {
-  return unet_forward_impl(P, v, sigma, x_out, preclamp, st, nullptr, active);
+  return unet_forward_impl(P, v, sigma, x_out, preclamp, st, nullptr, active, 0, int(P->ops.size()));
+}
+
+int unet_forward_ops(UnetPlan* P, const float* v, const float* sigma, float* x_out, float* preclamp, int first, int end,
+                     cudaStream_t st) {
+  if (first < 0 || end > int(P->ops.size()) || first > end) { set_error("unet: launch range out of bounds"); return -1; }
+  return unet_forward_impl(P, v, sigma, x_out, preclamp, st, nullptr, nullptr, first, end);
 }
 
 int unet_num_launches(const UnetPlan* P) { return int(P->ops.size()); }
+
+// What launch i of the plan is; the field order is documented at pnp_unet_op_describe (include/pnp_b200.h).
+int unet_op_describe(const UnetPlan* P, int i, long long* d) {
+  if (i < 0 || i >= int(P->ops.size())) { set_error("unet: launch index out of bounds"); return -1; }
+  const Op& op = P->ops[i];
+  for (int k = 0; k < kUnetOpDescLen; ++k) d[k] = -1;
+  d[0] = op.kind; d[1] = op.id; d[2] = P->Hl[op.level]; d[3] = P->Wl[op.level];
+  const TensorSlot* slots[4] = {op.in0, op.in1, op.out, op.pool};
+  for (int k = 0; k < 4; ++k)
+    if (slots[k]) { d[4 + 2 * k] = (long long)slots[k]->off; d[5 + 2 * k] = slots[k]->C; }
+  d[13] = d[14] = d[16] = 0;
+  d[15] = op.rev;
+  d[17] = d[18] = d[19] = d[20] = 0;
+  if (op.kind == K_FIRST) {
+    d[12] = 0;
+  } else if (op.kind == K_UPS) {
+    d[12] = ups_fast(P, op.level) ? 6 : 7;
+  } else {
+    const ConvLaunch& L = P->convs[op.conv];
+    const ConvParams& p = L.p;
+    d[12] = L.splitk ? 5 : L.pair ? 4 : L.kws ? 3 : L.EPI == EPI_FINAL ? 2 : 1;
+    d[13] = L.splitk ? p.sk_split : L.KC;
+    d[14] = L.splitk ? kSkBN : L.BN;
+    d[16] = L.splitk ? 0 : p.wres;
+    d[17] = L.kws ? kKwsTileW : kTile;
+    d[18] = L.kws ? kKwsTileH : kTile;
+    d[19] = p.total_tiles;
+    d[20] = L.grid;
+  }
+  return 0;
+}
 
 // Profiling pass: one forward with a CUDA-event pair around every launch; SYNCHRONISES the stream.
 // ms[i] = duration of launch i; kinds[i] in {0 first conv, 1 tcgen05 conv, 3 upsample};
@@ -924,7 +969,7 @@ int unet_profile(UnetPlan* P, const float* v, const float* sigma, float* x_out, 
                  int* kinds, int* ids, int* n_inout) {
   ProfileCtx prof;
   prof.st = st;
-  int rc = unet_forward_impl(P, v, sigma, x_out, nullptr, st, &prof);
+  int rc = unet_forward_impl(P, v, sigma, x_out, nullptr, st, &prof, nullptr, 0, int(P->ops.size()));
   cudaError_t e = cudaStreamSynchronize(st);
   const int n = int(prof.ev.size() / 2);
   const int cap = *n_inout;

@@ -505,6 +505,43 @@ class UNetPlan:
         n = self.B * h.value * w.value * c.value
         return self.workspace[off.value:off.value + 2 * n].view(torch.bfloat16).view(self.B, h.value, w.value, c.value)
 
+    # fields of pnp_unet_op_describe (include/pnp_b200.h), in order
+    _OP_FIELDS = ("kind", "id", "H", "W", "in0_off", "in0_C", "in1_off", "in1_C", "out_off", "out_C", "pool_off", "pool_C",
+                  "kernel", "kc", "bn", "rev", "wres", "tile_w", "tile_h", "tiles", "grid")
+    KERNELS = ("first", "umma", "final", "kws", "pair", "splitk", "ups_fast", "ups_general")
+
+    def describe(self) -> list[dict]:
+        """One dict per launch of the forward pass: what it reads and writes in the workspace and which kernel it runs
+        (``kernel`` is a name from ``KERNELS``; ``kc`` is the cluster size S for the split-K kernel)."""
+        l = _lib.lib()
+        desc = (C.c_longlong * len(self._OP_FIELDS))()
+        out = []
+        for i in range(l.pnp_unet_num_launches(self.handle)):
+            check(l.pnp_unet_op_describe(self.handle, i, desc), "pnp_unet_op_describe")
+            d = dict(zip(self._OP_FIELDS, (int(x) for x in desc)))
+            d["kernel"] = self.KERNELS[d["kernel"]]
+            out.append(d)
+        return out
+
+    def forward_ops(self, first: int, end: int, v: torch.Tensor, sigma: torch.Tensor, out: torch.Tensor,
+                    preclamp: torch.Tensor | None = None) -> None:
+        """Run launches ``[first, end)`` of ``forward`` (in place: activations stay in ``workspace``, the last launch
+        writes ``out`` / ``preclamp``)."""
+        v = _req(v, torch.float32, "v")
+        sigma = _req(sigma.reshape(-1).float(), torch.float32, "sigma")
+        assert v.numel() == self.B * self.H * self.W and sigma.numel() == self.B
+        assert out.is_contiguous() and out.dtype == torch.float32 and out.numel() == v.numel()
+        assert preclamp is None or (preclamp.is_contiguous() and preclamp.dtype == torch.float32
+                                    and preclamp.numel() == v.numel())
+        check(_lib.lib().pnp_unet_forward_ops(self.handle, v.data_ptr(), sigma.data_ptr(), out.data_ptr(),
+                                              preclamp.data_ptr() if preclamp is not None else None, first, end,
+                                              _lib.stream_ptr()), "pnp_unet_forward_ops")
+
+    def tensor_at(self, offset: int, C: int, H: int, W: int) -> torch.Tensor:
+        """NHWC bf16 view ``[B, H, W, C]`` of the workspace at byte ``offset`` (as ``describe`` reports it)."""
+        n = self.B * H * W * C
+        return self.workspace[offset:offset + 2 * n].view(torch.bfloat16).view(self.B, H, W, C)
+
 
 def pack_unet_weights(flat: torch.Tensor) -> torch.Tensor:
     """fp32 flat parameter vector (CUDA) -> packed bf16 tensor-core blobs (+ fp32 copy)."""

@@ -225,6 +225,26 @@ int pnp_unet_set_splitk(int mode);
 /* Locate a named NHWC bf16 activation inside the workspace (layer-wise parity tests), e.g. "down2.conv-1".  Fails (-1) for
  * micro-batched plans, whose workspace holds one micro-batch at a time. */
 int pnp_unet_plan_tensor(const pnp_unet_plan* plan, const char* name, size_t* byte_offset, int* C, int* H, int* W);
+/* Per-launch window into a plan, for tests that check each launch alone.  Both fail (-1) for micro-batched plans.
+ * pnp_unet_forward_ops runs launches [first_op, end_op) of pnp_unet_forward (0 <= first_op <= end_op <=
+ * pnp_unet_num_launches); the launches read their inputs from the workspace as the earlier launches left it.
+ * pnp_unet_op_describe writes PNP_UNET_OP_DESC_LEN values describing launch i to desc[]:
+ *   [0] kind (0 first conv, 1 tcgen05 conv, 3 upsample)   [1] id, as pnp_unet_profile reports it
+ *   [2] H, [3] W of the launch's output level
+ *   [4] [5]  in0 workspace byte offset, channels      [6] [7]  in1 (second concat segment)
+ *   [8] [9]  out                                      [10] [11] pool_out (fused MaxPool2d(2), H/2 x W/2)
+ *            (offset and channels -1 where the launch has none or the tensor is not in the workspace: the first conv
+ *             reads v and sigma, the FINAL conv writes x_out and preclamp)
+ *   [12] kernel: 0 first conv, 1 conv3x3_umma, 2 conv3x3_umma FINAL epilogue, 3 kw-stacked, 4 CTA pair, 5 split-K
+ *        cluster, 6 fast upsample (exact doubling), 7 general upsample (zero pad)
+ *   [13] KC, or the cluster size S of the split-K kernel     [14] BN (output channels per tile)
+ *   [15] rev (1: tiles walked in descending order)          [16] wres (1: weights resident in shared memory)
+ *   [17] [18] output tile width, height in pixels          [19] work tiles (pair kernel: tile pairs)   [20] grid (CTAs)
+ *   (fields 13, 14, 16 .. 20 are 0 for launches that are not tcgen05 convs) */
+#define PNP_UNET_OP_DESC_LEN 21
+int pnp_unet_forward_ops(pnp_unet_plan* plan, const float* v, const float* sigma, float* x_out, float* preclamp,
+                         int first_op, int end_op, void* stream);
+int pnp_unet_op_describe(const pnp_unet_plan* plan, int i, long long* desc);
 
 /* One 3x3 conv + bias + LeakyReLU(0.2) on the tensor cores (reference ConvLayer, noise.py:75-89) on NHWC bf16
  * tensors; the input is the channel concat of in0 (C0 ch) and in1 (C1 ch, may be NULL/0) as in `up`
